@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """Benchmark of the per-frame hot loop (BASELINE.json metric: 1080p frames/s, HBM roofline fraction).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
-One process per GPU (torchrun for N > 1).
+One process per GPU (torchrun for N > 1).  --dump-outputs writes a seeded sample of the overlay and compressed frames of the
+last timed step (rank 0's streams for N > 1) to DIR as float32 .npy files (dump_outputs).
 
 * N = 1: `value` is BASELINE configs[1] -- one 1080p stream, 1800 frames per step, K=5 window vote -- with the clip and
   the output buffers resident in HBM (11.2 GB in, 22.4 GB out per step, far larger than L2); `e2e` is the same loop
@@ -28,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from untouched (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -68,7 +70,15 @@ def parse_args():
     p.add_argument("--no-streams", action="store_true", help="N = 1: skip the 64-stream section")
     p.add_argument("--no-fd", action="store_true", help="N = 1: skip the fd-mode section")
     p.add_argument("--cpu-config1", action="store_true", help="also time BASELINE configs[0] (480p, 300 frames) on the host (~3-5 min)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write a seeded sample of what the last timed step computed (overlay and "
+                        "compressed frames) to DIR/<name>.npy as float32, for comparing two builds output for output")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        p.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 def peaks():
@@ -346,6 +356,23 @@ def timed_steps(ctx, pipe, one_pass, steps, warmup, sampler=None):
     return ctx.max_over_ranks(e0.elapsed_time(e1)), pipe.launch_count() - launches0
 
 
+DUMP_SAMPLES = 1 << 22          # elements kept per output array: 16 MB as float32
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each device array of `arrays` to out_dir/<name>.npy as a float32 vector: the elements of the flattened array at
+    the sorted positions np.random.default_rng(0).integers(0, size, DUMP_SAMPLES), or all of them when the array is no larger.
+    The positions depend only on the array's size, so two builds run with the same arguments dump comparable samples."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        flat = t.reshape(-1)
+        if flat.numel() > DUMP_SAMPLES:
+            pos = np.sort(np.random.default_rng(0).integers(0, flat.numel(), DUMP_SAMPLES))
+            flat = flat[torch.from_numpy(pos).to(flat.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), flat.cpu().numpy().astype(np.float32))
+
+
 def profile_pass(ctx, pipe, one_pass, steps):
     """Second timed region, same steps, strict stream order (kernels serialised) with CUDA events around every kernel group on
     its launch stream: per-kernel times for the roofline are not inflated by concurrently running kernels."""
@@ -415,8 +442,9 @@ def k4_roofline(prof, ms_serial, frames_per_step, steps, px, loop_fps_per_gpu, d
     return roofline
 
 
-def measure_single_stream(ctx, args, mode, steps, sampler=None, want_e2e=True):
-    """One 1080p stream per rank (BASELINE configs[1] at N = 1): resident loop, profile pass, end-to-end pass."""
+def measure_single_stream(ctx, args, mode, steps, sampler=None, want_e2e=True, dump_dir=None):
+    """One 1080p stream per rank (BASELINE configs[1] at N = 1): resident loop, profile pass, end-to-end pass.  dump_dir: where
+    to dump the last timed step's overlay and compressed frames (dump_outputs)."""
     import torch
     from dynamic_video_compression_surveillance_b200 import pipeline as P
     from dynamic_video_compression_surveillance_b200.synth import make_clip, RESOLUTIONS
@@ -446,6 +474,8 @@ def measure_single_stream(ctx, args, mode, steps, sampler=None, want_e2e=True):
         pipe.flush()          # the current stream re-joins the library's internal streams
 
     ms, launches = timed_steps(ctx, pipe, one_pass, steps, args.warmup, sampler)
+    if dump_dir is not None:
+        dump_outputs(dump_dir, {"overlay": ov, "compressed": cp})
     value = steps * n * ctx.world / (ms / 1e3)
     ms_serial, prof = profile_pass(ctx, pipe, one_pass, steps)
     res = {"value": value, "ms": ms, "launches": launches, "ms_serial": ms_serial, "prof": prof, "frames_per_step": n,
@@ -476,8 +506,9 @@ def measure_single_stream(ctx, args, mode, steps, sampler=None, want_e2e=True):
     return res
 
 
-def measure_streams(ctx, args, steps, sampler=None, want_e2e=True):
-    """BASELINE configs[3]: args.streams camera streams sharded over the ranks, one lock-step stream group per rank."""
+def measure_streams(ctx, args, steps, sampler=None, want_e2e=True, dump_dir=None):
+    """BASELINE configs[3]: args.streams camera streams sharded over the ranks, one lock-step stream group per rank.  dump_dir:
+    where to dump the last timed step's overlay and compressed frames of this rank's streams (dump_outputs)."""
     import torch
     from dynamic_video_compression_surveillance_b200 import pipeline as P, sharding
     from dynamic_video_compression_surveillance_b200.synth import make_clip, RESOLUTIONS
@@ -504,6 +535,8 @@ def measure_streams(ctx, args, steps, sampler=None, want_e2e=True):
         pipe.flush()
 
     ms, launches = timed_steps(ctx, pipe, one_pass, steps, args.warmup, sampler)
+    if dump_dir is not None:
+        dump_outputs(dump_dir, {"overlay": ov, "compressed": cp})
     frames_per_step_rank = S * F * nb
     value = steps * args.streams * F * nb / (ms / 1e3)
     ms_serial, prof = profile_pass(ctx, pipe, one_pass, steps)
@@ -605,8 +638,9 @@ def run_b200(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()                      # started early: nvidia-smi's own start-up must not fall into the timed region
     extra = {}
+    dump_dir = args.dump_outputs if rank == 0 else None
     if world == 1:
-        main = measure_single_stream(ctx, args, args.mode, args.steps, sampler, want_e2e=not args.no_e2e)
+        main = measure_single_stream(ctx, args, args.mode, args.steps, sampler, want_e2e=not args.no_e2e, dump_dir=dump_dir)
         clocks = sampler.stop()
         cfg, scaling = workload_config(args, h, w), "weak"
         if not args.no_fd and args.mode == "window":
@@ -632,7 +666,7 @@ def run_b200(args, rank, world, local_rank):
                                   "ms_per_step": st["ms"] / max(3, args.steps // 2), "frames_per_step": st["frames_per_step"],
                                   "e2e": st.get("e2e"), "vs_single_stream": st["value"] / main["value"]}
     else:
-        main = measure_streams(ctx, args, args.steps, sampler, want_e2e=not args.no_e2e)
+        main = measure_streams(ctx, args, args.steps, sampler, want_e2e=not args.no_e2e, dump_dir=dump_dir)
         clocks = sampler.stop() if rank == 0 else None
         cfg, scaling = streams_config(args, h, w, world), "strong"
         weak = measure_single_stream(ctx, args, "window", max(3, args.steps // 2), want_e2e=False)

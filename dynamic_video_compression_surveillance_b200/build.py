@@ -23,10 +23,10 @@ def find_nvcc() -> str:
     return nvcc
 
 
-def is_stale() -> bool:
-    if not os.path.exists(LIB):
+def is_stale(lib: str = LIB) -> bool:
+    if not os.path.exists(lib):
         return True
-    t = os.path.getmtime(LIB)
+    t = os.path.getmtime(lib)
     return any(os.path.getmtime(d) > t for d in DEPS if os.path.exists(d))
 
 
@@ -34,21 +34,18 @@ LIB_MEASURE = os.path.join(HERE, "libdvc_b200_measure.so")
 
 
 def build(force: bool = False, verbose: bool = False, measure: bool = False) -> str:
-    """measure=True builds the -DDVC_MEASURE flavour (environment switches for A/B runs, tools/ only) next to the product."""
-    if measure:
-        r = subprocess.run([find_nvcc()] + NVCC_FLAGS + ["-DDVC_MEASURE", "-o", LIB_MEASURE, SRC], capture_output=True, text=True)
-        if r.returncode != 0:
-            raise RuntimeError("nvcc failed:\n" + r.stdout + r.stderr)
-        return LIB_MEASURE
-    if not force and not is_stale():
-        return LIB
-    cmd = [find_nvcc()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB, SRC]
+    """measure=True builds the -DDVC_MEASURE flavour (environment switches for A/B runs: tools/ and the gray-variant test)
+    next to the product."""
+    lib = LIB_MEASURE if measure else LIB
+    if not force and not is_stale(lib):
+        return lib
+    cmd = [find_nvcc()] + NVCC_FLAGS + (["-DDVC_MEASURE"] if measure else []) + (["-Xptxas", "-v"] if verbose else []) + ["-o", lib, SRC]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + r.stdout + r.stderr)
     if verbose:
         sys.stderr.write(r.stderr)
-    return LIB
+    return lib
 
 
 if __name__ == "__main__":
