@@ -162,7 +162,7 @@ static void window_min_counts(double alpha, int K, MinCounts& mc) {
 // ------------------------------------------------------------------------------------------------
 // Function attributes and __constant__ uploads are per device: one-time set-up is tracked per CUDA device ordinal so that
 // handles on several GPUs in one process all get it.
-// Measurement switches (kernel generations, ring geometry, copy-only probes: DESIGN.md section 6a) exist only in the
+// Measurement switches (kernel generations, band and chunk sizes, copy-only probes: DESIGN.md section 6a) exist only in the
 // -DDVC_MEASURE flavour of the library that tools/ build for A/B runs.  The product build ignores the environment, so a
 // stray variable can never change what the loop computes.
 #ifdef DVC_MEASURE
@@ -463,16 +463,65 @@ static int launch_degrade_edges(char* ERRBUF, const uint8_t* frames, const uint3
     return DVC_OK;
 }
 
+// The kernel that degrades the whole blocks of a frame (partial blocks at the right / bottom edge: launch_degrade_edges).
+// `addr_bits` is the OR of the frame and output addresses.  4x4 blocks are FD only (MCO takes 8x8, checked by the caller).
+enum class DegradeKernel { edges, ring4, packed4, generic4, packed8, generic8 };
+
+static DegradeKernel degrade_kernel(int bs, int H, int W, float q, uintptr_t addr_bits) {
+    if (bs != 4 && bs != 8) return DegradeKernel::edges;      // rare block sizes: every block through the exact general path
+    // packed kernels (k_degrade4p.cuh): 8-byte vector access, Markstein quotient (exact for q in [0.01, 1e6]); otherwise the
+    // one-thread-per-block kernels, bytewise and with the IEEE division
+    const bool packed = W % 8 == 0 && q >= 0.01f && q <= 1.0e6f && addr_bits % 8 == 0;
+    if (bs == 8) return packed ? DegradeKernel::packed8 : DegradeKernel::generic8;
+    if (!packed) return DegradeKernel::generic4;
+    // the ring's bulk copies need every frame of the batch 16-byte aligned, and 16-byte row pieces when a block row is split
+    // over several tiles (W > 2048)
+    const bool ring = addr_bits % 16 == 0 && (size_t)H * W * 3 % 16 == 0 && (W / 8 <= 256 || W % 16 == 0);
+    return ring ? DegradeKernel::ring4 : DegradeKernel::packed4;
+}
+
+// Tiles and shared-memory ring of k_degrade4s for n frames, and the dynamic shared memory it needs; false if that does not fit.
+static bool k4_ring_geometry(int n, int H, int W, K4SGeom& sg, size_t& smem) {
+    const int wpr = words_per_row(W), gpr = W / 8, nbr = H / 4;
+    K4Geom& g = sg.g;
+    if (gpr <= 256) {
+        g.parts = 1; g.gp = gpr; g.nb = std::max(1, std::min(nbr, std::min(256 / gpr, 256 / wpr))); g.sp = W * 3;
+        g.span_bytes = g.nb * 4 * W * 3;
+    } else {
+        g.parts = (gpr + 255) / 256;
+        g.gp = (((gpr + g.parts - 1) / g.parts) + 15) & ~15;
+        g.parts = (gpr + g.gp - 1) / g.gp;
+        g.nb = 1; g.sp = g.gp * 24; g.span_bytes = 4 * g.sp;
+    }
+    g.mask_bytes = 4 * g.nb * wpr * 4;
+    sg.tiles_per_frame = g.parts == 1 ? (int)cdiv(nbr, g.nb) : nbr * g.parts;
+    sg.n_tiles = sg.tiles_per_frame * n;
+    sg.stage_bytes = (g.span_bytes + 2 * g.mask_bytes + 127) & ~127;
+    sg.ybuf_bytes = (g.span_bytes + 127) & ~127;
+    const size_t smem_cap = 224 * 1024;
+    auto smem_need = [&](int stages) {
+        return (size_t)stages * sg.stage_bytes + (size_t)K4S_GROUPS * sg.ybuf_bytes + 8 * (2 * stages) + 16 + 16 * stages;
+    };
+    int S = 6;
+    while (smem_need(S) > smem_cap && S > 2) --S;
+    sg.stages = S;
+    smem = smem_need(S);
+    // A group hands a stage back only while it works on its next tile, so every group needs a second stage to move on to:
+    // with stages <= groups the ring would wait on itself.
+    return S > K4S_GROUPS && smem <= smem_cap;
+}
+
 static int launch_degrade(char* ERRBUF, const uint8_t* frames, const uint32_t* over127, const uint32_t* nonzero,
                           uint8_t* compressed, uint8_t* overlay, int n, int H, int W, int bs, float q, int flavour,
                           Counters* counters, cudaStream_t st) {
-    const int wpr = words_per_row(W);
     if (bs < 1 || bs > 8)
         return set_err(ERRBUF, DVC_ERR_UNSUPPORTED, "block_size %d: the GPU path implements 1..8 (cv2's DCT routines for longer blocks are not restated)", bs);
     if (flavour == DVC_DEGRADE_MCO && bs != 8) return set_err(ERRBUF, DVC_ERR_INVALID, "MCO flavour uses 8x8 blocks");
     if (!(q > 0.0f)) return set_err(ERRBUF, DVC_ERR_INVALID, "quantization_level must be > 0");
     if (n <= 0) return DVC_OK;
-    if (bs != 4 && bs != 8)      // rare block sizes: every block through the general one-thread-per-block path (exact, not fast)
+
+    const DegradeKernel kern = degrade_kernel(bs, H, W, q, (uintptr_t)frames | (uintptr_t)compressed | (uintptr_t)overlay);
+    if (kern == DegradeKernel::edges)
         return launch_degrade_edges(ERRBUF, frames, over127, nonzero, compressed, overlay, n, H, W, bs, q, flavour, counters, st, true);
     if (H % bs || W % bs) {
         // full blocks by the kernels below (they floor H and W to whole blocks), partial edge blocks by a small second launch
@@ -480,135 +529,58 @@ static int launch_degrade(char* ERRBUF, const uint8_t* frames, const uint32_t* o
         if (rc) return rc;
         if (H < bs || W < bs) return DVC_OK;
     }
-    if (flavour == DVC_DEGRADE_FD && bs == 4 && W % 8 == 0) {
-        QuantConsts qc;
-        const float iq = 1.0f / q;
-        qc.k[0] = iq; qc.k[1] = iq * 0.5f; qc.k[2] = iq * 0.25f;
-        qc.o[0] = q; qc.o[1] = q * 0.5f; qc.o[2] = q * 0.25f;
-        qc.q = q;
-        // |t - fl(d/q)| <= 1.5 * 2^-23 * |d/q| and |d/q| <= 512/q (orthonormal 4x4 DCT of values in [-128,127]):
-        // outside a band of 4x that bound around the ties the fast rounding provably equals np.round(d/q).
-        const float band = std::max(1.0e-5f, 4.0f * 1.8e-7f * (512.0f / q));
-        qc.tie_lo = 0.5f - band;
-        qc.fast = band <= 0.01f && q <= 1.0e6f;
-        dim3 grid(cdiv((size_t)(W / 8) * (H / 4), 256), n);
-        static const bool luma_dp4a = measure_env("DVC_LUMA_DP4A", 1) != 0;
-        static const bool tma_env = measure_env("DVC_K4_TMA_STORE", 1) != 0;
-        const bool tma = tma_env && W % 16 == 0;
-        const size_t smem = tma ? (size_t)K4_STAGE_BYTES : 0;
-        static PerDeviceOnce attr_set;
-        if (auto once = attr_set.begin()) {
-            CU(cudaFuncSetAttribute(k_degrade4<true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            CU(cudaFuncSetAttribute(k_degrade4<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            once.commit();
+
+    static PerDeviceOnce attr_once;
+    if (auto once = attr_once.begin()) {
+        CU(cudaFuncSetAttribute(k_degrade4s, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        CU(cudaFuncSetAttribute(k_degrade8<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, k8_smem_bytes<0>()));
+        CU(cudaFuncSetAttribute(k_degrade8<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, k8_smem_bytes<1>()));
+        once.commit();
+    }
+    const int wpr = words_per_row(W);
+    const bool fd = flavour == DVC_DEGRADE_FD;
+    // quotient constants of the packed kernels; the 4x4 ones carry the DCT butterflies' folded power-of-two scalings
+    QuantP qp;
+    for (int ne = 0; ne < 3; ++ne) {
+        const float scale = bs == 4 ? (float)(1 << ne) : 1.0f;
+        qp.rcp[ne] = 1.0f / (q * scale);
+        qp.nqs[ne] = -(q * scale);
+        qp.o[ne] = q / scale;
+    }
+    const dim3 grid_generic(cdiv((size_t)(W / bs) * (H / bs), 128), n);
+    switch (kern) {
+        case DegradeKernel::ring4: {
+            K4SGeom sg;
+            size_t smem = 0;
+            if (!k4_ring_geometry(n, H, W, sg, smem))
+                return set_err(ERRBUF, DVC_ERR_UNSUPPORTED, "K4 ring: %d stages for %d consumer groups do not fit (%zu bytes of shared memory)",
+                               sg.stages, K4S_GROUPS, smem);
+            int dev = 0, sms = 0;
+            CU(cudaGetDevice(&dev));
+            CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+            k_degrade4s<<<(unsigned)std::min(sg.n_tiles, sms), K4S_THREADS, smem, st>>>(frames, over127, nonzero, compressed, overlay,
+                                                                                        H, W, wpr, qp, counters, sg);
+            break;
         }
-        static const bool packed_env = measure_env("DVC_K4_PACKED", 1) != 0;
-        if (packed_env && q >= 0.01f && q <= 1.0e6f) {
-            // packed-pair kernel: quotient by Markstein correction (exact for normal-range q), magic rounding needs |d/q| < 2^22
-            QuantP qp;
-            for (int ne = 0; ne < 3; ++ne) {
-                const float qs = q * (float)(1 << ne);
-                qp.rcp[ne] = 1.0f / qs;
-                qp.nqs[ne] = -qs;
-                qp.o[ne] = q / (float)(1 << ne);
-            }
-            static PerDeviceOnce attr_p;
-            if (auto once = attr_p.begin()) {
-                CU(cudaFuncSetAttribute(k_degrade4p<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                once.commit();
-            }
-            // DVC_K4_PERSIST=0 selects the CTA-per-256-groups kernel (k_degrade4p) for A/B; it is also the fallback for pointers
-            // that are not 16-byte aligned and for W > 2048 with W % 16 != 0 (bulk copies need 16-byte pieces)
-            static const bool ring_env = measure_env("DVC_K4_PERSIST", 1) != 0;
-            const int gpr = W / 8, nbr = H / 4;
-            const bool ptr16 = ((((uintptr_t)frames) | ((uintptr_t)compressed) | ((uintptr_t)overlay)) & 15u) == 0 &&
-                               ((size_t)H * W * 3) % 16 == 0;          // every frame of the batch starts 16-byte aligned
-            if (ring_env && ptr16 && (gpr <= 256 || W % 16 == 0)) {
-                K4Geom g;
-                if (gpr <= 256) {
-                    g.parts = 1; g.gp = gpr; g.nb = std::max(1, std::min(nbr, std::min(256 / gpr, 256 / wpr))); g.sp = W * 3;
-                    g.span_bytes = g.nb * 4 * W * 3;
-                } else {
-                    g.parts = (gpr + 255) / 256;
-                    g.gp = (((gpr + g.parts - 1) / g.parts) + 15) & ~15;
-                    g.parts = (gpr + g.gp - 1) / g.gp;
-                    g.nb = 1; g.sp = g.gp * 24; g.span_bytes = 4 * g.sp;
-                }
-                g.mask_bytes = 4 * g.nb * wpr * 4;
-                static const int dbg = measure_env("DVC_K4_DEBUG", 0);
-                g.debug = dbg;
-                {
-                    static const int env_stages = measure_env("DVC_K4_STAGES", 6);
-                    static const int env_groups = measure_env("DVC_K4_GROUPS", 2);
-                    static const int env_piece = measure_env("DVC_K4_PIECE", 0);
-                    static const int env_ctas = measure_env("DVC_K4_CTAS", 0);
-                    int dev = 0, sms = 0;
-                    CU(cudaGetDevice(&dev));
-                    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-                    K4SGeom sg;
-                    sg.g = g;
-                    sg.tiles_per_frame = g.parts == 1 ? (int)cdiv(nbr, g.nb) : nbr * g.parts;
-                    sg.n_tiles = sg.tiles_per_frame * n;
-                    sg.stage_bytes = (g.span_bytes + 2 * g.mask_bytes + 127) & ~127;
-                    sg.ybuf_bytes = (g.span_bytes + 127) & ~127;
-                    const int G = env_groups == 1 ? 1 : (env_groups == 3 ? 3 : 2);
-                    int S = std::max(G, env_stages);
-                    const size_t smem_cap = 224 * 1024;
-                    auto smem_need = [&](int stages) { return (size_t)stages * sg.stage_bytes + (size_t)G * sg.ybuf_bytes + 8 * (2 * stages) + 16 + 16 * stages; };
-                    while (smem_need(S) > smem_cap && S > 2) --S;
-                    // A group hands a stage back only while it works on its next tile, so every group needs a second stage to
-                    // move on to: with stages <= groups the ring would wait on itself.
-                    if (S <= G || smem_need(S) > smem_cap) {
-                        return set_err(ERRBUF, DVC_ERR_UNSUPPORTED, "K4 ring: %d stages for %d consumer groups do not fit (%zu bytes of shared memory)", S, G, smem_need(S));
-                    }
-                    sg.stages = S;
-                    // bulk-copy granularity: whole spans by default (piece sizes from 1.4 KB to the full 23 KB span were
-                    // measured: no gain from smaller pieces, profiles/README.md r1l)
-                    sg.piece_bytes = env_piece > 0 ? ((env_piece + 15) & ~15) : 32768;
-                    const size_t smem_s = smem_need(S);
-                    const unsigned ctas = (unsigned)std::min(sg.n_tiles, env_ctas > 0 ? env_ctas : sms);
-                    static PerDeviceOnce attr_s;
-                    if (auto once = attr_s.begin()) {
-                        CU(cudaFuncSetAttribute(k_degrade4s<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-                        CU(cudaFuncSetAttribute(k_degrade4s<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-                        CU(cudaFuncSetAttribute(k_degrade4s<3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-                        once.commit();
-                    }
-                    if (G == 1) k_degrade4s<1, 1><<<ctas, 32 + 256, smem_s, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qp, counters, sg);
-                    else if (G == 3) k_degrade4s<3, 1><<<ctas, 32 + 768, smem_s, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qp, counters, sg);
-                    else k_degrade4s<2, 1><<<ctas, 32 + 512, smem_s, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qp, counters, sg);
-                }
-            } else
-            if (tma) k_degrade4p<true><<<grid, 256, smem, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qp, counters);
-            else k_degrade4p<false><<<grid, 256, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qp, counters);
-        } else
-        if (luma_dp4a && tma) k_degrade4<true, true><<<grid, 256, smem, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qc, counters);
-        else if (luma_dp4a) k_degrade4<true, false><<<grid, 256, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qc, counters);
-        else if (tma) k_degrade4<false, true><<<grid, 256, smem, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qc, counters);
-        else k_degrade4<false, false><<<grid, 256, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qc, counters);
-    } else {
-        dim3 grid(cdiv((size_t)(W / bs) * (H / bs), 128), n);
-        static const bool k8_env = measure_env("DVC_K4_BLOCK8_FAST", 1) != 0;
-        const bool ptr8 = ((((uintptr_t)frames) | ((uintptr_t)compressed) | ((uintptr_t)overlay)) & 7u) == 0;
-        if (bs == 8 && W % 8 == 0 && k8_env && ptr8 && q >= 0.01f && q <= 1.0e6f) {
-            QuantP qp;
-            for (int ne = 0; ne < 3; ++ne) { qp.rcp[ne] = 1.0f / q; qp.nqs[ne] = -q; qp.o[ne] = q; }     // no folded scalings in the 8-point path
-            static PerDeviceOnce k8_attr;
-            if (auto once = k8_attr.begin()) {
-                CU(cudaFuncSetAttribute(k_degrade8<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, k8_smem_bytes<0>()));
-                CU(cudaFuncSetAttribute(k_degrade8<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, k8_smem_bytes<1>()));
-                once.commit();
-            }
-            dim3 g8(cdiv((size_t)(W / 8) * (H / 8), K8_THREADS), n);
-            if (flavour == DVC_DEGRADE_FD) k_degrade8<0><<<g8, K8_THREADS, k8_smem_bytes<0>(), st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qp, counters);
+        case DegradeKernel::packed4:
+            k_degrade4p<<<dim3(cdiv((size_t)(W / 8) * (H / 4), 256), n), 256, 0, st>>>(frames, over127, nonzero, compressed, overlay,
+                                                                                        H, W, wpr, qp, counters);
+            break;
+        case DegradeKernel::generic4:
+            k_degrade_generic<4, 0><<<grid_generic, 128, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, q, counters);
+            break;
+        case DegradeKernel::packed8: {
+            const dim3 g8(cdiv((size_t)(W / 8) * (H / 8), K8_THREADS), n);
+            if (fd) k_degrade8<0><<<g8, K8_THREADS, k8_smem_bytes<0>(), st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qp, counters);
             else k_degrade8<1><<<g8, K8_THREADS, k8_smem_bytes<1>(), st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, qp, counters);
-        } else
-        if (flavour == DVC_DEGRADE_FD && bs == 4)
-            k_degrade_generic<4, 0><<<grid, 128, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, q, counters);
-        else if (flavour == DVC_DEGRADE_FD)
-            k_degrade_generic<8, 0><<<grid, 128, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, q, counters);
-        else
-            k_degrade_generic<8, 1><<<grid, 128, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, q, counters);
+            break;
+        }
+        case DegradeKernel::generic8:
+            if (fd) k_degrade_generic<8, 0><<<grid_generic, 128, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, q, counters);
+            else k_degrade_generic<8, 1><<<grid_generic, 128, 0, st>>>(frames, over127, nonzero, compressed, overlay, H, W, wpr, q, counters);
+            break;
+        case DegradeKernel::edges:
+            break;
     }
     CHECK_LAUNCH();
     return DVC_OK;

@@ -63,143 +63,6 @@ __global__ void k_counters_add(Counters* c, unsigned long long frames, unsigned 
     atomicAdd(&c->blocks, blocks);
 }
 
-// ------------------------------------------------------------------------------------------------
-// Fast path: block_size 4, W % 8 == 0, H % 4 == 0.  One thread owns 8 pixels x 4 rows = two 4x4 blocks
-// = 4 x 24 contiguous bytes (twelve 8-byte streaming loads in flight, 64 registers -> 32 warps per SM).
-// Algorithmic HBM bytes: 3 read + 3 (+3) written per pixel plus the mask bit-plane(s).
-//
-// Instruction diet for the static-block path (97 % of blocks on surveillance content):
-//  * the x0.5 factors of the DCT butterflies are exact power-of-two scalings, so they are folded into the
-//    quantiser constants instead of being multiplied out (bitwise identical results);
-//  * round(d / q) is computed as magic-number rounding of d * (1/q); only coefficients that land within
-//    1e-3 of a rounding tie (where the float32 division's own rounding can matter) take the exact
-//    IEEE-division path, so the result equals np.round(d / q) always;
-//  * float <-> byte conversions avoid the conversion (XU) pipe: bytes enter as 2^23 + b bit patterns, leave
-//    through a round-down add of 2^23 whose low mantissa byte is floor(v), picked up by PRMT.
-// grid: (ceil(W/8 * H/4 / 256), n_frames)
-// ------------------------------------------------------------------------------------------------
-struct QuantConsts {
-    float k[3];     // (1/q) * {1, 1/2, 1/4}: forward scale by number of even indices among (row, col)
-    float o[3];     // q * {1, 1/2, 1/4}: output scale (pre-applies the inverse butterflies' x0.5)
-    float q;
-    float tie_lo;   // coefficients whose distance from the rounded value exceeds this are re-done exactly
-    int fast;       // magic-number path valid (q large enough for tie_lo to be meaningful)
-};
-
-// forward 4-point DCT without the x0.5 on outputs 0 and 2 (folded into QuantConsts::k)
-DEVI void dct4_fwd_ns(float& x0, float& x1, float& x2, float& x3) {
-    const float s0 = __fadd_rn(x0, x3), s1 = __fadd_rn(x1, x2);
-    const float d0 = __fsub_rn(x0, x3), d1 = __fsub_rn(x1, x2);
-    x0 = __fadd_rn(s0, s1);
-    x2 = __fsub_rn(s0, s1);
-    x1 = __fmaf_rn(DVC_C3, d1, __fmul_rn(DVC_C1, d0));
-    x3 = __fmaf_rn(DVC_C3, d0, -__fmul_rn(DVC_C1, d1));
-}
-// inverse 4-point DCT whose inputs 0 and 2 arrive pre-multiplied by 0.5 (QuantConsts::o)
-DEVI void dct4_inv_ps(float& x0, float& x1, float& x2, float& x3) {
-    const float e0 = __fadd_rn(x0, x2), e1 = __fsub_rn(x0, x2);
-    const float o0 = __fmaf_rn(DVC_C3, x3, __fmul_rn(DVC_C1, x1));
-    const float o1 = __fmaf_rn(DVC_C3, x1, -__fmul_rn(DVC_C1, x3));
-    x0 = __fadd_rn(e0, o0);
-    x3 = __fsub_rn(e0, o0);
-    x1 = __fadd_rn(e1, o1);
-    x2 = __fsub_rn(e1, o1);
-}
-
-// NE = number of even indices among (row, col): the coefficient carries a pending scale 2^-NE.
-template <int NE>
-DEVI float quantise_fast(float d, const QuantConsts& qc, float& tie_dist) {
-    const float magic = 12582912.0f;                      // 1.5 * 2^23: add/sub rounds half to even
-    const float t = __fmul_rn(d, qc.k[NE]);
-    const float n = __fsub_rn(__fadd_rn(t, magic), magic);
-    tie_dist = fmaxf(tie_dist, fabsf(__fsub_rn(t, n)));   // 0.5 = on a rounding tie
-    return __fmul_rn(n, qc.o[NE]);
-}
-template <int NE>
-DEVI float quantise_exact(float d, const QuantConsts& qc) {   // np.round(d / q) with the IEEE division
-    const float n = rintf(__fdiv_rn(__fmul_rn(d, NE == 0 ? 1.0f : (NE == 1 ? 0.5f : 0.25f)), qc.q));
-    return __fmul_rn(n, qc.o[NE]);
-}
-
-DEVI void fwd_dct_block(float (&v)[4][4]) {
-#pragma unroll
-    for (int r = 0; r < 4; ++r) dct4_fwd_ns(v[r][0], v[r][1], v[r][2], v[r][3]);
-#pragma unroll
-    for (int c = 0; c < 4; ++c) dct4_fwd_ns(v[0][c], v[1][c], v[2][c], v[3][c]);
-}
-DEVI void inv_dct_block(float (&v)[4][4]) {
-#pragma unroll
-    for (int r = 0; r < 4; ++r) dct4_inv_ps(v[r][0], v[r][1], v[r][2], v[r][3]);
-#pragma unroll
-    for (int c = 0; c < 4; ++c) dct4_inv_ps(v[0][c], v[1][c], v[2][c], v[3][c]);
-}
-// Fast quantiser for a whole block.  The four coefficients with even row and column index are exact
-// integers / 4 (their basis is +-1/2), so real ties (d/q = n + 1/2 exactly) do occur there: they are checked
-// and redone with the IEEE division individually.  The other twelve have irrational basis functions; a value
-// within tie_lo of a rounding tie is a ~1e-5 event, reported through the return value (the caller then redoes
-// the block exactly).
-DEVI float quantise_block_fast(float (&v)[4][4], const QuantConsts& qc) {
-    float tie = 0.0f, tie_r = 0.0f;
-    const float d00 = v[0][0], d02 = v[0][2], d20 = v[2][0], d22 = v[2][2];
-    v[0][0] = quantise_fast<2>(d00, qc, tie_r); v[0][2] = quantise_fast<2>(d02, qc, tie_r);
-    v[2][0] = quantise_fast<2>(d20, qc, tie_r); v[2][2] = quantise_fast<2>(d22, qc, tie_r);
-    if (tie_r > qc.tie_lo) {
-        v[0][0] = quantise_exact<2>(d00, qc); v[0][2] = quantise_exact<2>(d02, qc);
-        v[2][0] = quantise_exact<2>(d20, qc); v[2][2] = quantise_exact<2>(d22, qc);
-    }
-    v[0][1] = quantise_fast<1>(v[0][1], qc, tie); v[0][3] = quantise_fast<1>(v[0][3], qc, tie);
-    v[2][1] = quantise_fast<1>(v[2][1], qc, tie); v[2][3] = quantise_fast<1>(v[2][3], qc, tie);
-#pragma unroll
-    for (int r = 1; r < 4; r += 2) {
-        v[r][0] = quantise_fast<1>(v[r][0], qc, tie); v[r][1] = quantise_fast<0>(v[r][1], qc, tie);
-        v[r][2] = quantise_fast<1>(v[r][2], qc, tie); v[r][3] = quantise_fast<0>(v[r][3], qc, tie);
-    }
-    return tie;
-}
-DEVI void quantise_block_exact(float (&v)[4][4], const QuantConsts& qc) {
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-        if ((r & 1) == 0) {
-            v[r][0] = quantise_exact<2>(v[r][0], qc); v[r][1] = quantise_exact<1>(v[r][1], qc);
-            v[r][2] = quantise_exact<2>(v[r][2], qc); v[r][3] = quantise_exact<1>(v[r][3], qc);
-        } else {
-            v[r][0] = quantise_exact<1>(v[r][0], qc); v[r][1] = quantise_exact<0>(v[r][1], qc);
-            v[r][2] = quantise_exact<1>(v[r][2], qc); v[r][3] = quantise_exact<0>(v[r][3], qc);
-        }
-    }
-}
-
-// luma - 128 as float without the conversion pipe: (2^23 | y) read as float is 2^23 + y exactly
-DEVI float luma_m128_f(uint32_t b, uint32_t g, uint32_t r) {
-    const uint32_t y = (1868u * b + 9617u * g + 4899u * r + 8192u) >> 14;
-    return __fsub_rn(__uint_as_float(0x4B000000u | y), 8388736.0f);      // 2^23 + 128
-}
-// luma - 128 of the four pixels held in three packed BGR words.
-// Y << 14 = 1868 B + 9617 G + 4899 R + 8192 is evaluated with IDP.4A on the packed words (no byte extraction):
-// each coefficient is split into a high and a low byte, sum = 256 * dot(px, hi) + dot(px, lo).
-DEVI float luma_from_sum(uint32_t hi, uint32_t lo) {
-    const uint32_t y = ((hi << 8) + lo) >> 14;
-    return __fsub_rn(__uint_as_float(0x4B000000u | y), 8388736.0f);      // 2^23 + 128
-}
-template <bool DP4A>
-DEVI void luma_row4(uint32_t w0, uint32_t w1, uint32_t w2, float (&v)[4]) {
-  if (!DP4A) {
-    v[0] = luma_m128_f(w0 & 0xffu, (w0 >> 8) & 0xffu, (w0 >> 16) & 0xffu);
-    v[1] = luma_m128_f(w0 >> 24, w1 & 0xffu, (w1 >> 8) & 0xffu);
-    v[2] = luma_m128_f((w1 >> 16) & 0xffu, w1 >> 24, w2 & 0xffu);
-    v[3] = luma_m128_f((w2 >> 8) & 0xffu, (w2 >> 16) & 0xffu, w2 >> 24);
-  } else {
-    // 1868 = 7*256+76, 9617 = 37*256+145, 4899 = 19*256+35
-    const uint32_t L0 = 76u | (145u << 8) | (35u << 16), H0 = 7u | (37u << 8) | (19u << 16);            // B G R .
-    const uint32_t L1a = 76u << 24, H1a = 7u << 24, L1b = 145u | (35u << 8), H1b = 37u | (19u << 8);     // ...B | G R
-    const uint32_t L2a = (76u << 16) | (145u << 24), H2a = (7u << 16) | (37u << 24), L2b = 35u, H2b = 19u;  // ..BG | R
-    const uint32_t L3 = (76u << 8) | (145u << 16) | (35u << 24), H3 = (7u << 8) | (37u << 16) | (19u << 24); // .BGR
-    v[0] = luma_from_sum(__dp4a(w0, H0, 0u), __dp4a(w0, L0, 8192u));
-    v[1] = luma_from_sum(__dp4a(w1, H1b, __dp4a(w0, H1a, 0u)), __dp4a(w1, L1b, __dp4a(w0, L1a, 8192u)));
-    v[2] = luma_from_sum(__dp4a(w2, H2b, __dp4a(w1, H2a, 0u)), __dp4a(w2, L2b, __dp4a(w1, L2a, 8192u)));
-    v[3] = luma_from_sum(__dp4a(w2, H3, 0u), __dp4a(w2, L3, 8192u));
-  }
-}
 // np.clip(v + 128, 0, 255) stored to uint8 (truncation): one saturating round-toward-zero conversion
 DEVI uint32_t out_byte_bits(float v) {
     uint32_t r;
@@ -207,191 +70,12 @@ DEVI uint32_t out_byte_bits(float v) {
     return r;
 }
 
-// TMA_STORE: results are staged per CTA in shared memory (256 adjacent pixel groups = 6 KB contiguous per row) and
-// written with cp.async.bulk (one TMA store per row and output, issued by one thread), so HBM sees whole lines
-// instead of 8-byte pieces at a 24-byte lane stride.  Needs W % 16 == 0 (16-byte aligned row segments).
-constexpr int K4_ROW_BYTES = 256 * 24;                 // one row of a CTA's 256 pixel groups
-constexpr int K4_STAGE_BYTES = 2 * 4 * K4_ROW_BYTES;   // two outputs x four rows
-
-DEVI void sts64(uint32_t saddr, uint32_t a, uint32_t b) {
-    asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(saddr), "r"(a), "r"(b) : "memory");
-}
-DEVI void bulk_store(const void* gdst, uint32_t ssrc, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(ssrc), "r"(bytes) : "memory");
-}
-
-template <bool DP4A, bool TMA_STORE>
-__global__ void __launch_bounds__(256, 4)
-k_degrade4(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ over127,
-           const uint32_t* __restrict__ nonzero, uint8_t* __restrict__ compressed, uint8_t* __restrict__ overlay,
-           int H, int W, int wpr, QuantConsts qc, Counters* __restrict__ counters) {
-    extern __shared__ __align__(128) uint8_t k4_stage[];
-    const int gpr = W >> 3, nbr = H >> 2;
-    const int gid = blockIdx.x * blockDim.x + threadIdx.x;
-    const int lane = threadIdx.x & 31;
-    // CTA staging area as a shared-window address: row r of output o sits at (o * 4 + r) * K4_ROW_BYTES, thread t at 24 t
-    const uint32_t wst = (uint32_t)__cvta_generic_to_shared(k4_stage) + threadIdx.x * 24;
-    unsigned n_motion = 0, n_static = 0;
-    if (gid < gpr * nbr) {
-        const int br = gid / gpr, gx = gid - br * gpr;
-        const size_t frame_off = (size_t)blockIdx.y * H * W * 3;
-        const size_t plane_off = (size_t)blockIdx.y * H * wpr;
-        const size_t base = frame_off + ((size_t)(br * 4) * W + (size_t)gx * 8) * 3;
-        const size_t pitch = (size_t)W * 3;
-        uint32_t w[4][6];
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-#pragma unroll
-            for (int i = 0; i < 3; ++i) {
-                const uint2 t = __ldcs(reinterpret_cast<const uint2*>(frames + base + r * pitch + 8 * i));
-                w[r][2 * i] = t.x; w[r][2 * i + 1] = t.y;
-            }
-        uint32_t hi[4], nz = 0;
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const size_t wo = plane_off + (size_t)(br * 4 + r) * wpr;
-            hi[r] = reinterpret_cast<const uint8_t*>(over127 + wo)[gx];
-            nz |= reinterpret_cast<const uint8_t*>(nonzero + wo)[gx];
-        }
-        // ---- overlay: paint (B,G,R) = (0,0,255) where acc > 127 ----
-        if (overlay) {
-#pragma unroll
-            for (int r = 0; r < 4; ++r) {
-                if (hi[r] == 0u) {
-#pragma unroll
-                    for (int i = 0; i < 3; ++i) {
-                        if (TMA_STORE) sts64(wst + r * K4_ROW_BYTES + 8 * i, w[r][2 * i], w[r][2 * i + 1]);
-                        else __stcs(reinterpret_cast<uint2*>(overlay + base + r * pitch + 8 * i), make_uint2(w[r][2 * i], w[r][2 * i + 1]));
-                    }
-                    continue;
-                }
-                uint32_t o[6];
-#pragma unroll
-                for (int i = 0; i < 6; ++i) o[i] = w[r][i];
-                {
-#pragma unroll
-                    for (int b = 0; b < 2; ++b) {
-                        const uint32_t m = hi[r] >> (4 * b);
-                        if (m & 1u) { o[3 * b] = (o[3 * b] & 0xff000000u) | 0x00ff0000u; }
-                        if (m & 2u) { o[3 * b] &= 0x00ffffffu; o[3 * b + 1] = (o[3 * b + 1] & 0xffff0000u) | 0x0000ff00u; }
-                        if (m & 4u) { o[3 * b + 1] &= 0x0000ffffu; o[3 * b + 2] = (o[3 * b + 2] & 0xffffff00u) | 0x000000ffu; }
-                        if (m & 8u) { o[3 * b + 2] = (o[3 * b + 2] & 0x000000ffu) | 0xff000000u; }
-                    }
-                }
-#pragma unroll
-                for (int i = 0; i < 3; ++i) {
-                    if (TMA_STORE) sts64(wst + r * K4_ROW_BYTES + 8 * i, o[2 * i], o[2 * i + 1]);
-                    else __stcs(reinterpret_cast<uint2*>(overlay + base + r * pitch + 8 * i), make_uint2(o[2 * i], o[2 * i + 1]));
-                }
-            }
-        }
-        n_motion = __popc(hi[0]) + __popc(hi[1]) + __popc(hi[2]) + __popc(hi[3]);
-        // ---- compressed: per 4x4 block ----
-#pragma unroll
-        for (int b = 0; b < 2; ++b) {
-            const bool is_static = ((nz >> (4 * b)) & 0xfu) == 0u;
-            n_static += is_static ? 1u : 0u;
-            if (!compressed) continue;
-            if (is_static) {
-                float v[4][4];
-#pragma unroll
-                for (int r = 0; r < 4; ++r) luma_row4<DP4A>(w[r][3 * b], w[r][3 * b + 1], w[r][3 * b + 2], v[r]);
-                fwd_dct_block(v);
-                const float tie = quantise_block_fast(v, qc);
-                if (!qc.fast || tie > qc.tie_lo) {       // rare (~1e-4 of blocks): near-tie on an irrational coefficient
-#pragma unroll
-                    for (int r = 0; r < 4; ++r) luma_row4<DP4A>(w[r][3 * b], w[r][3 * b + 1], w[r][3 * b + 2], v[r]);
-                    fwd_dct_block(v);
-                    quantise_block_exact(v, qc);
-                }
-                inv_dct_block(v);
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-                    const uint32_t y0 = out_byte_bits(v[r][0]), y1 = out_byte_bits(v[r][1]);
-                    const uint32_t y2 = out_byte_bits(v[r][2]), y3 = out_byte_bits(v[r][3]);
-                    w[r][3 * b] = __byte_perm(y0, y1, 0x4000);          // y0 y0 y0 y1
-                    w[r][3 * b + 1] = __byte_perm(y1, y2, 0x4400);      // y1 y1 y2 y2
-                    w[r][3 * b + 2] = __byte_perm(y2, y3, 0x4440);      // y2 y3 y3 y3
-                }
-            } else {
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-                    uint32_t o[3] = {0, 0, 0};
-#pragma unroll
-                    for (int p = 0; p < 4; ++p) {
-                        const int i = 12 * b + 3 * p;
-                        int bb = byte_at(w[r], i), gg = byte_at(w[r], i + 1), rr = byte_at(w[r], i + 2);
-                        ycc_roundtrip(bb, gg, rr);
-                        const int j = 3 * p;
-                        o[j >> 2] |= (uint32_t)bb << ((j & 3) * 8);
-                        o[(j + 1) >> 2] |= (uint32_t)gg << (((j + 1) & 3) * 8);
-                        o[(j + 2) >> 2] |= (uint32_t)rr << (((j + 2) & 3) * 8);
-                    }
-                    w[r][3 * b] = o[0]; w[r][3 * b + 1] = o[1]; w[r][3 * b + 2] = o[2];
-                }
-            }
-        }
-        if (compressed) {
-#pragma unroll
-            for (int r = 0; r < 4; ++r)
-#pragma unroll
-                for (int i = 0; i < 3; ++i) {
-                    if (TMA_STORE) sts64(wst + (4 + r) * K4_ROW_BYTES + 8 * i, w[r][2 * i], w[r][2 * i + 1]);
-                    else __stcs(reinterpret_cast<uint2*>(compressed + base + r * pitch + 8 * i), make_uint2(w[r][2 * i], w[r][2 * i + 1]));
-                }
-        }
-    }
-    if (TMA_STORE) {
-        // generic-proxy writes to shared memory -> visible to the async proxy, then one thread issues the bulk stores:
-        // the CTA's 256 groups are contiguous in a row (6 KB per row and output); a CTA that crosses the end of a block
-        // row issues two parts.  Few large bulk operations keep the TMA unit's issue rate off the critical path.
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncthreads();
-        const int g0 = blockIdx.x * blockDim.x;                 // first group of this CTA
-        if (threadIdx.x == 0) {
-            const int total = gpr * nbr;
-            const size_t pitch = (size_t)W * 3;
-            const size_t fo = (size_t)blockIdx.y * H * W * 3;
-            const uint32_t sbase = wst;                          // thread 0: start of the staging area
-            const int g_end = min(g0 + (int)blockDim.x, total);
-            for (int g = g0; g < g_end;) {                       // one part per block row the CTA touches
-                const int brp = g / gpr, gxp = g - brp * gpr;
-                const int np = min(gpr - gxp, g_end - g);
-                const size_t seg = fo + ((size_t)(brp * 4) * W + (size_t)gxp * 8) * 3;
-                const uint32_t soff = (uint32_t)(g - g0) * 24u;
-#pragma unroll
-                for (int o = 0; o < 2; ++o) {
-                    uint8_t* dst = o == 0 ? overlay : compressed;
-                    if (!dst) continue;
-#pragma unroll
-                    for (int r = 0; r < 4; ++r)
-                        bulk_store(dst + seg + r * pitch, sbase + (o * 4 + r) * K4_ROW_BYTES + soff, (uint32_t)np * 24u);
-                }
-                g += np;
-            }
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");      // shared memory must outlive the reads
-        }
-    }
-    // ---- statistics: warp shuffle reduction, one atomic pair per warp ----
-    if (counters) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            n_motion += __shfl_xor_sync(0xffffffffu, n_motion, o);
-            n_static += __shfl_xor_sync(0xffffffffu, n_static, o);
-        }
-        if ((threadIdx.x & 31) == 0) {
-            if (n_motion) atomicAdd(&counters->motion_pixels, (unsigned long long)n_motion);
-            if (n_static) atomicAdd(&counters->static_blocks, (unsigned long long)n_static);
-        }
-    }
-}
-
 // ------------------------------------------------------------------------------------------------
 // General path: block_size 4 or 8, any W, H that are multiples of block_size, both flavours.
-// One thread per block, bytewise access.  Used for block_size 8 (frame_differencing.py:203 main
-// config), for the MCO flavour (motion_compression_opt.py:152-183) and for widths the fast path
-// cannot take.  8x8 blocks use the exact restatement of cv2's 2-D routine in k_dct8.cuh.
+// One thread per block, bytewise access, IEEE division in the quantiser: exact for every q and any
+// pointer alignment.  The fallback of the packed kernels (k_degrade4p.cuh) for W % 8 != 0, q outside
+// [0.01, 1e6] and pointers that are not 8-byte aligned.  8x8 blocks use the exact restatement of cv2's
+// 2-D routine in k_dct8.cuh.
 // ------------------------------------------------------------------------------------------------
 template <int BS>
 DEVI void degrade_plane(float (&v)[BS][BS], float q) {

@@ -1,7 +1,6 @@
-// K4, packed-pair version (the default for block_size 4): same contract as k_degrade4 in k_degrade.cuh
-// (frame_differencing.py:110-111,115-130), restructured around two facts measured in profiles/r1f:
-// the kernel was issue-bound (70 % issue-slot utilisation, 860 warp instructions per 4x4 block), not
-// HBM-bound.
+// K4 for block_size 4 (frame_differencing.py:110-111,115-130; arithmetic contract in k_degrade.cuh) and the 8x8 kernel.
+// The arithmetic is built around what profiles/r1f measured on the first, scalar K4: it was issue-bound (70 % issue-slot
+// utilisation, 860 warp instructions per 4x4 block), not HBM-bound.
 //
 //  * Blackwell's packed fp32 pipe (FADD2 / FMUL2 / FFMA2, PTX add/mul/fma.rn.f32x2) processes two IEEE
 //    binary32 lanes per instruction with the same per-lane rounding as the scalar instructions.  A thread
@@ -12,7 +11,9 @@
 //    which is the correctly rounded quotient (Markstein 1990, Thm. 8; re-checked for this value range against the
 //    hardware division on 3e9 samples, tests/test_oracle_vs_cv2.py::test_markstein_quotient for a sample).  Then
 //    rint() is the usual magic-number add/sub.  No tie detection, no slow path, no second evaluation: the
-//    quantiser is six packed instructions per coefficient pair.
+//    quantiser is six packed instructions per coefficient pair.  The host takes this path for q in [0.01, 1e6],
+//    where the step is exact and |d / q| < 2^22 keeps the magic-number rounding valid; other levels go to
+//    k_degrade_generic.
 //  * luma: Y << 14 = 1868 B + 9617 G + 4899 R + 8192 as two IDP.2A (u16 x u8 pairs) per pixel instead of
 //    three-to-four IDP.4A + shift-add, and (s >> 14) | 0x4B000000 (the 2^23 + Y float pattern) is one funnel
 //    shift.
@@ -27,7 +28,8 @@ struct QuantP {
     float o[3];      // q * 2^-NE: output scale with the inverse butterflies' x0.5 pre-applied
 };
 
-// forward / inverse 4-point DCT with the power-of-two scalings folded out (see dct4_fwd_ns / dct4_inv_ps)
+// forward / inverse 4-point DCT without the x0.5 of outputs 0 and 2 / inputs 0 and 2: those power-of-two scalings are
+// folded into QuantP
 template <typename T>
 DEVI void dct4_fwd_t(T& x0, T& x1, T& x2, T& x3) {
     const T c1 = splat<T>(DVC_C1), c3 = splat<T>(DVC_C3), nc1 = splat<T>(-DVC_C1);
@@ -180,16 +182,14 @@ DEVI void k4_blocks(uint32_t (&w)[4][6], bool st_a, bool st_b, const QuantP& qp)
     }
 }
 
-template <bool TMA_STORE>
+// One thread per pair of 4x4 blocks (8 px x 4 rows, 8-byte loads and stores: pointers must be 8-byte aligned).  The fallback
+// for shapes and pointers the ring kernel below cannot take.
 __global__ void __launch_bounds__(256, 4)
 k_degrade4p(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ over127,
             const uint32_t* __restrict__ nonzero, uint8_t* __restrict__ compressed, uint8_t* __restrict__ overlay,
             int H, int W, int wpr, QuantP qp, Counters* __restrict__ counters) {
-    extern __shared__ __align__(128) uint8_t k4_stage[];
     const int gpr = W >> 3, nbr = H >> 2;
     const int gid = blockIdx.x * blockDim.x + threadIdx.x;
-    // CTA staging area as a shared-window address: row r of output o sits at (o * 4 + r) * K4_ROW_BYTES, thread t at 24 t
-    const uint32_t wst = (uint32_t)__cvta_generic_to_shared(k4_stage) + threadIdx.x * 24;
     unsigned n_motion = 0, n_static = 0;
     if (gid < gpr * nbr) {
         const int br = gid / gpr, gx = gid - br * gpr;
@@ -230,10 +230,8 @@ k_degrade4p(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
                     }
                 }
 #pragma unroll
-                for (int i = 0; i < 3; ++i) {
-                    if (TMA_STORE) sts64(wst + r * K4_ROW_BYTES + 8 * i, o[2 * i], o[2 * i + 1]);
-                    else __stcs(reinterpret_cast<uint2*>(overlay + base + r * pitch + 8 * i), make_uint2(o[2 * i], o[2 * i + 1]));
-                }
+                for (int i = 0; i < 3; ++i)
+                    __stcs(reinterpret_cast<uint2*>(overlay + base + r * pitch + 8 * i), make_uint2(o[2 * i], o[2 * i + 1]));
             }
         }
         n_motion = __popc(hi[0]) + __popc(hi[1]) + __popc(hi[2]) + __popc(hi[3]);
@@ -244,42 +242,8 @@ k_degrade4p(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
 #pragma unroll
             for (int r = 0; r < 4; ++r)
 #pragma unroll
-                for (int i = 0; i < 3; ++i) {
-                    if (TMA_STORE) sts64(wst + (4 + r) * K4_ROW_BYTES + 8 * i, w[r][2 * i], w[r][2 * i + 1]);
-                    else __stcs(reinterpret_cast<uint2*>(compressed + base + r * pitch + 8 * i), make_uint2(w[r][2 * i], w[r][2 * i + 1]));
-                }
-        }
-    }
-    if (TMA_STORE) {
-        // generic-proxy writes to shared memory -> visible to the async proxy, then one thread issues the bulk stores:
-        // the CTA's 256 groups are contiguous in a row (6 KB per row and output); a CTA that crosses the end of a block
-        // row issues two parts.
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncthreads();
-        const int g0 = blockIdx.x * blockDim.x;                 // first group of this CTA
-        if (threadIdx.x == 0) {
-            const int total = gpr * nbr;
-            const size_t pitch = (size_t)W * 3;
-            const size_t fo = (size_t)blockIdx.y * H * W * 3;
-            const uint32_t sbase = wst;                          // thread 0: start of the staging area
-            const int g_end = min(g0 + (int)blockDim.x, total);
-            for (int g = g0; g < g_end;) {                       // one part per block row the CTA touches
-                const int brp = g / gpr, gxp = g - brp * gpr;
-                const int np = min(gpr - gxp, g_end - g);
-                const size_t seg = fo + ((size_t)(brp * 4) * W + (size_t)gxp * 8) * 3;
-                const uint32_t soff = (uint32_t)(g - g0) * 24u;
-#pragma unroll
-                for (int o = 0; o < 2; ++o) {
-                    uint8_t* dst = o == 0 ? overlay : compressed;
-                    if (!dst) continue;
-#pragma unroll
-                    for (int r = 0; r < 4; ++r)
-                        bulk_store(dst + seg + r * pitch, sbase + (o * 4 + r) * K4_ROW_BYTES + soff, (uint32_t)np * 24u);
-                }
-                g += np;
-            }
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");      // shared memory must outlive the reads
+                for (int i = 0; i < 3; ++i)
+                    __stcs(reinterpret_cast<uint2*>(compressed + base + r * pitch + 8 * i), make_uint2(w[r][2 * i], w[r][2 * i + 1]));
         }
     }
     // ---- statistics: warp shuffle reduction, one atomic pair per warp ----
@@ -296,7 +260,9 @@ k_degrade4p(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
     }
 }
 
-
+DEVI void sts64(uint32_t saddr, uint32_t a, uint32_t b) {
+    asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(saddr), "r"(a), "r"(b) : "memory");
+}
 DEVI void lds64(uint32_t saddr, uint32_t& a, uint32_t& b) {
     asm volatile("ld.shared.v2.b32 {%0, %1}, [%2];" : "=r"(a), "=r"(b) : "r"(saddr));
 }
@@ -308,6 +274,10 @@ DEVI uint32_t lds_u8(uint32_t saddr) {
 DEVI void bulk_load(uint32_t sdst, const void* gsrc, uint32_t bytes, uint32_t bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(sdst), "l"(gsrc), "r"(bytes), "r"(bar) : "memory");
+}
+
+DEVI void bulk_store(const void* gdst, uint32_t ssrc, uint32_t bytes) {
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(ssrc), "r"(bytes) : "memory");
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -564,39 +534,39 @@ struct K4Geom {
     int sp;          // shared-memory row pitch in bytes (= W * 3 when parts == 1, gp * 24 otherwise)
     int span_bytes;  // bytes of one span buffer
     int mask_bytes;  // bytes of one mask-plane row group buffer (4 * nb rows of wpr words)
-    int debug;       // measurement switches (DVC_K4_DEBUG): 1 = no stores, 2 = no block arithmetic; 0 in production
 };
 
 // ------------------------------------------------------------------------------------------------
-// Persistent, warp-specialised version (the default): one CTA per SM walks tiles t = blockIdx.x, blockIdx.x +
-// gridDim.x, ... over all frames of the launch.  A tile is the K4Geom span (whole block rows, or part of one for
-// W > 2048).
-//   loader warp (last warp)    waits for "free[s]", then cp.async.bulk loads of span + mask rows into stage s of a
-//                              ring of `stages` input buffers, completing on "full[s]" (mbarrier expect_tx).  Its
-//                              per-tile instruction chain is a barrier wait and a handful of copies, nothing else.
-//   G consumer groups of 256   wait for "full", LDS.64 their 8 px x 4 rows, paint the overlay in place in the
-//   threads                    input buffer, run k4_blocks, STS.64 the compressed pixels into the group's output
-//                              buffer, fence.proxy.async, group barrier; then the group's 8 issuer lanes send the
-//                              tile out with cp.async.bulk stores (overlay from the input stage, compressed from
-//                              the output buffer) and, one tile later, after cp.async.bulk.wait_group.read, hand
-//                              the stage back to the loader ("free") and the output buffer back to the group.
-// Copies can be cut into pieces (piece_bytes, dealt out over the loader's lanes / the issuer lanes); measured from
-// 1.4 KB to the whole 23 KB span without a gain, so the default is one bulk operation per span (profiles/README.md, r1l).
-// Shared memory: `stages` x (span + 2 mask row groups) + G x span (6 x 25 KB + 2 x 23 KB at 1080p).
+// Persistent, warp-specialised K4 (block_size 4): one CTA per SM walks tiles t = blockIdx.x, blockIdx.x + gridDim.x, ...
+// over all frames of the launch.  A tile is the K4Geom span (whole block rows, or part of one for W > 2048).
+//   loader (lane 0 of the       waits for "free[s]", then cp.async.bulk loads of span + mask rows into stage s of a
+//   last warp)                  ring of `stages` input buffers, completing on "full[s]" (mbarrier expect_tx).  Its
+//                               per-tile instruction chain is a barrier wait and a handful of copies, nothing else.
+//   2 consumer groups of 256    wait for "full", LDS.64 their 8 px x 4 rows, paint the overlay in place in the
+//   threads                     input buffer, run k4_blocks, STS.64 the compressed pixels into the group's output
+//                               buffer, fence.proxy.async, group barrier; then the group's two issuer lanes send the
+//                               tile out with cp.async.bulk stores (lane 0 the overlay from the input stage, lane 1
+//                               the compressed pixels from the output buffer) and, one tile later, after
+//                               cp.async.bulk.wait_group.read, hand the stage back to the loader ("free") and the
+//                               output buffer back to the group.
+// A contiguous span is at most 256 pixel groups x 96 B = 24 KB and moves as one bulk operation per buffer (smaller pieces
+// were measured from 1.4 KB up without a gain: profiles/README.md, r1l); a part of a block row moves as its four rows.
+// Shared memory: `stages` x (span + 2 mask row groups) + 2 x span (6 x 25 KB + 2 x 23 KB at 1080p).
 // HBM sees a steady stream of bulk operations whose depth is `stages`, independent of CTA launch / drain behaviour;
 // consumers never touch global memory (statistics: one atomic pair per warp per launch).
 // ------------------------------------------------------------------------------------------------
 struct K4SGeom {
     K4Geom g;
-    int stages;            // input ring depth (multiple of the number of consumer groups)
+    int stages;            // input ring depth (more than K4S_GROUPS)
     int tiles_per_frame;
     int n_tiles;           // tiles_per_frame * frames
     int stage_bytes;       // span_bytes + 2 * mask_bytes, rounded up to 128
     int ybuf_bytes;        // span_bytes rounded up to 128
-    int piece_bytes;       // bulk-copy granularity inside a contiguous span (multiple of 16)
 };
 
-constexpr int K4S_ISSUERS = 8;          // lanes 0..7 of a consumer group's first warp issue its stores
+constexpr int K4S_GROUPS = 2;                               // consumer groups of 256 threads
+constexpr int K4S_THREADS = K4S_GROUPS * 256 + 32;          // + the loader warp
+constexpr int K4S_ISSUERS = 2;                              // lanes 0 and 1 of a consumer group issue its stores
 
 DEVI void mbar_wait(uint32_t bar, uint32_t parity) {
     uint32_t done = 0;
@@ -628,8 +598,7 @@ DEVI K4Tile k4_tile(const K4Walk& wk, const K4Geom& g, int H, int W, int wpr) {
     return r;
 }
 
-template <int G, int MINB>
-__global__ void __launch_bounds__(32 + G * 256, MINB)
+__global__ void __launch_bounds__(K4S_THREADS, 1)
 k_degrade4s(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ over127,
             const uint32_t* __restrict__ nonzero, uint8_t* __restrict__ compressed, uint8_t* __restrict__ overlay,
             int H, int W, int wpr, QuantP qp, Counters* __restrict__ counters, K4SGeom sg) {
@@ -637,16 +606,15 @@ k_degrade4s(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
     const K4Geom& g = sg.g;
     const uint32_t s0 = (uint32_t)__cvta_generic_to_shared(k4_smem);
     const int S = sg.stages;
-    const uint32_t ybufs = s0 + (uint32_t)S * (uint32_t)sg.stage_bytes;     // G output buffers
-    const uint32_t bars = ybufs + (uint32_t)G * (uint32_t)sg.ybuf_bytes;    // full[S], free[S]
-    const uint32_t desc = (bars + 8u * (uint32_t)(2 * S) + 15u) & ~15u;     // per stage: {nbv, g0, ng, -}
+    const uint32_t ybufs = s0 + (uint32_t)S * (uint32_t)sg.stage_bytes;              // K4S_GROUPS output buffers
+    const uint32_t bars = ybufs + (uint32_t)K4S_GROUPS * (uint32_t)sg.ybuf_bytes;    // full[S], free[S]
+    const uint32_t desc = (bars + 8u * (uint32_t)(2 * S) + 15u) & ~15u;              // per stage: {nbv, g0, ng, -}
     const int tid = threadIdx.x;
     const int first = blockIdx.x, stride = gridDim.x;
     const int nj = first < sg.n_tiles ? (sg.n_tiles - first + stride - 1) / stride : 0;
     const uint32_t pitch = (uint32_t)W * 3u;
     const uint32_t mrow_bytes = (uint32_t)wpr * 4u;
     const bool contiguous = g.parts == 1;
-    const uint32_t piece = (uint32_t)sg.piece_bytes;
 
     if (tid == 0) {
         for (int s = 0; s < S; ++s) {
@@ -657,9 +625,9 @@ k_degrade4s(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
     }
     __syncthreads();
 
-    if (tid >= G * 256) {
-        // ------------------------------ loader warp ------------------------------
-        const int lane = tid - G * 256;
+    if (tid >= K4S_GROUPS * 256) {
+        // ------------------------------ loader ------------------------------
+        if (tid > K4S_GROUPS * 256) return;
         K4Walk wl;
         wl.init(first, stride, sg.tiles_per_frame);
         for (int j = 0; j < nj; ++j) {
@@ -673,19 +641,13 @@ k_degrade4s(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
             const uint32_t rows = contiguous ? (uint32_t)(4 * t.nbv) : 4u;
             const uint32_t rbytes = contiguous ? pitch : (uint32_t)t.ng * 24u;
             if (j >= S) mbar_wait(bars + 8u * (S + s), (uint32_t)(j / S - 1) & 1u);       // the stage's previous tile has left
-            if (lane == 0) {
-                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(desc + 16u * s), "r"(t.nbv), "r"(t.g0), "r"(t.ng), "r"(0) : "memory");
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "r"(rows * rbytes + 2u * mbytes) : "memory");
-            }
-            if (contiguous) {
-                const uint32_t total = rows * rbytes;
-                for (uint32_t off = (uint32_t)lane * piece; off < total; off += 32u * piece)
-                    bulk_load(sX + off, frames + t.span_off + off, min(piece, total - off), full);
-            } else {
-                for (uint32_t r = lane; r < rows; r += 32) bulk_load(sX + r * g.sp, frames + t.span_off + (size_t)r * pitch, rbytes, full);
-            }
-            if (lane == 30) bulk_load(sMh, over127 + t.mask_off, mbytes, full);
-            if (lane == 31) bulk_load(sMn, nonzero + t.mask_off, mbytes, full);
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(desc + 16u * s), "r"(t.nbv), "r"(t.g0), "r"(t.ng), "r"(0) : "memory");
+            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "r"(rows * rbytes + 2u * mbytes) : "memory");
+            if (contiguous) bulk_load(sX, frames + t.span_off, rows * rbytes, full);
+            else
+                for (uint32_t r = 0; r < rows; ++r) bulk_load(sX + r * g.sp, frames + t.span_off + (size_t)r * pitch, rbytes, full);
+            bulk_load(sMh, over127 + t.mask_off, mbytes, full);
+            bulk_load(sMn, nonzero + t.mask_off, mbytes, full);
         }
         return;
     }
@@ -700,9 +662,9 @@ k_degrade4s(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
     const uint32_t sY = ybufs + (uint32_t)grp * (uint32_t)sg.ybuf_bytes;
     unsigned n_motion = 0, n_static = 0;
     K4Walk ws;                              // this group's tiles, for the store addresses
-    ws.init(first + grp * stride, G * stride, sg.tiles_per_frame);
+    ws.init(first + grp * stride, K4S_GROUPS * stride, sg.tiles_per_frame);
     int s_prev = -1;
-    for (int j = grp; j < nj; j += G) {
+    for (int j = grp; j < nj; j += K4S_GROUPS) {
         const int s = j % S;
         const uint32_t sX = s0 + (uint32_t)s * (uint32_t)sg.stage_bytes;
         const uint32_t sMh = sX + g.span_bytes, sMn = sMh + g.mask_bytes;
@@ -745,7 +707,7 @@ k_degrade4s(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
             n_motion += __popc(hi[0]) + __popc(hi[1]) + __popc(hi[2]) + __popc(hi[3]);
             const bool st_a = (nz & 0xfu) == 0u, st_b = (nz >> 4) == 0u;
             n_static += (st_a ? 1u : 0u) + (st_b ? 1u : 0u);
-            if (compressed && !(g.debug & 2)) k4_blocks(w, st_a, st_b, qp);
+            if (compressed) k4_blocks(w, st_a, st_b, qp);
         }
         // the previous tile's stores have read their shared-memory sources: its input stage goes back to the loader,
         // the output buffer back to the group
@@ -763,25 +725,15 @@ k_degrade4s(const uint8_t* __restrict__ frames, const uint32_t* __restrict__ ove
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         group_sync(1 + grp);
         if (issuer) {
-            if (!(g.debug & 1)) {
+            uint8_t* dst = t == 0 ? overlay : compressed;
+            if (dst) {
                 const K4Tile tl = k4_tile(ws, g, H, W, wpr);
-                const uint32_t rows = contiguous ? 4u * nbv : 4u;
-                const uint32_t rbytes = contiguous ? pitch : tng * 24u;
-                const uint32_t np = contiguous ? (rows * rbytes + piece - 1) / piece : rows;       // pieces per output
-                for (uint32_t i = (uint32_t)t; i < 2u * np; i += K4S_ISSUERS) {
-                    const uint32_t o = i >= np ? 1u : 0u, k = i - o * np;
-                    uint8_t* dst = o == 0 ? overlay : compressed;
-                    if (!dst) continue;
-                    const uint32_t src = o == 0 ? sX : sY;
-                    if (contiguous) {
-                        const uint32_t off = k * piece;
-                        bulk_store(dst + tl.span_off + off, src + off, min(piece, rows * rbytes - off));
-                    } else {
-                        bulk_store(dst + tl.span_off + (size_t)k * pitch, src + k * g.sp, rbytes);
-                    }
-                }
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                const uint32_t src = t == 0 ? sX : sY;
+                if (contiguous) bulk_store(dst + tl.span_off, src, 4u * nbv * pitch);
+                else
+                    for (uint32_t r = 0; r < 4; ++r) bulk_store(dst + tl.span_off + (size_t)r * pitch, src + r * g.sp, tng * 24u);
             }
+            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
             s_prev = s;
         }
         ws.next();

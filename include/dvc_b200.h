@@ -130,7 +130,8 @@ int dvc_reset_counters(dvc_handle* h);
  * overlay_dev  [n][H][W][3]  what mask_out.write() receives (:110-112), may be NULL
  * compressed_dev [n][H][W][3] what final_out.write() receives (:115-131), may be NULL
  * mask_dev     [n][H][W]     accumulated_mask after each frame (FD) / final mask (WINDOW), may be NULL
- * n_frames <= cfg.max_batch. */
+ * n_frames <= cfg.max_batch.  When W % 16 == 0, frames_dev must be 16-byte aligned: the front kernels load it
+ * 16 bytes at a time. */
 int dvc_process_batch(dvc_handle* h, const uint8_t* frames_dev, int32_t n_frames, uint8_t* overlay_dev,
                       uint8_t* compressed_dev, uint8_t* mask_dev, void* stream);
 /* Software pipelining across batches (off by default).  When on, dvc_process_batch runs the mask kernels and the
@@ -205,7 +206,8 @@ int dvc_mask_rectangles_u8(const uint8_t* src_dev, uint8_t* dst_dev, int32_t n, 
 /* overlay paint + colour round trip + block-DCT degrade, frame_differencing.py:110-111,115-130
  * (flavour FD) or motion_compression_opt.py:152-183 (flavour MCO).  mask_dev [n][H][W] is
  * accumulated_mask (any uint8 values).  Either output may be NULL.  counters_dev (5 x uint64 in
- * dvc_counters order, accumulated atomically) may be NULL. */
+ * dvc_counters order, accumulated atomically) may be NULL.  bgr_dev, compressed_dev and overlay_dev may have
+ * any alignment; 16-byte aligned pointers take the fastest kernels. */
 int dvc_degrade_blend_u8(const uint8_t* bgr_dev, const uint8_t* mask_dev, uint8_t* compressed_dev,
                          uint8_t* overlay_dev, int32_t n, int32_t H, int32_t W, int32_t block_size,
                          float quantization_level, int32_t flavour, uint64_t* counters_dev, void* stream);

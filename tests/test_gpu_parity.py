@@ -455,10 +455,10 @@ def test_degrade_fd(P, shape, bs):
     assert c[3] == 3 * (shape[0] // bs) * (shape[1] // bs) and c[4] == n_static
 
 
-@pytest.mark.parametrize("q", [100, 100.0, 33.3, 8, 7.5, 1, 250, 0.25, 0.3, 7.3, 0.05, 1000.5])
+@pytest.mark.parametrize("q", [100, 100.0, 33.3, 8, 7.5, 1, 250, 0.25, 0.3, 7.3, 0.05, 1000.5, 0.005, 2e6])
 def test_degrade_fd_quantiser_ties_and_levels(P, q):
     """Blocks built to sit exactly on quantiser ties (d/q = n + 1/2) and a sweep of quantisation levels,
-    including levels small enough to disable the fast rounding path."""
+    including levels outside [0.01, 1e6], which the packed kernels leave to the general one."""
     if not so.cv2_dct4_matches_closed_form():
         pytest.skip("host cv2 does not follow the recovered float32 DCT sequence; covered by tolerance tests")
     r = rng(21)
@@ -493,6 +493,41 @@ def test_degrade_fd_widths_multiple_of_8(P, shape):
     for i in range(2):
         assert np.array_equal(ov[i], so.overlay_paint(frames[i], acc[i]))
         _check_degraded(comp[i], so.degrade_fd(frames[i], acc[i], 4, 100), frames[i], acc[i], 4, 100, exact)
+
+
+@pytest.mark.parametrize("offset", [1, 8, 16])
+@pytest.mark.parametrize("shape,bs", [((48, 64), 4), ((12, 2056), 4), ((48, 64), 8), ((12, 2056), 8)])
+def test_degrade_fd_any_frame_alignment(P, shape, bs, offset):
+    """Frames at byte offsets 1, 8 and 16 inside a larger allocation: kernels that need 8- or 16-byte aligned addresses
+    (8-byte vector access, the ring's bulk copies) give way to ones that do not, with the outputs and counters of the
+    aligned call."""
+    r = rng(24)
+    h, w = shape
+    frames = r.integers(0, 256, (2, h, w, 3), dtype=np.uint8)
+    acc = (r.random((2, h, w)) < 0.01).astype(np.uint8) * r.integers(1, 256, (2, h, w), dtype=np.uint8)
+    buf = torch.empty(frames.size + 16, dtype=torch.uint8, device="cuda")
+    shifted = buf[offset:offset + frames.size].view(frames.shape)
+    shifted.copy_(dev(frames))
+    assert shifted.data_ptr() % 16 == offset % 16
+    outs = []
+    for bgr in (dev(frames), shifted):
+        cnt = torch.zeros(5, dtype=torch.int64, device="cuda")
+        comp, ov = P.degrade_blend(bgr, dev(acc), bs, 100, "fd", True, cnt)
+        outs.append((host(comp), host(ov), host(cnt)))
+    for aligned, unaligned in zip(*outs):
+        assert np.array_equal(aligned, unaligned)
+    comp, ov, c = outs[1]
+    exact = _exact(bs, h, w)
+    hf, wf = (h // bs) * bs, (w // bs) * bs
+    for i in range(2):
+        ref = so.degrade_fd(frames[i], acc[i], bs, 100)
+        assert np.array_equal(ov[i], so.overlay_paint(frames[i], acc[i]))
+        if exact:
+            assert np.array_equal(comp[i], ref)
+        else:
+            _check_degraded(comp[i][:hf, :wf], ref[:hf, :wf], frames[i][:hf, :wf], acc[i][:hf, :wf], bs, 100, False)
+    assert c[2] == int((acc > 127).sum())
+    assert c[4] == sum(int(so.block_all_zero(acc[i], bs).sum()) for i in range(2))
 
 
 def test_degrade_fd_ring_wraps_many_tiles_per_cta(P):
