@@ -75,6 +75,8 @@ SYMBOLS = {
     "dvc_degrade_blend_u8": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _F, _I, _P, _P]),
     "dvc_dct_blocks_f32": (C.c_int, [_P, _P, _L, _I, _I, _I, _P]),
     "dvc_gaussian_blur_u8": (C.c_int, [_P, _P, _I, _I, _I, _I, _D, _P]),
+    "dvc_farneback_flow_f32": (C.c_int, [_P, _P, _P, _I, _I, _I, _D, _I, _I, _I, _I, _D, _I, _P]),
+    "dvc_flow_masks_u8": (C.c_int, [_P, _P, _I, _I, _I, _D, _I, _I, _I, _I, _D, _I, _F, _P]),
 }
 
 _lib = None

@@ -17,6 +17,7 @@
 #include "k_ccl_sweep.cuh"
 #include "k_degrade.cuh"
 #include "k_degrade4p.cuh"
+#include "k_flow.cuh"
 #include "k_front.cuh"
 #include "k_mask.cuh"
 
@@ -1601,5 +1602,246 @@ extern "C" int dvc_begin_stream_frames(dvc_handle* h, const uint8_t* first_frame
     if (h->ring) CU(cudaMemsetAsync(h->ring, 0, h->plane_words * 4 * h->ring_cap * S, st));
     h->n_masks = 0;
     CU(cudaStreamSynchronize(st));
+    return DVC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Farneback flow (motion_compression_opt.py:72-83)
+// ------------------------------------------------------------------------------------------------
+struct FlowPlan {
+    int levels = 0;                       // index of the coarsest level
+    std::vector<FlowLevelGeom> geo;       // per level, 0 = full resolution
+    std::vector<size_t> off;              // pixel offset of each level inside one frame's pyramid
+    size_t P = 0;                         // pixels of all levels of one frame
+    FlowPolyTab poly;
+};
+
+// getGaussianKernel(n, sigma, CV_32F): the small fixed kernels when sigma <= 0, float taps normalised in double
+static void gauss_kernel_f32(int n, double sigma, float* half) {
+    static const float fixed[4][7] = {{1.f}, {0.25f, 0.5f, 0.25f}, {0.0625f, 0.25f, 0.375f, 0.25f, 0.0625f},
+                                      {0.03125f, 0.109375f, 0.21875f, 0.28125f, 0.21875f, 0.109375f, 0.03125f}};
+    const bool use_fixed = n % 2 == 1 && n <= 7 && sigma <= 0;
+    const double sx = sigma > 0 ? sigma : ((n - 1) * 0.5 - 1) * 0.3 + 0.8;
+    const double scale2x = -0.5 / (sx * sx);
+    std::vector<float> c(n);
+    double sum = 0;
+    for (int i = 0; i < n; ++i) {
+        const double x = i - (n - 1) * 0.5;
+        c[i] = (float)(use_fixed ? (double)fixed[n / 2][i] : std::exp(scale2x * x * x));
+        sum += c[i];
+    }
+    sum = 1. / sum;
+    for (int i = n / 2; i < n; ++i) half[i - n / 2] = (float)(c[i] * sum);
+}
+
+// FarnebackPrepareGaussian: float taps, the 6 x 6 Gram matrix in double and four entries of its inverse
+static void flow_poly_tab(int n, double sigma, FlowPolyTab& t) {
+    if (sigma < 1.1920928955078125e-07) sigma = n * 0.3;
+    float g[2 * FLOW_MAX_POLY_N + 1];
+    double s = 0;
+    for (int x = -n; x <= n; ++x) { g[x + n] = (float)std::exp(-x * x / (2 * sigma * sigma)); s += g[x + n]; }
+    s = 1. / s;
+    for (int x = -n; x <= n; ++x) g[x + n] = (float)(g[x + n] * s);
+    t.n = n;
+    for (int k = 0; k <= n; ++k) { t.g[k] = g[k + n]; t.xg[k] = (float)k * g[k + n]; t.xxg[k] = (float)(k * k) * g[k + n]; }
+    double G[6][12] = {};
+    for (int y = -n; y <= n; ++y)
+        for (int x = -n; x <= n; ++x) {
+            const float gy = g[y + n], gx = g[x + n], fx = (float)x, fy = (float)y;
+            G[0][0] += gy * gx;
+            G[1][1] += gy * gx * fx * fx;
+            G[3][3] += gy * gx * fx * fx * fx * fx;
+            G[5][5] += gy * gx * fx * fx * fy * fy;
+        }
+    G[2][2] = G[0][3] = G[0][4] = G[3][0] = G[4][0] = G[1][1];
+    G[4][4] = G[3][3];
+    G[3][4] = G[4][3] = G[5][5];
+    for (int i = 0; i < 6; ++i) G[i][6 + i] = 1.0;
+    for (int c = 0; c < 6; ++c) {                         // Gauss-Jordan with partial pivoting (G is positive definite)
+        int piv = c;
+        for (int r = c + 1; r < 6; ++r) if (std::fabs(G[r][c]) > std::fabs(G[piv][c])) piv = r;
+        for (int j = 0; j < 12; ++j) std::swap(G[c][j], G[piv][j]);
+        const double d = G[c][c];
+        for (int j = 0; j < 12; ++j) G[c][j] /= d;
+        for (int r = 0; r < 6; ++r)
+            if (r != c && G[r][c] != 0.0) {
+                const double f = G[r][c];
+                for (int j = 0; j < 12; ++j) G[r][j] -= f * G[c][j];
+            }
+    }
+    t.ig11 = G[1][7]; t.ig03 = G[0][9]; t.ig33 = G[3][9]; t.ig55 = G[5][11];
+}
+
+static int cv_round(double v) { return (int)std::lrint(v); }
+
+// Argument rules of both entry points, then the pyramid: cv2 stops adding levels once a side drops below 32 pixels.
+static int flow_plan(const char* who, int n, int H, int W, double pyr_scale, int levels, int winsize, int iterations, int poly_n,
+                     double poly_sigma, int flags, FlowPlan& pl) {
+    if (n < 0 || H < 1 || W < 1) return set_err(nullptr, DVC_ERR_INVALID, "%s: bad dimensions n=%d H=%d W=%d", who, n, H, W);
+    if (!(pyr_scale > 0 && pyr_scale < 1)) return set_err(nullptr, DVC_ERR_INVALID, "%s: pyr_scale %g outside (0, 1)", who, pyr_scale);
+    if (levels < 0 || winsize < 1 || iterations < 1)
+        return set_err(nullptr, DVC_ERR_INVALID, "%s: levels %d, winsize %d, iterations %d: need levels >= 0, winsize >= 1, iterations >= 1",
+                       who, levels, winsize, iterations);
+    if (!(poly_sigma >= 0) || !(poly_sigma < 1e6)) return set_err(nullptr, DVC_ERR_INVALID, "%s: poly_sigma %g", who, poly_sigma);
+    if (poly_n != 5 && poly_n != 7) return set_err(nullptr, DVC_ERR_UNSUPPORTED, "%s: poly_n %d: the GPU path implements 5 and 7", who, poly_n);
+    if (flags != 0)
+        return set_err(nullptr, DVC_ERR_UNSUPPORTED, "%s: flags %d: OPTFLOW_USE_INITIAL_FLOW and OPTFLOW_FARNEBACK_GAUSSIAN are not implemented", who, flags);
+    if (H > 32767 || W > 32767) return set_err(nullptr, DVC_ERR_UNSUPPORTED, "%s: image larger than 32767", who);
+    if (winsize > 32767) return set_err(nullptr, DVC_ERR_UNSUPPORTED, "%s: winsize %d larger than 32767", who, winsize);
+    double scale = 1;
+    int k = 0;
+    for (; k < levels; ++k) {
+        scale *= pyr_scale;
+        if (W * scale < 32 || H * scale < 32) break;
+        if (k == 64) return set_err(nullptr, DVC_ERR_UNSUPPORTED, "%s: more than 64 pyramid levels", who);
+    }
+    pl.levels = k;
+    pl.geo.assign(k + 1, FlowLevelGeom());
+    pl.off.assign(k + 1, 0);
+    pl.P = 0;
+    for (int l = 0; l <= k; ++l) {
+        double s = 1;
+        for (int i = 0; i < l; ++i) s *= pyr_scale;
+        const double sigma = (1. / s - 1) * 0.5;
+        const int ks = std::max(cv_round(sigma * 5) | 1, 3);
+        if (ks / 2 > FLOW_MAX_BLUR_HALF)
+            return set_err(nullptr, DVC_ERR_UNSUPPORTED, "%s: level %d needs a %d-tap Gaussian, more than %d", who, l, ks, 2 * FLOW_MAX_BLUR_HALF + 1);
+        FlowLevelGeom& g = pl.geo[l];
+        gauss_kernel_f32(ks, sigma, g.k);
+        g.half = ks / 2;
+        g.w = cv_round(W * s);
+        g.h = cv_round(H * s);
+        g.scale_x = 1. / ((double)g.w / W);
+        g.scale_y = 1. / ((double)g.h / H);
+        pl.off[l] = pl.P;
+        pl.P += (size_t)g.w * g.h;
+    }
+    flow_poly_tab(poly_n, poly_sigma, pl.poly);
+    return DVC_OK;
+}
+
+// frames [F][H][W] -> their pyramids of polynomial coefficients, R [F][P][5]
+static int flow_pyramids(const uint8_t* src, int F, int H, int W, const FlowPlan& pl, float* img, float* R, cudaStream_t st) {
+    char* ERRBUF = nullptr;
+    for (int l = 0; l <= pl.levels; ++l) {
+        const FlowLevelGeom& g = pl.geo[l];
+        k_flow_level<<<dim3(cdiv((size_t)g.w * g.h, 256), F), 256, 0, st>>>(src, H, W, img, (size_t)H * W, g);
+        k_flow_poly<<<dim3(cdiv(g.w, POLY_TW), cdiv(g.h, POLY_TH), F), 256, 0, st>>>(img, (size_t)H * W, g.w, g.h, R + pl.off[l] * 5,
+                                                                                    pl.P * 5, pl.poly);
+        CHECK_LAUNCH();
+    }
+    return DVC_OK;
+}
+
+struct FlowScratch {
+    float* img;       // [F][H][W] level image
+    float* R;         // [F][P][5]
+    float* M;         // [G][H][W][5]
+    double* V;        // [G][H][W][5] column sums
+    double* S;        // [G][H][W][5] box sums
+    float2* fl[2];    // [G][H][W] flow of the last two levels
+};
+
+// G pairs, coarse to fine.  Pair p's polynomial pyramids are R0 + p * P * 5 and R1 + p * P * 5.  The finest level's last
+// solve writes flow_out (stride H*W) or mask_out.
+static int flow_pairs(const float* R0, const float* R1, int G, int H, int W, const FlowPlan& pl, double pyr_scale, int winsize,
+                      int iterations, const FlowScratch& sc, float2* flow_out, uint8_t* mask_out, float thr, cudaStream_t st) {
+    char* ERRBUF = nullptr;
+    const size_t WH = (size_t)H * W;
+    const int m = winsize / 2;
+    const double box = 1. / ((double)winsize * winsize);
+    const float up = (float)(1. / pyr_scale);
+    const float2* coarse = nullptr;
+    int cw = 0, ch = 0, cur = 0;
+    for (int l = pl.levels; l >= 0; --l) {
+        const FlowLevelGeom& g = pl.geo[l];
+        const FlowPair pr{R0 + pl.off[l] * 5, R1 + pl.off[l] * 5, pl.P * 5, WH, g.w, g.h};
+        const dim3 gp(cdiv((size_t)g.w * g.h, 256), G);
+        k_flow_matrices<<<gp, 256, 0, st>>>(pr, coarse, cw, ch, coarse ? 1. / ((double)g.w / cw) : 0., coarse ? 1. / ((double)g.h / ch) : 0.,
+                                            up, sc.M);
+        CHECK_LAUNCH();
+        for (int it = 0; it < iterations; ++it) {
+            const bool last = it == iterations - 1;
+            float2* fo = last ? sc.fl[cur] : nullptr;
+            uint8_t* mo = nullptr;
+            if (last && l == 0) { fo = flow_out; mo = mask_out; }
+            k_flow_vsum<<<dim3(cdiv((size_t)g.w * 5, 128), G), 128, 0, st>>>(sc.M, sc.V, g.w, g.h, m, WH);
+            k_flow_hsum<<<dim3(cdiv((size_t)g.h * 5, 128), G), 128, 0, st>>>(sc.V, sc.S, g.w, g.h, m, WH);
+            k_flow_solve<<<gp, 256, 0, st>>>(pr, sc.S, box, fo, WH, mo, WH, thr, last ? nullptr : sc.M);
+            CHECK_LAUNCH();
+        }
+        coarse = sc.fl[cur];
+        cw = g.w; ch = g.h;
+        cur ^= 1;
+    }
+    return DVC_OK;
+}
+
+// Pairs per launch group: scratch for one group stays near 1 GiB.
+static int flow_group(int n, int H, int W, const FlowPlan& pl) {
+    const size_t WH = (size_t)H * W;
+    const size_t per_pair = 2 * (pl.P * 20 + WH * 4) + WH * (20 + 80 + 16);
+    return (int)std::max<size_t>(1, std::min<size_t>({(size_t)n, ((size_t)1 << 30) / per_pair, 4096}));
+}
+
+static int flow_alloc(ScopedAsyncBuf* b, int F, int G, int H, int W, const FlowPlan& pl, FlowScratch& sc) {
+    char* ERRBUF = nullptr;
+    const size_t WH = (size_t)H * W;
+    CU(b[0].alloc((size_t)F * WH * 4));
+    CU(b[1].alloc((size_t)F * pl.P * 20));
+    CU(b[2].alloc((size_t)G * WH * 20));
+    CU(b[3].alloc((size_t)G * WH * 80));
+    CU(b[4].alloc((size_t)G * WH * 16));
+    sc.img = (float*)b[0].p; sc.R = (float*)b[1].p; sc.M = (float*)b[2].p; sc.V = (double*)b[3].p; sc.S = sc.V + (size_t)G * WH * 5;
+    sc.fl[0] = (float2*)b[4].p; sc.fl[1] = sc.fl[0] + (size_t)G * WH;
+    return DVC_OK;
+}
+
+extern "C" int dvc_farneback_flow_f32(const uint8_t* prev, const uint8_t* next, float* flow, int32_t n, int32_t H, int32_t W,
+                                      double pyr_scale, int32_t levels, int32_t winsize, int32_t iterations, int32_t poly_n,
+                                      double poly_sigma, int32_t flags, void* stream) {
+    FlowPlan pl;
+    int rc = flow_plan("dvc_farneback_flow_f32", n, H, W, pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags, pl);
+    if (rc || n == 0) return rc;
+    if (!prev || !next || !flow) return set_err(nullptr, DVC_ERR_INVALID, "dvc_farneback_flow_f32: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t WH = (size_t)H * W;
+    const int G = flow_group(n, H, W, pl);
+    ScopedAsyncBuf b[5] = {ScopedAsyncBuf(st), ScopedAsyncBuf(st), ScopedAsyncBuf(st), ScopedAsyncBuf(st), ScopedAsyncBuf(st)};
+    FlowScratch sc;
+    if ((rc = flow_alloc(b, 2 * G, G, H, W, pl, sc))) return rc;
+    float* R1 = sc.R + (size_t)G * pl.P * 5;
+    for (int i0 = 0; i0 < n; i0 += G) {
+        const int g = std::min(G, n - i0);
+        if ((rc = flow_pyramids(prev + i0 * WH, g, H, W, pl, sc.img, sc.R, st))) return rc;
+        if ((rc = flow_pyramids(next + i0 * WH, g, H, W, pl, sc.img, R1, st))) return rc;
+        if ((rc = flow_pairs(sc.R, R1, g, H, W, pl, pyr_scale, winsize, iterations, sc, (float2*)flow + i0 * WH, nullptr, 0.f, st))) return rc;
+    }
+    return DVC_OK;
+}
+
+extern "C" int dvc_flow_masks_u8(const uint8_t* gray, uint8_t* mask, int32_t n, int32_t H, int32_t W, double pyr_scale, int32_t levels,
+                                 int32_t winsize, int32_t iterations, int32_t poly_n, double poly_sigma, int32_t flags,
+                                 float flow_threshold, void* stream) {
+    char* ERRBUF = nullptr;
+    FlowPlan pl;
+    int rc = flow_plan("dvc_flow_masks_u8", n, H, W, pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags, pl);
+    if (rc || n == 0) return rc;
+    if (!gray || !mask) return set_err(nullptr, DVC_ERR_INVALID, "dvc_flow_masks_u8: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t WH = (size_t)H * W, RF = pl.P * 5;
+    const int G = flow_group(n, H, W, pl);
+    ScopedAsyncBuf b[5] = {ScopedAsyncBuf(st), ScopedAsyncBuf(st), ScopedAsyncBuf(st), ScopedAsyncBuf(st), ScopedAsyncBuf(st)};
+    FlowScratch sc;
+    if ((rc = flow_alloc(b, G + 1, G, H, W, pl, sc))) return rc;
+    // frame i + 1's pyramid serves pair i and pair i + 1: the last frame of a group moves to slot 0 for the next group
+    if ((rc = flow_pyramids(gray, 1, H, W, pl, sc.img, sc.R, st))) return rc;
+    for (int i0 = 0; i0 < n; i0 += G) {
+        const int g = std::min(G, n - i0);
+        if (i0 > 0) CU(cudaMemcpyAsync(sc.R, sc.R + (size_t)G * RF, RF * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        if ((rc = flow_pyramids(gray + (i0 + 1) * WH, g, H, W, pl, sc.img, sc.R + RF, st))) return rc;
+        if ((rc = flow_pairs(sc.R, sc.R + RF, g, H, W, pl, pyr_scale, winsize, iterations, sc, nullptr, mask + i0 * WH, flow_threshold, st)))
+            return rc;
+    }
     return DVC_OK;
 }

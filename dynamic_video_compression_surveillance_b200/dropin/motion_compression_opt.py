@@ -1,7 +1,9 @@
 """Drop-in for the reference module of the same name: ``windows.py`` imports ``process_single_video_of`` from
 here (windows.py:13,151).  Contracts follow motion_compression_opt.py:8-247.  GPU (C ABI): the K-frame window
 vote (:84-86), close/open (:89-90), contours -> bounding rectangles (:93-97) and all of compress_with_motion's
-arithmetic (:152-183).  Host, as scoped by SURVEY.md section 8: Farneback flow + cartToPolar (:72-82), codecs.
+arithmetic (:152-183).  Farneback flow + cartToPolar + threshold (:71-83) run on the host by default, as in the
+reference; ``flow_device="gpu"`` moves gray conversion, flow and masks to the GPU (host_loop.flow_masks_gpu), which agrees
+with cv2 about as closely as cv2's own dispatch paths agree with each other (DESIGN.md section 6).  Codecs stay on the host.
 """
 import logging
 import os
@@ -32,8 +34,11 @@ def _open_writer(path, fps, size, color=True):
 
 
 def temporal_smoothing_flow(video_path, output_dir, flow_threshold=0.5, alpha_fraction=0.2, window_size=30, morph_kernel=2,
-                            save_name="overlay.mp4", mask_save_name="mask.mp4"):
-    """motion_compression_opt.py:29-109 -> (frames, total seconds, seconds per frame)."""
+                            save_name="overlay.mp4", mask_save_name="mask.mp4", flow_device="cpu"):
+    """motion_compression_opt.py:29-109 -> (frames, total seconds, seconds per frame).  flow_device "cpu" (default):
+    cv2 Farneback per frame on the host; "gpu": gray, flow and raw masks of each chunk on the GPU."""
+    if flow_device not in ("cpu", "gpu"):
+        raise ValueError(f"flow_device must be 'cpu' or 'gpu', not {flow_device!r}")
     t_start = time.time()
     cap = cv2.VideoCapture(video_path)
     if not cap.isOpened():
@@ -49,7 +54,8 @@ def temporal_smoothing_flow(video_path, output_dir, flow_threshold=0.5, alpha_fr
         cap.release()
         return 0, 0, 0
 
-    prev_gray = cv2.cvtColor(frame, cv2.COLOR_BGR2GRAY)
+    on_gpu = flow_device == "gpu"
+    prev_gray = _hl.first_gray_gpu(frame) if on_gpu else cv2.cvtColor(frame, cv2.COLOR_BGR2GRAY)
     n_frames, history, exhausted = 0, [], False
     while not exhausted:
         frames, raws = [], []
@@ -58,14 +64,18 @@ def temporal_smoothing_flow(video_path, output_dir, flow_threshold=0.5, alpha_fr
             if not ok:
                 exhausted = True
                 break
-            gray = cv2.cvtColor(frame, cv2.COLOR_BGR2GRAY)
-            flow = cv2.calcOpticalFlowFarneback(prev_gray, gray, None, *_FARNEBACK)      # host: out of scope
-            mag, _ = cv2.cartToPolar(flow[..., 0], flow[..., 1])
-            raws.append((mag > flow_threshold).astype(np.uint8) * 255)
+            if not on_gpu:
+                gray = cv2.cvtColor(frame, cv2.COLOR_BGR2GRAY)
+                flow = cv2.calcOpticalFlowFarneback(prev_gray, gray, None, *_FARNEBACK)
+                mag, _ = cv2.cartToPolar(flow[..., 0], flow[..., 1])
+                raws.append((mag > flow_threshold).astype(np.uint8) * 255)
+                prev_gray = gray
             frames.append(frame)
-            prev_gray = gray
         if not frames:
             break
+        if on_gpu:
+            masks, prev_gray = _hl.flow_masks_gpu(frames, prev_gray, flow_threshold, _FARNEBACK)
+            raws = list(masks)
         rects = _hl.smooth_rect_masks_gpu(raws, history, window_size, alpha_fraction, morph_kernel)
         seen = history + raws
         # while the stream is shorter than the window keep all of it (the vote's L = len(deque) must match);
@@ -123,8 +133,9 @@ def compress_with_motion(input_video, mask_video, output_dir):
     return n_frames, total, avg
 
 
-def process_single_video_of(video_path, output_dir):
-    """motion_compression_opt.py:195-247: motion detection, then compression, then execution_times.txt."""
+def process_single_video_of(video_path, output_dir, flow_device="cpu"):
+    """motion_compression_opt.py:195-247: motion detection, then compression, then execution_times.txt.  flow_device: see
+    temporal_smoothing_flow."""
     name = _hl.video_stem(video_path)
     out_dir = os.path.join(output_dir, name)
     os.makedirs(out_dir, exist_ok=True)
@@ -134,7 +145,7 @@ def process_single_video_of(video_path, output_dir):
     logging.info("Step 1/2: Starting motion detection...")
     md = _hl.StageTiming("Motion Detection", *temporal_smoothing_flow(
         video_path, out_dir, flow_threshold=0.5, alpha_fraction=0.2, window_size=30, morph_kernel=2,
-        save_name="overlay.mp4", mask_save_name="mask.mp4"))
+        save_name="overlay.mp4", mask_save_name="mask.mp4", flow_device=flow_device))
     logging.info(f"Step 1/2: Motion detection completed (elapsed: {md.total_s:.2f} s, avg per frame: {md.avg_s:.4f} s).")
 
     logging.info("Step 2/2: Starting compression...")

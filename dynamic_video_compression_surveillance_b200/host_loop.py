@@ -4,8 +4,8 @@ reference's GUI and performance_analysis.py depend on (file names, ``execution_t
 Design (not the reference's): a decode thread fills pinned batch buffers from cv2.VideoCapture, the GPU loop runs
 per batch through ``FramePipeline.process_host`` (upload / kernels / download double-buffered inside the library),
 an encode thread feeds the two VideoWriters.  What stays on the host is what SURVEY.md section 8 leaves
-there: codecs, the first frame's resize + heavy blur (frame_differencing.py:74,77; once per stream), Farneback
-flow (motion_compression_opt.py:72-82).
+there: codecs, the first frame's resize + heavy blur (frame_differencing.py:74,77; once per stream) and, unless the
+caller asks for the GPU (``flow_masks_gpu``), Farneback flow (motion_compression_opt.py:72-82).
 """
 from __future__ import annotations
 
@@ -207,6 +207,25 @@ def smooth_rect_masks_gpu(raw_masks: list, history: list, window_size: int, alph
     voted = P.temporal_ring(stack, window_size, alpha_fraction)[len(history):].contiguous()
     closed = P.morph(voted, "close", morph_kernel, "ellipse")
     return P.mask_rectangles(P.morph(closed, "open", morph_kernel, "ellipse")).cpu().numpy()
+
+
+def first_gray_gpu(frame: np.ndarray) -> torch.Tensor:
+    """cv2.cvtColor(frame, BGR2GRAY) of one host frame on the GPU (motion_compression_opt.py:60), left there."""
+    return P.bgr2gray(torch.from_numpy(np.ascontiguousarray(frame))[None].cuda())[0]
+
+
+def flow_masks_gpu(frames: list, prev_gray, flow_threshold: float = 0.5, farneback: tuple = (0.3, 2, 9, 2, 5, 1.1, 0)):
+    """Raw flow masks of a chunk of BGR frames (motion_compression_opt.py:71-83) on the GPU: upload, BGR2GRAY, prepend
+    the carried gray of the frame before the chunk, Farneback + magnitude + threshold.  ``prev_gray`` is that gray, a
+    host array or a CUDA tensor [H,W]; ``farneback`` = (pyr_scale, levels, winsize, iterations, poly_n, poly_sigma,
+    flags).  Returns (masks [N,H,W] uint8 host array, the last gray as a CUDA tensor to pass with the next chunk)."""
+    prev = prev_gray if isinstance(prev_gray, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(prev_gray))
+    prev = prev.cuda()
+    if not frames:
+        return np.empty((0,) + tuple(prev.shape), np.uint8), prev
+    grays = P.bgr2gray(torch.from_numpy(np.stack(frames)).cuda())
+    masks = P.flow_masks(torch.cat([prev[None], grays]), flow_threshold, *farneback)
+    return masks.cpu().numpy(), grays[-1].clone()
 
 
 def degrade_mco_gpu(frames: list, masks: list) -> np.ndarray:

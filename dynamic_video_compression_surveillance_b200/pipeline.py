@@ -335,3 +335,38 @@ def gaussian_blur(planes: torch.Tensor, ksize: int, sigma: float) -> torch.Tenso
     out = torch.empty_like(planes)
     _lib_call("dvc_gaussian_blur_u8", planes.data_ptr(), out.data_ptr(), n, h, w, int(ksize), float(sigma), _stream_ptr(None))
     return out
+
+
+def _flow_args(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags):
+    return (float(pyr_scale), int(levels), int(winsize), int(iterations), int(poly_n), float(poly_sigma), int(flags))
+
+
+def farneback_flow(prev: torch.Tensor, next: torch.Tensor, pyr_scale: float = 0.3, levels: int = 2, winsize: int = 9,
+                   iterations: int = 2, poly_n: int = 5, poly_sigma: float = 1.1, flags: int = 0) -> torch.Tensor:
+    """cv2.calcOpticalFlowFarneback(prev, next, None, pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags)
+    (motion_compression_opt.py:72-81) for uint8 planes [H,W] or pairs [N,H,W] -> float32 flow [H,W,2] or [N,H,W,2].
+    Defaults are the call site's.  poly_n other than 5 / 7 and flags other than 0 raise NotImplementedError."""
+    _dev_u8(prev, "prev"); _dev_u8(next, "next")
+    if prev.shape != next.shape or prev.dim() not in (2, 3):
+        raise ValueError("prev and next must be [H, W] or [N, H, W] of the same shape")
+    p, q = (prev[None], next[None]) if prev.dim() == 2 else (prev, next)
+    n, h, w = p.shape
+    out = torch.empty((n, h, w, 2), dtype=torch.float32, device=prev.device)
+    _lib_call("dvc_farneback_flow_f32", p.data_ptr(), q.data_ptr(), out.data_ptr(), n, h, w,
+              *_flow_args(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags), _stream_ptr(None))
+    return out[0] if prev.dim() == 2 else out
+
+
+def flow_masks(grays: torch.Tensor, flow_threshold: float = 0.5, pyr_scale: float = 0.3, levels: int = 2, winsize: int = 9,
+               iterations: int = 2, poly_n: int = 5, poly_sigma: float = 1.1, flags: int = 0) -> torch.Tensor:
+    """The raw masks of temporal_smoothing_flow (motion_compression_opt.py:72-83) for a uint8 gray sequence [N+1,H,W]:
+    [N,H,W], mask i = 255 where the float32 flow magnitude from frame i to frame i + 1 exceeds float32(flow_threshold)."""
+    _dev_u8(grays, "grays")
+    if grays.dim() != 3 or grays.shape[0] < 1:
+        raise ValueError("grays must be [N+1, H, W] with N >= 0")
+    n1, h, w = grays.shape
+    out = torch.empty((n1 - 1, h, w), dtype=torch.uint8, device=grays.device)
+    _lib_call("dvc_flow_masks_u8", grays.data_ptr(), out.data_ptr(), n1 - 1, h, w,
+              *_flow_args(pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags), float(flow_threshold),
+              _stream_ptr(None))
+    return out

@@ -222,6 +222,30 @@ int dvc_gaussian_blur_u8(const uint8_t* src_dev, uint8_t* dst_dev, int32_t n, in
 int dvc_dct_blocks_f32(const float* src_dev, float* dst_dev, int64_t n, int32_t bh, int32_t bw, int32_t inverse,
                        void* stream);
 
+/* cv2.calcOpticalFlowFarneback(prev, next, None, pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags),
+ * motion_compression_opt.py:72-81, for n independent pairs of uint8 planes prev_dev / next_dev [n][H][W].  flow_dev is
+ * float32 [n][H][W][2] (x, y), the layout cv2 returns.  Parity: OpenCV's CPU algorithm stage by stage, with the same
+ * float / double roundings where cv2 rounds, including the order of its box filter's running sums, except for the
+ * Gaussian blur and resize that build the pyramid levels (float rounding of the sums may differ by an ulp).  cv2 itself does not
+ * reproduce its own flow across dispatch paths; DESIGN.md section 6 gives the measured agreement.
+ *   DVC_ERR_INVALID:     pyr_scale outside (0, 1), levels < 0, winsize < 1, iterations < 1, negative poly_sigma, null
+ *                        pointers, bad sizes.
+ *   DVC_ERR_UNSUPPORTED: poly_n other than 5 or 7; flags other than 0 (OPTFLOW_USE_INITIAL_FLOW and
+ *                        OPTFLOW_FARNEBACK_GAUSSIAN are not implemented); H or W above 32767; a pyramid level whose
+ *                        Gaussian would need more than 255 taps.
+ * Scratch comes from the stream-ordered allocator's cached pool. */
+int dvc_farneback_flow_f32(const uint8_t* prev_dev, const uint8_t* next_dev, float* flow_dev, int32_t n, int32_t H, int32_t W,
+                           double pyr_scale, int32_t levels, int32_t winsize, int32_t iterations, int32_t poly_n,
+                           double poly_sigma, int32_t flags, void* stream);
+/* The raw motion masks of temporal_smoothing_flow, motion_compression_opt.py:72-83, for a sequence gray_dev [n+1][H][W]:
+ * mask_dev[i] [H][W] = 255 * (|flow(gray[i], gray[i+1])| > flow_threshold), 0 elsewhere, where |flow| is cartToPolar's
+ * float32 magnitude.  flow_threshold is compared as float32, as numpy compares a float32 array with a Python float.
+ * Each frame's pyramid is built once and serves both pairs it belongs to; the flow is never stored.  Same parameters and
+ * error codes as dvc_farneback_flow_f32. */
+int dvc_flow_masks_u8(const uint8_t* gray_dev, uint8_t* mask_dev, int32_t n, int32_t H, int32_t W, double pyr_scale,
+                      int32_t levels, int32_t winsize, int32_t iterations, int32_t poly_n, double poly_sigma, int32_t flags,
+                      float flow_threshold, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
