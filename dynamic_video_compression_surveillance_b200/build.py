@@ -12,8 +12,10 @@ LIB = os.path.join(HERE, "libdvc_b200.so")
 DEPS = [os.path.join(HERE, "csrc", f) for f in os.listdir(os.path.join(HERE, "csrc"))] + [
     os.path.join(os.path.dirname(HERE), "include", "dvc_b200.h")]
 
+# -ffp-contract=off: host-side constants (the Farneback taps and Gram inverse) must round each operation as OpenCV does,
+# also on hosts whose compiler would otherwise fuse multiply-adds.
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
-              "-shared", "-Xcompiler", "-fPIC", "--threads", "2"]
+              "-shared", "-Xcompiler", "-fPIC,-ffp-contract=off", "--threads", "2"]
 
 
 def find_nvcc() -> str:

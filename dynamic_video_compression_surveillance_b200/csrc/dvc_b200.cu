@@ -1616,22 +1616,62 @@ struct FlowPlan {
     FlowPolyTab poly;
 };
 
-// getGaussianKernel(n, sigma, CV_32F): the small fixed kernels when sigma <= 0, float taps normalised in double
+// getGaussianKernel(n, sigma, CV_32F) for odd n, as getGaussianKernelBitExact computes it: the small fixed kernels when
+// sigma <= 0; otherwise, in double, exp at doubled coordinates x = 1 - n, 3 - n, .. (scale -0.125 / sigma^2), the sum of
+// those taps doubled plus 1 for the centre, one reciprocal, and each tap times that reciprocal rounded to float once.
+// Rounding the taps to float before normalising (as a plain exp/sum replay does) moves some of them by one ulp.
 static void gauss_kernel_f32(int n, double sigma, float* half) {
-    static const float fixed[4][7] = {{1.f}, {0.25f, 0.5f, 0.25f}, {0.0625f, 0.25f, 0.375f, 0.25f, 0.0625f},
-                                      {0.03125f, 0.109375f, 0.21875f, 0.28125f, 0.21875f, 0.109375f, 0.03125f}};
-    const bool use_fixed = n % 2 == 1 && n <= 7 && sigma <= 0;
-    const double sx = sigma > 0 ? sigma : ((n - 1) * 0.5 - 1) * 0.3 + 0.8;
-    const double scale2x = -0.5 / (sx * sx);
-    std::vector<float> c(n);
-    double sum = 0;
-    for (int i = 0; i < n; ++i) {
-        const double x = i - (n - 1) * 0.5;
-        c[i] = (float)(use_fixed ? (double)fixed[n / 2][i] : std::exp(scale2x * x * x));
-        sum += c[i];
+    static const double fixed[5][5] = {{1.}, {0.5, 0.25}, {0.375, 0.25, 0.0625}, {0.28125, 0.21875, 0.109375, 0.03125},
+                                       {60 / 256., 51 / 256., 30 / 256., 13 / 256., 4 / 256.}};
+    const int n2 = n / 2;
+    if (sigma <= 0 && n <= 9) {
+        for (int i = 0; i <= n2; ++i) half[i] = (float)fixed[n2][i];
+        return;
     }
-    sum = 1. / sum;
-    for (int i = n / 2; i < n; ++i) half[i - n / 2] = (float)(c[i] * sum);
+    const double sx = sigma > 0 ? sigma : std::fma((double)n, 0.15, 0.35);     // softfloat mulAdd: one rounding
+    const double scale2x = -0.125 / (sx * sx);
+    std::vector<double> v(n2);
+    double sum = 0;
+    for (int i = 0; i < n2; ++i) {
+        const int x = 1 - n + 2 * i;
+        v[i] = std::exp((double)(x * x) * scale2x);
+        sum += v[i];
+    }
+    sum = sum * 2 + 1;
+    const double mul = 1. / sum;
+    half[0] = (float)mul;
+    for (int i = 0; i < n2; ++i) half[n2 - i] = (float)(v[i] * mul);
+}
+
+// Mat::inv(DECOMP_CHOLESKY) of the symmetric positive definite 6 x 6 Gram matrix, in hal::Cholesky64f's order: L with the
+// reciprocal of its diagonal, then forward and back substitution against the identity.  Gauss-Jordan elimination gives
+// inverse entries a few ulps away from these, which moves the polynomial coefficients.
+static void cholesky_inverse6(double A[6][6], double B[6][6]) {
+    for (int i = 0; i < 6; ++i) {
+        int j = 0;
+        for (; j < i; ++j) {
+            double s = A[i][j];
+            for (int k = 0; k < j; ++k) s -= A[i][k] * A[j][k];
+            A[i][j] = s * A[j][j];
+        }
+        double s = A[i][i];
+        for (int k = 0; k < j; ++k) s -= A[i][k] * A[i][k];
+        A[i][i] = 1. / std::sqrt(s);
+    }
+    for (int i = 0; i < 6; ++i)
+        for (int j = 0; j < 6; ++j) B[i][j] = i == j ? 1. : 0.;
+    for (int i = 0; i < 6; ++i)
+        for (int j = 0; j < 6; ++j) {
+            double s = B[i][j];
+            for (int k = 0; k < i; ++k) s -= A[i][k] * B[k][j];
+            B[i][j] = s * A[i][i];
+        }
+    for (int i = 5; i >= 0; --i)
+        for (int j = 0; j < 6; ++j) {
+            double s = B[i][j];
+            for (int k = 5; k > i; --k) s -= A[k][i] * B[k][j];
+            B[i][j] = s * A[i][i];
+        }
 }
 
 // FarnebackPrepareGaussian: float taps, the 6 x 6 Gram matrix in double and four entries of its inverse
@@ -1644,7 +1684,7 @@ static void flow_poly_tab(int n, double sigma, FlowPolyTab& t) {
     for (int x = -n; x <= n; ++x) g[x + n] = (float)(g[x + n] * s);
     t.n = n;
     for (int k = 0; k <= n; ++k) { t.g[k] = g[k + n]; t.xg[k] = (float)k * g[k + n]; t.xxg[k] = (float)(k * k) * g[k + n]; }
-    double G[6][12] = {};
+    double G[6][6] = {}, iG[6][6];
     for (int y = -n; y <= n; ++y)
         for (int x = -n; x <= n; ++x) {
             const float gy = g[y + n], gx = g[x + n], fx = (float)x, fy = (float)y;
@@ -1656,20 +1696,8 @@ static void flow_poly_tab(int n, double sigma, FlowPolyTab& t) {
     G[2][2] = G[0][3] = G[0][4] = G[3][0] = G[4][0] = G[1][1];
     G[4][4] = G[3][3];
     G[3][4] = G[4][3] = G[5][5];
-    for (int i = 0; i < 6; ++i) G[i][6 + i] = 1.0;
-    for (int c = 0; c < 6; ++c) {                         // Gauss-Jordan with partial pivoting (G is positive definite)
-        int piv = c;
-        for (int r = c + 1; r < 6; ++r) if (std::fabs(G[r][c]) > std::fabs(G[piv][c])) piv = r;
-        for (int j = 0; j < 12; ++j) std::swap(G[c][j], G[piv][j]);
-        const double d = G[c][c];
-        for (int j = 0; j < 12; ++j) G[c][j] /= d;
-        for (int r = 0; r < 6; ++r)
-            if (r != c && G[r][c] != 0.0) {
-                const double f = G[r][c];
-                for (int j = 0; j < 12; ++j) G[r][j] -= f * G[c][j];
-            }
-    }
-    t.ig11 = G[1][7]; t.ig03 = G[0][9]; t.ig33 = G[3][9]; t.ig55 = G[5][11];
+    cholesky_inverse6(G, iG);
+    t.ig11 = iG[1][1]; t.ig03 = iG[0][3]; t.ig33 = iG[3][3]; t.ig55 = iG[5][5];
 }
 
 static int cv_round(double v) { return (int)std::lrint(v); }
@@ -1713,6 +1741,7 @@ static int flow_plan(const char* who, int n, int H, int W, double pyr_scale, int
         g.h = cv_round(H * s);
         g.scale_x = 1. / ((double)g.w / W);
         g.scale_y = 1. / ((double)g.h / H);
+        g.area_tail = W == 2 * g.w && H == 2 * g.h ? g.w / 4 * 4 : g.w;
         pl.off[l] = pl.P;
         pl.P += (size_t)g.w * g.h;
     }

@@ -1,6 +1,7 @@
 // Dense optical flow: cv2.calcOpticalFlowFarneback (motion_compression_opt.py:72-81) with flags 0, box-filtered solve.
 //
-// The stages follow OpenCV's CPU code (optflowgf.cpp) and were pinned down against cv2 4.13 as a black box:
+// The stages follow OpenCV's CPU code (optflowgf.cpp) in the operation order of cv2's scalar path, which oracle/flow_ops.py
+// restates in numpy; tests/test_flow_exact_gpu.py requires equal bytes against that model at every pixel:
 //   level image   float32 frame -> GaussianBlur(ksize, sigma), REFLECT_101 -> resize INTER_LINEAR   k_flow_level
 //   polynomial    separable Gaussian-weighted fit, replicated borders, 5 coefficients per pixel       k_flow_poly
 //   matrices      R1 sampled bilinearly at x + flow, border taper, M = (G11, G12, G22, h1, h2)       k_flow_matrices
@@ -33,6 +34,7 @@ struct FlowLevelGeom {
     int half;                   // ksize / 2
     int w, h;                   // level size
     double scale_x, scale_y;    // cv2.resize's 1 / (dst / src)
+    int area_tail;              // first column of INTER_AREA's scalar loop on an exact 2x reduction, else w
 };
 
 // cv2.resize INTER_LINEAR source index and weight of destination index d (resizeGeneric's table)
@@ -43,12 +45,19 @@ DEVI void resize_tap(int d, double scale, int& s, float& f) {
 }
 
 // ---- level image ---------------------------------------------------------------------------------------------------
-// Row filter then column filter (cv2's separable order), each as k0 * c + sum k_i * (l_i + r_i).
+// Row filter then column filter (cv2's separable order), summed as cv2's scalar filters sum.  Rows: up to 5 taps the small
+// symmetric filter c * k0 + (l_i + r_i) * k_i; wider kernels the generic filter, left to right over all taps.  Columns: the
+// symmetric filter k0 * c + sum k_i * (above_i + below_i).
 DEVI float blur_row(const uint8_t* src, int W, int r, int c, const FlowLevelGeom& g) {
     const uint8_t* row = src + (size_t)r * W;
-    float s = __fmul_rn((float)row[c], g.k[0]);
-    for (int i = 1; i <= g.half; ++i)
-        s = __fadd_rn(s, __fmul_rn(g.k[i], __fadd_rn((float)row[reflect101(c - i, W)], (float)row[reflect101(c + i, W)])));
+    if (g.half <= 2) {
+        float s = __fmul_rn((float)row[c], g.k[0]);
+        for (int i = 1; i <= g.half; ++i)
+            s = __fadd_rn(s, __fmul_rn(g.k[i], __fadd_rn((float)row[reflect101(c - i, W)], (float)row[reflect101(c + i, W)])));
+        return s;
+    }
+    float s = __fmul_rn(g.k[g.half], (float)row[reflect101(c - g.half, W)]);
+    for (int j = 1 - g.half; j <= g.half; ++j) s = __fadd_rn(s, __fmul_rn(g.k[abs(j)], (float)row[reflect101(c + j, W)]));
     return s;
 }
 DEVI float blur_at(const uint8_t* src, int H, int W, int r, int c, const FlowLevelGeom& g) {
@@ -69,6 +78,12 @@ __global__ void __launch_bounds__(256) k_flow_level(const uint8_t* __restrict__ 
     float v;
     if (g.w == W && g.h == H) {                          // cv2.resize to the same size copies
         v = blur_at(src, H, W, y, x, g);
+    } else if (x >= g.area_tail) {
+        // An exact 2x reduction runs INTER_AREA's fast path: its 4-lane loop equals the bilinear formula below, and the last
+        // w % 4 columns take its scalar loop, (((a + b) + c) + d) / 4.
+        const float a = blur_at(src, H, W, 2 * y, 2 * x, g), b = blur_at(src, H, W, 2 * y, 2 * x + 1, g);
+        const float c = blur_at(src, H, W, 2 * y + 1, 2 * x, g), d = blur_at(src, H, W, 2 * y + 1, 2 * x + 1, g);
+        v = __fmul_rn(__fadd_rn(__fadd_rn(__fadd_rn(a, b), c), d), 0.25f);
     } else {
         int sx, sy;
         float fx, fy;
@@ -135,9 +150,11 @@ __global__ void __launch_bounds__(256) k_flow_poly(const float* __restrict__ img
 }
 
 // ---- update matrices (FarnebackUpdateMatrices) for one pixel -----------------------------------------------------------
-DEVI float flow_border(int i, int len) {
+// cv2's taper ((x_lo * x_hi) * y_lo) * y_hi: on sides below 10 both factors of an axis apply, and the grouping matters
+DEVI float flow_border(int x, int y, int w, int h) {
     const float tab[5] = {0.14f, 0.14f, 0.4472f, 0.4472f, 0.4472f};
-    return __fmul_rn(i < 5 ? tab[i] : 1.f, i >= len - 5 ? tab[len - i - 1] : 1.f);
+    const float s = __fmul_rn(x < 5 ? tab[x] : 1.f, x >= w - 5 ? tab[w - x - 1] : 1.f);
+    return __fmul_rn(__fmul_rn(s, y < 5 ? tab[y] : 1.f), y >= h - 5 ? tab[h - y - 1] : 1.f);
 }
 
 DEVI void flow_matrix(const float* __restrict__ R0, const float* __restrict__ R1, int w, int h, int x, int y, float dx, float dy,
@@ -174,7 +191,7 @@ DEVI void flow_matrix(const float* __restrict__ R0, const float* __restrict__ R1
     r2 = __fadd_rn(r2, __fadd_rn(__fmul_rn(r4, dy), __fmul_rn(r6, dx)));
     r3 = __fadd_rn(r3, __fadd_rn(__fmul_rn(r6, dy), __fmul_rn(r5, dx)));
     if ((unsigned)(x - 5) >= (unsigned)(w - 10) || (unsigned)(y - 5) >= (unsigned)(h - 10)) {
-        const float s = __fmul_rn(flow_border(x, w), flow_border(y, h));
+        const float s = flow_border(x, y, w, h);
         r2 = __fmul_rn(r2, s); r3 = __fmul_rn(r3, s); r4 = __fmul_rn(r4, s); r5 = __fmul_rn(r5, s); r6 = __fmul_rn(r6, s);
     }
     M[0] = __fadd_rn(__fmul_rn(r4, r4), __fmul_rn(r6, r6));
@@ -217,8 +234,9 @@ __global__ void __launch_bounds__(256) k_flow_matrices(FlowPair pr, const float2
         const float2 p10 = c[(size_t)y1 * cw + sx], p11 = c[(size_t)y1 * cw + sx1];
         const float hx0 = __fadd_rn(__fmul_rn(p00.x, a0), __fmul_rn(p01.x, fx)), hx1 = __fadd_rn(__fmul_rn(p10.x, a0), __fmul_rn(p11.x, fx));
         const float hy0 = __fadd_rn(__fmul_rn(p00.y, a0), __fmul_rn(p01.y, fx)), hy1 = __fadd_rn(__fmul_rn(p10.y, a0), __fmul_rn(p11.y, fx));
-        dx = __fmul_rn(__fadd_rn(__fmul_rn(hx0, b0), __fmul_rn(hx1, fy)), up);
-        dy = __fmul_rn(__fadd_rn(__fmul_rn(hy0, b0), __fmul_rn(hy1, fy)), up);
+        // cv2 scales with convertTo: x * a + 0, which turns -0 into +0
+        dx = __fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(hx0, b0), __fmul_rn(hx1, fy)), up), 0.f);
+        dy = __fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(hy0, b0), __fmul_rn(hy1, fy)), up), 0.f);
     }
     float m[5];
     flow_matrix(pr.R0 + p * pr.r_stride, pr.R1 + p * pr.r_stride, pr.w, pr.h, x, y, dx, dy, m);

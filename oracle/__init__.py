@@ -16,6 +16,9 @@ SURVEY.md section 4):
   the real ``cv2`` call (opencv-python is the reference's pinned third-party
   dependency, requirements.txt:2 ``==4.11.0.86``; the image has 4.13.0).
 * ``oracle/loops.py``      -- the loop bodies restated on arrays.
+* ``oracle/flow_ops.py``   -- cv2.calcOpticalFlowFarneback in cv2's scalar
+  operation order; ``tests/test_flow_oracle_cpu.py`` checks it against cv2
+  byte for byte and ``tests/test_flow_exact_gpu.py`` the kernels against it.
 * ``oracle/cv2_proxy.py`` + ``oracle/make_golden.py`` -- run the UNMODIFIED
   reference modules from /root/reference on array-backed VideoCapture /
   VideoWriter fakes (no lossy codec) and commit the outputs as fixtures under
