@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # that file does not exist unless such a tool built it
 LIB_PATH = os.path.join(HERE, "libdvc_b200_measure.so" if os.environ.get("DVC_LIB_FLAVOUR") == "measure" else "libdvc_b200.so")
 
-DVC_MODE_FD, DVC_MODE_WINDOW = 0, 1
+DVC_MODE_FD, DVC_MODE_WINDOW, DVC_MODE_FLOW = 0, 1, 2
 DVC_MORPH_ERODE, DVC_MORPH_DILATE, DVC_MORPH_OPEN, DVC_MORPH_CLOSE = 0, 1, 2, 3
 DVC_SHAPE_RECT, DVC_SHAPE_ELLIPSE = 0, 1
 DVC_DEGRADE_FD, DVC_DEGRADE_MCO = 0, 1
@@ -57,6 +57,7 @@ SYMBOLS = {
     "dvc_set_state": (C.c_int, [_P, _P, C.c_size_t]),
     "dvc_get_counters": (C.c_int, [_P, C.POINTER(DvcCounters)]),
     "dvc_reset_counters": (C.c_int, [_P]),
+    "dvc_set_flow_params": (C.c_int, [_P, _F, _D, _I, _I, _I, _I, _D, _I]),
     "dvc_process_batch": (C.c_int, [_P, _P, _I, _P, _P, _P, _P]),
     "dvc_set_overlap": (C.c_int, [_P, _I]),
     "dvc_flush": (C.c_int, [_P, _P]),

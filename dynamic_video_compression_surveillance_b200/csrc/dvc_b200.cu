@@ -4,12 +4,14 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
+#include <string>
 #include <vector>
 
 #include "../../include/dvc_b200.h"
@@ -50,6 +52,13 @@ static inline unsigned cdiv(size_t a, size_t b) { return (unsigned)((a + b - 1) 
 
 static int pack_to_bits(const uint8_t* src, uint32_t* dst, int n, int H, int W, cudaStream_t st);
 static int unpack_from_bits(const uint32_t* src, uint8_t* dst, int n, int H, int W, cudaStream_t st);
+struct dvc_handle;
+static int flow_create(dvc_handle* h);
+static void flow_destroy(dvc_handle* h);
+static int flow_front(dvc_handle* h, const uint8_t* frames, int T, cudaStream_t st);
+static int flow_rect_launch(dvc_handle* h, const uint32_t* src, uint32_t* dst, int n, cudaStream_t st);
+static int flow_rebuild_prev(dvc_handle* h);
+static constexpr int RECT_FRAMES = 8;      // flow loop: planes per launch of the rectangle kernels
 
 // ------------------------------------------------------------------------------------------------
 // structuring elements -> MorphChain
@@ -352,6 +361,38 @@ static void ccl_scratch_free(CclScratch& sc) {
     sc = CclScratch();
 }
 
+// Bounding rectangles of the 8-connected components (motion_compression_opt.py:93-97) of n bit-planes src -> dst.  Scratch
+// (rect_scratch_bytes) holds the union-find parents and the three bounding-box arrays of `frames` planes, each a dense +
+// overflow pair; the planes go through in chunks of that many.
+static size_t rect_scratch_bytes(int frames, int H, int W) {
+    return 4 * (ccl_dense_ints(H, W) + ccl_overflow_ints(H, W)) * sizeof(int) * frames;
+}
+static int launch_rectangles(char* ERRBUF, const uint32_t* src, uint32_t* dst, int n, int H, int W, void* scratch, int frames,
+                             cudaStream_t st) {
+    const int wpr = words_per_row(W);
+    const size_t pw = (size_t)H * wpr;
+    const size_t d = ccl_dense_ints(H, W) * sizeof(int) * frames, o = ccl_overflow_ints(H, W) * sizeof(int) * frames;
+    char* const pp = (char*)scratch;                     // parents: dense | overflow
+    char* const bd = pp + d + o;                         // bounding boxes: 3 dense | 3 overflow
+    char* const bo = bd + 3 * d;
+    CU(cudaMemsetAsync(dst, 0, pw * 4 * n, st));
+    BBoxArrays bb;
+    for (int k = 0; k < 3; ++k) { bb.d[k] = (int*)(bd + k * d); bb.ov[k] = (int*)(bo + k * o); }
+    for (int i0 = 0; i0 < n; i0 += frames) {
+        const int m = std::min(frames, n - i0);
+        dim3 grid(cdiv(pw, 256), m), grow((H + 7) / 8, m);
+        const uint32_t* r = src + (size_t)i0 * pw;
+        CU(cudaMemsetAsync(bd, 0x7f, 3 * d, st));           // 0x7f7f7f7f: larger than any coordinate or negated coordinate
+        CU(cudaMemsetAsync(bo, 0x7f, 3 * o, st));
+        k_ccl_rowlink<false, false><<<grow, 256, 0, st>>>(r, (int*)pp, (int*)(pp + d), nullptr, nullptr, H, W, wpr, nullptr);
+        k_ccl_union<false, 8><<<CCL_GRID(wpr, H, m), 256, 0, st>>>(r, (int*)pp, (int*)(pp + d), H, W, wpr, nullptr);
+        k_ccl_bbox<<<grid, 256, 0, st>>>(r, (int*)pp, (int*)(pp + d), bb, H, W, wpr);
+        k_ccl_paint_rects<<<grid, 256, 0, st>>>(r, (int*)pp, (int*)(pp + d), bb, dst + (size_t)i0 * pw, H, W, wpr);
+        CHECK_LAUNCH();
+    }
+    return DVC_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // cv2.resize INTER_LINEAR tables (OpenCV resize(): scale = 1 / ((double)dst / src); fx = (float)((d + 0.5) * scale - 0.5);
 // sx = floor(fx); fx -= sx; columns clamp (sx, fx) at the image border, rows keep fx and clip the row index instead;
@@ -591,6 +632,7 @@ static int launch_degrade(char* ERRBUF, const uint8_t* frames, const uint32_t* o
 // handle
 // ------------------------------------------------------------------------------------------------
 struct ProfRec { int kid; int launches; cudaEvent_t a, b; };
+struct FlowLoop;                  // DVC_MODE_FLOW: Farneback parameters and scratch (defined with the flow code below)
 
 struct dvc_handle {
     dvc_config cfg;
@@ -605,13 +647,14 @@ struct dvc_handle {
     uint8_t* prev_gray[2];
     int cur;
     uint8_t* acc;                 // FD: accumulated_mask
-    uint32_t* ring;               // WINDOW: raw-mask ring, ring_cap planes
+    uint32_t* ring;               // WINDOW / FLOW: raw-mask ring, ring_cap planes
     int ring_cap;
     MinCounts min_counts;
     // scratch (max_batch planes each)
     uint32_t* bits[2][3];         // two sets (software pipelining across batches) of three bit-plane arrays
     uint8_t* blurred;             // FD: [max_batch] gray planes
     CclScratch ccl;
+    FlowLoop* flow;               // FLOW only
     MorphChain chain;
     Counters* counters_dev;
     dvc_counters counters_host;   // frames / pixels / blocks are counted on the host
@@ -786,6 +829,7 @@ static int create_impl(const dvc_config* cfg, dvc_handle* h) {
         }
         if (cfg->kernel_size > 0 && !chain_push(h->chain, DVC_MORPH_DILATE, DVC_SHAPE_RECT, cfg->kernel_size))
             return set_err(h->err, DVC_ERR_UNSUPPORTED, "kernel_size %d: supported range is 1..%d", cfg->kernel_size, MORPH_MAX_K);
+        if (cfg->mode == DVC_MODE_FLOW) return flow_create(h);
     }
     return DVC_OK;
 }
@@ -804,6 +848,7 @@ extern "C" int dvc_destroy(dvc_handle* h) {
     if (h->ev_user) cudaEventDestroy(h->ev_user);
     for (int s = 0; s < 2; ++s) { if (h->ev_front[s]) cudaEventDestroy(h->ev_front[s]); if (h->ev_mask[s]) cudaEventDestroy(h->ev_mask[s]); if (h->ev_k4[s]) cudaEventDestroy(h->ev_k4[s]); }
     ccl_scratch_free(h->ccl);
+    flow_destroy(h);
     if (h->staging) {
         for (int b = 0; b < 2; ++b) {
             cudaFree(h->st_in[b]); cudaFree(h->st_ov[b]); cudaFree(h->st_cp[b]); cudaFree(h->st_mask[b]);
@@ -822,7 +867,17 @@ extern "C" int dvc_create(const dvc_config* cfg, dvc_handle** out) {
     *out = nullptr;
     if (cfg->width < 1 || cfg->height < 1 || cfg->max_batch < 1)
         return set_err(nullptr, DVC_ERR_INVALID, "dvc_create: width, height and max_batch must be >= 1");
-    if (cfg->mode != DVC_MODE_FD && cfg->mode != DVC_MODE_WINDOW) return set_err(nullptr, DVC_ERR_INVALID, "dvc_create: unknown mode %d", cfg->mode);
+    if (cfg->mode != DVC_MODE_FD && cfg->mode != DVC_MODE_WINDOW && cfg->mode != DVC_MODE_FLOW)
+        return set_err(nullptr, DVC_ERR_INVALID, "dvc_create: unknown mode %d", cfg->mode);
+    if (cfg->mode == DVC_MODE_FLOW) {
+        // the fields of the other loops that this one has no stage for are refused, not ignored
+        if (cfg->block_size != 8)
+            return set_err(nullptr, DVC_ERR_UNSUPPORTED, "dvc_create: block_size %d: the flow loop degrades as compress_with_motion does, 8x8 only", cfg->block_size);
+        if (cfg->kernel_size != 0)
+            return set_err(nullptr, DVC_ERR_INVALID, "dvc_create: kernel_size %d: the flow loop has no dilate, set 0", cfg->kernel_size);
+        if (cfg->src_width != 0 || cfg->src_height != 0)
+            return set_err(nullptr, DVC_ERR_UNSUPPORTED, "dvc_create: src_width / src_height: the flow loop does not resize, set 0");
+    }
     if (cfg->block_size < 1 || cfg->block_size > 8)
         return set_err(nullptr, DVC_ERR_UNSUPPORTED, "block_size %d: the GPU path implements 1..8 (cv2's DCT routines for longer blocks are not restated)", cfg->block_size);
     if (!(cfg->quantization_level > 0.0f)) return set_err(nullptr, DVC_ERR_INVALID, "quantization_level must be > 0");
@@ -854,7 +909,7 @@ extern "C" int dvc_begin_stream(dvc_handle* h, const uint8_t* prev_gray_host) {
     if (h->acc) CU(h_fill0(h, h->acc, h->plane_bytes * h->S));
     if (h->ring) CU(h_fill0(h, h->ring, h->plane_words * 4 * h->ring_cap * h->S));
     h->n_masks = 0;
-    return DVC_OK;
+    return h->flow ? flow_rebuild_prev(h) : DVC_OK;
 }
 
 // ---- state blob: header | prev_gray | acc (FD)  or  K raw planes oldest..newest (WINDOW) ----------
@@ -901,7 +956,7 @@ extern "C" int dvc_set_state(dvc_handle* h, const void* buf, size_t bytes) {
     const uint8_t* p = (const uint8_t*)buf;
     memcpy(&hd, p, sizeof(hd)); p += sizeof(hd);
     if (hd.magic != STATE_MAGIC || hd.mode != (uint32_t)h->cfg.mode || hd.W != (uint32_t)h->W || hd.H != (uint32_t)h->H ||
-        (h->cfg.mode == DVC_MODE_WINDOW && hd.K != (uint32_t)h->cfg.window_size) || std::max(1u, hd.reserved) != (uint32_t)h->S)
+        (h->cfg.mode != DVC_MODE_FD && hd.K != (uint32_t)h->cfg.window_size) || std::max(1u, hd.reserved) != (uint32_t)h->S)
         return set_err(h->err, DVC_ERR_INVALID, "dvc_set_state: blob does not match this handle's configuration");
     CU(cudaSetDevice(h->cfg.device));
     CU(handle_join(h));
@@ -920,7 +975,7 @@ extern "C" int dvc_set_state(dvc_handle* h, const void* buf, size_t bytes) {
             }
         }
     }
-    return DVC_OK;
+    return h->flow ? flow_rebuild_prev(h) : DVC_OK;
 }
 
 extern "C" int dvc_get_counters(dvc_handle* h, dvc_counters* out) {
@@ -1008,12 +1063,18 @@ static int process_batch_impl(dvc_handle* h, const uint8_t* frames, int T, uint8
     const uint32_t* over127 = nullptr;
     const uint32_t* nonzero = nullptr;
     const unsigned g16 = cdiv((size_t)((W + 15) / 16) * H, 256);
-    if (h->cfg.mode == DVC_MODE_WINDOW) {
+    if (h->cfg.mode != DVC_MODE_FD) {
         uint8_t* pg_in = h->prev_gray[h->cur];
         uint8_t* pg_out = h->prev_gray[h->cur ^ 1];
         const int K = h->cfg.window_size;
         static const bool fuse_env = measure_env("DVC_FUSE_VOTE", 1) != 0;
-        if (h->aligned && K <= 8 && h->gray_impl == 2 && fuse_env) {
+        const bool fused = !h->flow && h->aligned && K <= 8 && h->gray_impl == 2 && fuse_env;
+        const int nseg = (T + h->seg_len - 1) / h->seg_len;
+        if (h->flow) {
+            // gray, pyramids and flow: the raw masks land in the ring as bit-planes (the vote below reads them there)
+            int rc = flow_front(h, frames, T, st);
+            if (rc) return rc;
+        } else if (fused) {
             // K1 + K2 in one kernel (k_gray_diff_vote): long segments, each rebuilding its K - 1 frames of history
             const int seg = std::max(K, std::max(8, measure_env("DVC_FUSE_SEG", 64))), nsegf = (T + seg - 1) / seg;
             dim3 gf(g16, nsegf, S);
@@ -1030,7 +1091,6 @@ static int process_batch_impl(dvc_handle* h, const uint8_t* frames, int T, uint8
             if (st_front != st) { CU(cudaEventRecord(h->ev_front[set], st_front)); CU(cudaStreamWaitEvent(st, h->ev_front[set], 0)); }
             h->cur ^= 1;
         } else {
-        const int nseg = (T + h->seg_len - 1) / h->seg_len;
         dim3 g1(g16, nseg, S);
         { ProfScope ps(h, DVC_PROF_FRONT, 1, st);
         if (h->aligned && h->gray_impl == 2)
@@ -1044,6 +1104,8 @@ static int process_batch_impl(dvc_handle* h, const uint8_t* frames, int T, uint8
         }
         CHECK_LAUNCH();
         h->cur ^= 1;
+        }
+        if (!fused) {
         dim3 g2(cdiv(h->plane_words, 256), nseg, S);
         { ProfScope ps(h, DVC_PROF_VOTE, 1, st);
         if (K <= 31) k_window_vote<5><<<g2, 256, 0, st>>>(h->ring, h->ring_cap, H, W, wpr, h->n_masks, (int)(h->n_masks % h->ring_cap), T, K, h->min_counts, bits_a, h->seg_len);
@@ -1057,6 +1119,13 @@ static int process_batch_impl(dvc_handle* h, const uint8_t* frames, int T, uint8
             int rc = launch_morph_chain(h->err, bits_a, bits_b, ST, H, W, h->chain, st);
             if (rc) return rc;
             fin = bits_b;
+        }
+        if (h->flow) {
+            // contours -> filled bounding rectangles (motion_compression_opt.py:93-97): the mask.mp4 frame
+            ProfScope ps(h, DVC_PROF_CCL, 4 * ((ST + RECT_FRAMES - 1) / RECT_FRAMES), st);
+            int rc = flow_rect_launch(h, fin, bits_c, ST, st);
+            if (rc) return rc;
+            fin = bits_c;
         }
         over127 = nonzero = fin;
         if (mask_out) {
@@ -1107,8 +1176,9 @@ static int process_batch_impl(dvc_handle* h, const uint8_t* frames, int T, uint8
     }
     if (overlay || compressed) {
         ProfScope ps(h, DVC_PROF_DEGRADE, 1, st_k4);
+        // flow mode: compress_with_motion's arithmetic (motion_compression_opt.py:152-183) with the rectangle mask
         int rc = launch_degrade(h->err, frames, over127, nonzero, compressed, overlay, ST, H, W, h->cfg.block_size,
-                                h->cfg.quantization_level, DVC_DEGRADE_FD, h->counters_dev, st_k4);
+                                h->cfg.quantization_level, h->flow ? DVC_DEGRADE_MCO : DVC_DEGRADE_FD, h->counters_dev, st_k4);
         if (rc) return rc;
     }
     if (st_k4 != st) {
@@ -1138,6 +1208,7 @@ extern "C" int dvc_process_batch(dvc_handle* h, const uint8_t* frames_dev, int32
     if (n_frames < 0 || n_frames > h->cfg.max_batch) return set_err(h->err, DVC_ERR_INVALID, "dvc_process_batch: n_frames %d outside 0..max_batch (%d)", n_frames, h->cfg.max_batch);
     if (n_frames == 0) return DVC_OK;
     if (!frames_dev) return set_err(h->err, DVC_ERR_INVALID, "dvc_process_batch: null frames");
+    if (h->flow && overlay_dev) return set_err(h->err, DVC_ERR_INVALID, "dvc_process_batch: the flow loop has no overlay output (overlay.mp4 is the unmodified frame)");
     CU(cudaSetDevice(h->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
     if (!h->overlap) {
@@ -1187,6 +1258,7 @@ extern "C" int dvc_process_host(dvc_handle* h, const uint8_t* frames_host, int64
     if (n_frames < 0) return set_err(h->err, DVC_ERR_INVALID, "dvc_process_host: negative n_frames");
     if (n_frames == 0) return DVC_OK;
     if (!frames_host) return set_err(h->err, DVC_ERR_INVALID, "dvc_process_host: null frames");
+    if (h->flow && overlay_host) return set_err(h->err, DVC_ERR_INVALID, "dvc_process_host: the flow loop has no overlay output (overlay.mp4 is the unmodified frame)");
     CU(cudaSetDevice(h->cfg.device));
     int rc = alloc_staging(h);
     if (rc) return rc;
@@ -1483,32 +1555,16 @@ extern "C" int dvc_mask_rectangles_u8(const uint8_t* src, uint8_t* dst, int32_t 
     if (!src || !dst) return set_err(nullptr, DVC_ERR_INVALID, "dvc_mask_rectangles_u8: null pointer");
     if (W > 32767 || H > 32767) return set_err(nullptr, DVC_ERR_UNSUPPORTED, "dvc_mask_rectangles_u8: image larger than 32767");
     cudaStream_t st = (cudaStream_t)stream;
-    const int wpr = words_per_row(W);
-    const size_t pw = (size_t)H * wpr;
+    const size_t pw = (size_t)H * words_per_row(W);
     const int fr = std::min(n, 4);
-    const size_t d = ccl_dense_ints(H, W) * sizeof(int) * fr, o = ccl_overflow_ints(H, W) * sizeof(int) * fr;
-    ScopedAsyncBuf a(st), b(st), pp(st), bbuf(st);
+    ScopedAsyncBuf a(st), b(st), sc(st);
     CU(a.alloc(pw * 4 * n));
     CU(b.alloc(pw * 4 * n));
-    CU(pp.alloc(d + o)); CU(bbuf.alloc(3 * (d + o)));                     // dense + overflow pairs, one allocation each
-    struct { void* p; } p0{pp.p}, pov{(char*)pp.p + d}, bd{bbuf.p}, bo{(char*)bbuf.p + 3 * d};
+    CU(sc.alloc(rect_scratch_bytes(fr, H, W)));
     rc = pack_to_bits(src, (uint32_t*)a.p, n, H, W, st);
     if (rc) return rc;
-    CU(cudaMemsetAsync(b.p, 0, pw * 4 * n, st));
-    BBoxArrays bb;
-    for (int k = 0; k < 3; ++k) { bb.d[k] = (int*)((char*)bd.p + k * d); bb.ov[k] = (int*)((char*)bo.p + k * o); }
-    for (int i0 = 0; i0 < n; i0 += fr) {
-        const int m = std::min(fr, n - i0);
-        dim3 grid(cdiv(pw, 256), m), grow((H + 7) / 8, m);
-        const uint32_t* r = (const uint32_t*)a.p + (size_t)i0 * pw;
-        CU(cudaMemsetAsync(bd.p, 0x7f, 3 * d, st));           // 0x7f7f7f7f: larger than any coordinate or negated coordinate
-        CU(cudaMemsetAsync(bo.p, 0x7f, 3 * o, st));
-        k_ccl_rowlink<false, false><<<grow, 256, 0, st>>>(r, (int*)p0.p, (int*)pov.p, nullptr, nullptr, H, W, wpr, nullptr);
-        k_ccl_union<false, 8><<<CCL_GRID(wpr, H, m), 256, 0, st>>>(r, (int*)p0.p, (int*)pov.p, H, W, wpr, nullptr);
-        k_ccl_bbox<<<grid, 256, 0, st>>>(r, (int*)p0.p, (int*)pov.p, bb, H, W, wpr);
-        k_ccl_paint_rects<<<grid, 256, 0, st>>>(r, (int*)p0.p, (int*)pov.p, bb, (uint32_t*)b.p + (size_t)i0 * pw, H, W, wpr);
-        CHECK_LAUNCH();
-    }
+    rc = launch_rectangles(nullptr, (const uint32_t*)a.p, (uint32_t*)b.p, n, H, W, sc.p, fr, st);
+    if (rc) return rc;
     return unpack_from_bits((const uint32_t*)b.p, dst, n, H, W, st);
 }
 
@@ -1602,7 +1658,7 @@ extern "C" int dvc_begin_stream_frames(dvc_handle* h, const uint8_t* first_frame
     if (h->ring) CU(cudaMemsetAsync(h->ring, 0, h->plane_words * 4 * h->ring_cap * S, st));
     h->n_masks = 0;
     CU(cudaStreamSynchronize(st));
-    return DVC_OK;
+    return h->flow ? flow_rebuild_prev(h) : DVC_OK;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1771,10 +1827,14 @@ struct FlowScratch {
     float2* fl[2];    // [G][H][W] flow of the last two levels
 };
 
-// G pairs, coarse to fine.  Pair p's polynomial pyramids are R0 + p * P * 5 and R1 + p * P * 5.  The finest level's last
-// solve writes flow_out (stride H*W) or mask_out.
-static int flow_pairs(const float* R0, const float* R1, int G, int H, int W, const FlowPlan& pl, double pyr_scale, int winsize,
-                      int iterations, const FlowScratch& sc, float2* flow_out, uint8_t* mask_out, float thr, cudaStream_t st) {
+// G pairs, coarse to fine.  `seq` gives the pyramids of the pairs (FlowPair's R0, R1, first, run, r_stride and run_stride;
+// the level offsets and sizes are filled in here).  The finest level's last solve writes flow_out (stride H*W), mask_out or
+// the bit-planes of `bits`.
+static FlowPair flow_seq(const float* R0, const float* R1, const FlowPlan& pl) {
+    return FlowPair{R0, R1, pl.P * 5, 0, 0, 0, 0, INT_MAX, 0};
+}
+static int flow_pairs(const FlowPair& seq, int G, int H, int W, const FlowPlan& pl, double pyr_scale, int winsize, int iterations,
+                      const FlowScratch& sc, float2* flow_out, uint8_t* mask_out, float thr, const FlowBits& bits, cudaStream_t st) {
     char* ERRBUF = nullptr;
     const size_t WH = (size_t)H * W;
     const int m = winsize / 2;
@@ -1784,7 +1844,12 @@ static int flow_pairs(const float* R0, const float* R1, int G, int H, int W, con
     int cw = 0, ch = 0, cur = 0;
     for (int l = pl.levels; l >= 0; --l) {
         const FlowLevelGeom& g = pl.geo[l];
-        const FlowPair pr{R0 + pl.off[l] * 5, R1 + pl.off[l] * 5, pl.P * 5, WH, g.w, g.h};
+        FlowPair pr = seq;
+        pr.R0 += pl.off[l] * 5;
+        pr.R1 += pl.off[l] * 5;
+        pr.px_stride = WH;
+        pr.w = g.w;
+        pr.h = g.h;
         const dim3 gp(cdiv((size_t)g.w * g.h, 256), G);
         k_flow_matrices<<<gp, 256, 0, st>>>(pr, coarse, cw, ch, coarse ? 1. / ((double)g.w / cw) : 0., coarse ? 1. / ((double)g.h / ch) : 0.,
                                             up, sc.M);
@@ -1793,10 +1858,12 @@ static int flow_pairs(const float* R0, const float* R1, int G, int H, int W, con
             const bool last = it == iterations - 1;
             float2* fo = last ? sc.fl[cur] : nullptr;
             uint8_t* mo = nullptr;
-            if (last && l == 0) { fo = flow_out; mo = mask_out; }
+            FlowBits bo{};
+            if (last && l == 0) { fo = flow_out; mo = mask_out; bo = bits; }
+            const dim3 gs = bo.ring ? dim3(cdiv((size_t)g.h * bo.wpr * 32, 256), G) : gp;
             k_flow_vsum<<<dim3(cdiv((size_t)g.w * 5, 128), G), 128, 0, st>>>(sc.M, sc.V, g.w, g.h, m, WH);
             k_flow_hsum<<<dim3(cdiv((size_t)g.h * 5, 128), G), 128, 0, st>>>(sc.V, sc.S, g.w, g.h, m, WH);
-            k_flow_solve<<<gp, 256, 0, st>>>(pr, sc.S, box, fo, WH, mo, WH, thr, last ? nullptr : sc.M);
+            k_flow_solve<<<gs, 256, 0, st>>>(pr, sc.S, box, fo, WH, mo, WH, thr, last ? nullptr : sc.M, bo);
             CHECK_LAUNCH();
         }
         coarse = sc.fl[cur];
@@ -1844,7 +1911,9 @@ extern "C" int dvc_farneback_flow_f32(const uint8_t* prev, const uint8_t* next, 
         const int g = std::min(G, n - i0);
         if ((rc = flow_pyramids(prev + i0 * WH, g, H, W, pl, sc.img, sc.R, st))) return rc;
         if ((rc = flow_pyramids(next + i0 * WH, g, H, W, pl, sc.img, R1, st))) return rc;
-        if ((rc = flow_pairs(sc.R, R1, g, H, W, pl, pyr_scale, winsize, iterations, sc, (float2*)flow + i0 * WH, nullptr, 0.f, st))) return rc;
+        if ((rc = flow_pairs(flow_seq(sc.R, R1, pl), g, H, W, pl, pyr_scale, winsize, iterations, sc, (float2*)flow + i0 * WH, nullptr, 0.f,
+                             FlowBits{}, st)))
+            return rc;
     }
     return DVC_OK;
 }
@@ -1869,8 +1938,151 @@ extern "C" int dvc_flow_masks_u8(const uint8_t* gray, uint8_t* mask, int32_t n, 
         const int g = std::min(G, n - i0);
         if (i0 > 0) CU(cudaMemcpyAsync(sc.R, sc.R + (size_t)G * RF, RF * sizeof(float), cudaMemcpyDeviceToDevice, st));
         if ((rc = flow_pyramids(gray + (i0 + 1) * WH, g, H, W, pl, sc.img, sc.R + RF, st))) return rc;
-        if ((rc = flow_pairs(sc.R, sc.R + RF, g, H, W, pl, pyr_scale, winsize, iterations, sc, nullptr, mask + i0 * WH, flow_threshold, st)))
+        if ((rc = flow_pairs(flow_seq(sc.R, sc.R + RF, pl), g, H, W, pl, pyr_scale, winsize, iterations, sc, nullptr, mask + i0 * WH,
+                             flow_threshold, FlowBits{}, st)))
             return rc;
     }
     return DVC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// DVC_MODE_FLOW: temporal_smoothing_flow + compress_with_motion's arithmetic (motion_compression_opt.py:65-101,152-183)
+// ------------------------------------------------------------------------------------------------
+// Pairs per flow launch group of a handle: all S * max_batch pairs of a batch, as long as the group's M / V / S / flow scratch
+// (116 bytes per pixel and pair) stays within FLOW_GROUP_BYTES.  More pairs per launch give the serial box-sum walks more
+// threads; at 1080p the budget holds 17 pairs.
+static constexpr size_t FLOW_GROUP_BYTES = (size_t)4 << 30;
+static int flow_handle_group(int pairs, int H, int W) {
+    const size_t per_pair = (size_t)H * W * (20 + 80 + 16);
+    return (int)std::max<size_t>(1, std::min<size_t>({(size_t)pairs, FLOW_GROUP_BYTES / per_pair, 4096}));
+}
+
+struct FlowLoop {
+    FlowPlan pl;
+    double pyr_scale = 0.3;
+    int winsize = 9, iterations = 2;
+    float thr = 0.5f;
+    int G = 1;                    // pairs per launch group (flow_handle_group)
+    uint8_t* gray = nullptr;      // [S][max_batch] gray planes of the batch
+    float* R = nullptr;           // [S][max_batch + 1] polynomial pyramids; slot 0 = the frame before the batch
+    FlowScratch sc{};             // img [max_batch][H][W], M / V / S / flow for G pairs (sc.R = R)
+    void* rect = nullptr;         // rectangle kernels' scratch, rect_frames planes
+    int rect_frames = 1;
+};
+
+static int flow_alloc_pyramids(dvc_handle* h) {
+    char* ERRBUF = h->err;
+    FlowLoop& f = *h->flow;
+    cudaFree(f.R);
+    f.R = nullptr;
+    CU(cudaMalloc(&f.R, (size_t)h->S * (h->cfg.max_batch + 1) * f.pl.P * 20));
+    f.sc.R = f.R;
+    return DVC_OK;
+}
+
+static int flow_create(dvc_handle* h) {
+    char* ERRBUF = h->err;
+    h->flow = new FlowLoop();
+    FlowLoop& f = *h->flow;
+    const int S = h->S, mb = h->cfg.max_batch;
+    const size_t WH = h->plane_bytes;
+    // the call site's parameters (motion_compression_opt.py:65,72-81); dvc_set_flow_params changes them
+    int rc = flow_plan("dvc_create", 0, h->H, h->W, f.pyr_scale, 2, f.winsize, f.iterations, 5, 1.1, 0, f.pl);
+    if (rc) return set_err(h->err, rc, "%s", std::string(g_err).c_str());
+    f.G = flow_handle_group(S * mb, h->H, h->W);
+    f.rect_frames = std::min(S * mb, RECT_FRAMES);
+    CU(cudaMalloc(&f.gray, (size_t)S * mb * WH));
+    CU(cudaMalloc(&f.sc.img, (size_t)mb * WH * 4));
+    CU(cudaMalloc(&f.sc.M, (size_t)f.G * WH * 20));
+    CU(cudaMalloc(&f.sc.V, (size_t)f.G * WH * 80));
+    f.sc.S = f.sc.V + (size_t)f.G * WH * 5;
+    CU(cudaMalloc(&f.sc.fl[0], (size_t)f.G * WH * 16));
+    f.sc.fl[1] = f.sc.fl[0] + (size_t)f.G * WH;
+    CU(cudaMalloc(&f.rect, rect_scratch_bytes(f.rect_frames, h->H, h->W)));
+    if ((rc = flow_alloc_pyramids(h))) return rc;
+    return flow_rebuild_prev(h);
+}
+
+static void flow_destroy(dvc_handle* h) {
+    if (!h->flow) return;
+    FlowLoop& f = *h->flow;
+    cudaFree(f.gray); cudaFree(f.R); cudaFree(f.sc.img); cudaFree(f.sc.M); cudaFree(f.sc.V); cudaFree(f.sc.fl[0]); cudaFree(f.rect);
+    delete h->flow;
+    h->flow = nullptr;
+}
+
+// Every stream's pyramid of its prev_gray into slot 0 (after begin_stream*, set_state and a parameter change).  Synchronous.
+static int flow_rebuild_prev(dvc_handle* h) {
+    char* ERRBUF = h->err;
+    FlowLoop& f = *h->flow;
+    const size_t RF = f.pl.P * 5;
+    for (int s = 0; s < h->S; ++s) {
+        int rc = flow_pyramids(h->prev_gray[h->cur] + (size_t)s * h->plane_bytes, 1, h->H, h->W, f.pl, f.sc.img,
+                               f.R + (size_t)s * (h->cfg.max_batch + 1) * RF, h->s_mask);
+        if (rc) return set_err(h->err, rc, "%s", std::string(g_err).c_str());
+    }
+    CU(cudaStreamSynchronize(h->s_mask));
+    return DVC_OK;
+}
+
+// motion_compression_opt.py:71-83 for T frames of each stream: gray, each frame's pyramid built once, the flow of every pair
+// (frame before, frame) in groups of G pairs across the streams, and the thresholded magnitude written by the last solve
+// into the ring slot of its frame.  The last frame's pyramid and gray carry over to the next batch.
+static int flow_front(dvc_handle* h, const uint8_t* frames, int T, cudaStream_t st) {
+    char* ERRBUF = h->err;
+    FlowLoop& f = *h->flow;
+    const int S = h->S, H = h->H, W = h->W, mb = h->cfg.max_batch, L = f.pl.levels;
+    const size_t WH = h->plane_bytes, RF = f.pl.P * 5;
+    const int pairs = S * T, groups = (pairs + f.G - 1) / f.G;
+    ProfScope ps(h, DVC_PROF_FRONT, S * (1 + 2 * (L + 1)) + groups * (L + 1) * (1 + 3 * f.iterations), st);
+    const dim3 g(cdiv((size_t)((W + 15) / 16) * H, 256), T);
+    for (int s = 0; s < S; ++s) {
+        uint8_t* gray = f.gray + (size_t)s * mb * WH;
+        if (h->aligned) k_bgr2gray<true><<<g, 256, 0, st>>>(frames + (size_t)s * T * h->frame_bytes, gray, H, W);
+        else k_bgr2gray<false><<<g, 256, 0, st>>>(frames + (size_t)s * T * h->frame_bytes, gray, H, W);
+        CHECK_LAUNCH();
+        int rc = flow_pyramids(gray, T, H, W, f.pl, f.sc.img, f.R + ((size_t)s * (mb + 1) + 1) * RF, st);
+        if (rc) return set_err(h->err, rc, "%s", std::string(g_err).c_str());
+    }
+    FlowPair seq = flow_seq(f.R, f.R + RF, f.pl);
+    seq.run = T;
+    seq.run_stride = (size_t)(mb + 1) * RF;
+    const FlowBits bits{h->ring, (size_t)h->ring_cap * h->plane_words, h->plane_words, h->n_masks, h->ring_cap, h->wpr};
+    for (int i0 = 0; i0 < pairs; i0 += f.G) {
+        seq.first = i0;
+        int rc = flow_pairs(seq, std::min(f.G, pairs - i0), H, W, f.pl, f.pyr_scale, f.winsize, f.iterations, f.sc, nullptr, nullptr,
+                            f.thr, bits, st);
+        if (rc) return set_err(h->err, rc, "%s", std::string(g_err).c_str());
+    }
+    for (int s = 0; s < S; ++s) {
+        float* R = f.R + (size_t)s * (mb + 1) * RF;
+        CU(cudaMemcpyAsync(R, R + (size_t)T * RF, RF * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        CU(cudaMemcpyAsync(h->prev_gray[h->cur] + (size_t)s * WH, f.gray + ((size_t)s * mb + T - 1) * WH, WH, cudaMemcpyDeviceToDevice, st));
+    }
+    return DVC_OK;
+}
+
+static int flow_rect_launch(dvc_handle* h, const uint32_t* src, uint32_t* dst, int n, cudaStream_t st) {
+    return launch_rectangles(h->err, src, dst, n, h->H, h->W, h->flow->rect, h->flow->rect_frames, st);
+}
+
+extern "C" int dvc_set_flow_params(dvc_handle* h, float flow_threshold, double pyr_scale, int32_t levels, int32_t winsize,
+                                   int32_t iterations, int32_t poly_n, double poly_sigma, int32_t flags) {
+    char* ERRBUF = h ? h->err : nullptr;
+    if (!h) return set_err(nullptr, DVC_ERR_INVALID, "dvc_set_flow_params: null handle");
+    if (!h->flow) return set_err(h->err, DVC_ERR_INVALID, "dvc_set_flow_params: the handle runs mode %d, not DVC_MODE_FLOW", h->cfg.mode);
+    FlowPlan pl;
+    int rc = flow_plan("dvc_set_flow_params", 0, h->H, h->W, pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags, pl);
+    if (rc) return set_err(h->err, rc, "%s", std::string(g_err).c_str());
+    CU(cudaSetDevice(h->cfg.device));
+    CU(handle_join(h));
+    FlowLoop& f = *h->flow;
+    const bool resize = pl.P != f.pl.P;
+    f.pl = pl;
+    f.pyr_scale = pyr_scale;
+    f.winsize = winsize;
+    f.iterations = iterations;
+    f.thr = flow_threshold;
+    if (resize && (rc = flow_alloc_pyramids(h))) return rc;
+    return flow_rebuild_prev(h);
 }

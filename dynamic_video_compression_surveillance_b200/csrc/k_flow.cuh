@@ -6,7 +6,7 @@
 //   polynomial    separable Gaussian-weighted fit, replicated borders, 5 coefficients per pixel       k_flow_poly
 //   matrices      R1 sampled bilinearly at x + flow, border taper, M = (G11, G12, G22, h1, h2)       k_flow_matrices
 //   box sum       cv2's vertical and horizontal running sums, in cv2's order                         k_flow_vsum, k_flow_hsum
-//   solve         regularised 2x2 solve (+1e-3), then either the next matrices or the mask           k_flow_solve
+//   solve         regularised 2x2 solve (+1e-3), then the next matrices, or the mask as bytes or bits   k_flow_solve
 // Float products and sums that cv2 rounds one by one are written with __fmul_rn / __fadd_rn so that ptxas cannot
 // contract them.  Every sum has a fixed order: results are identical from run to run.
 #pragma once
@@ -201,13 +201,29 @@ DEVI void flow_matrix(const float* __restrict__ R0, const float* __restrict__ R1
     M[4] = __fadd_rn(__fmul_rn(r6, r2), __fmul_rn(r5, r3));
 }
 
-// Pair p reads R0 + p * r_stride and R1 + p * r_stride (sequence: R1 = R0 + one frame); M, V and flow are [p][h][w][...]
-// with a stride of `px_stride` pixels.
+// Pair p of a launch is pair q = first + p of the sequence.  Pairs come in runs of `run` (one run per stream of a handle's
+// lock-step group): pair q reads R0 + off and R1 + off with off = (q / run) * run_stride + (q % run) * r_stride (sequence:
+// R1 = R0 + one frame).  M, V and flow are [p][h][w][...] with a stride of `px_stride` pixels.
 struct FlowPair {
     const float* R0;
     const float* R1;
     size_t r_stride, px_stride;
     int w, h;
+    int first, run;
+    size_t run_stride;
+};
+DEVI size_t flow_pair_offset(const FlowPair& pr, int p) {
+    const int q = pr.first + p;
+    return (size_t)(q / pr.run) * pr.run_stride + (size_t)(q % pr.run) * pr.r_stride;
+}
+
+// Bit-plane output of the mask (the layout of common.cuh): pair q writes frame f = f0 + q % run of stream q / run into ring
+// slot f % cap of that stream, ring + (q / run) * stream_words + (f % cap) * plane_words.
+struct FlowBits {
+    uint32_t* ring;
+    size_t stream_words, plane_words;
+    long long f0;
+    int cap, wpr;
 };
 
 // grid (ceil(w*h / 256), pairs): the level's starting flow (zero, or the coarser level's flow resized INTER_LINEAR and
@@ -239,7 +255,8 @@ __global__ void __launch_bounds__(256) k_flow_matrices(FlowPair pr, const float2
         dy = __fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(hy0, b0), __fmul_rn(hy1, fy)), up), 0.f);
     }
     float m[5];
-    flow_matrix(pr.R0 + p * pr.r_stride, pr.R1 + p * pr.r_stride, pr.w, pr.h, x, y, dx, dy, m);
+    const size_t ro = flow_pair_offset(pr, (int)p);
+    flow_matrix(pr.R0 + ro, pr.R1 + ro, pr.w, pr.h, x, y, dx, dy, m);
     float* d = M + (p * pr.px_stride + idx) * 5;
 #pragma unroll
     for (int c = 0; c < 5; ++c) d[c] = m[c];
@@ -288,33 +305,59 @@ __global__ void __launch_bounds__(128) k_flow_hsum(const double* __restrict__ V,
 
 // ---- solve ------------------------------------------------------------------------------------------------------------
 // Box sums scaled by 1 / winsize^2, then the regularised solve.  Outputs: the flow (flow != NULL), the mask
-// 255 * (|flow| > thr) (mask != NULL), and the matrices of the new flow for the next iteration (M != NULL).
-// grid (ceil(w*h / 256), pairs)
+// 255 * (|flow| > thr) as bytes (mask != NULL) or as bits (bits.ring != NULL), and the matrices of the new flow for the next
+// iteration (M != NULL).
+// grid (ceil(w*h / 256), pairs); with bits.ring, grid (ceil(h * wpr * 32 / 256), pairs): one thread per bit of the padded
+// rows, so that the ballot of a warp is one word of the plane (bits of columns >= w are zero)
 __global__ void __launch_bounds__(256) k_flow_solve(FlowPair pr, const double* __restrict__ S, double scale,
                                                     float2* __restrict__ flow, size_t flow_stride, uint8_t* __restrict__ mask,
-                                                    size_t mask_stride, float thr, float* __restrict__ M) {
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+                                                    size_t mask_stride, float thr, float* __restrict__ M, FlowBits bits) {
     const int w = pr.w, h = pr.h;
-    if (idx >= w * h) return;
-    const int x = idx % w, y = idx / w;
     const size_t p = blockIdx.y;
-    const double* s = S + (p * pr.px_stride + idx) * 5;
-    const double g11 = __dmul_rn(s[0], scale), g12 = __dmul_rn(s[1], scale), g22 = __dmul_rn(s[2], scale);
-    const double h1 = __dmul_rn(s[3], scale), h2 = __dmul_rn(s[4], scale);
-    const double idet = 1.0 / __dadd_rn(__dsub_rn(__dmul_rn(g11, g22), __dmul_rn(g12, g12)), 1e-3);
-    const float fx = (float)__dmul_rn(__dsub_rn(__dmul_rn(g11, h2), __dmul_rn(g12, h1)), idet);
-    const float fy = (float)__dmul_rn(__dsub_rn(__dmul_rn(g22, h1), __dmul_rn(g12, h2)), idet);
-    if (flow) flow[p * flow_stride + idx] = make_float2(fx, fy);
-    if (mask) {                                                   // cv2.cartToPolar magnitude, then mag > thr
-        const float mag = __fsqrt_rn(__fadd_rn(__fmul_rn(fx, fx), __fmul_rn(fy, fy)));
-        mask[p * mask_stride + idx] = mag > thr ? 255 : 0;
+    int x, y;
+    if (bits.ring) {
+        const int rw = bits.wpr * 32, v = blockIdx.x * blockDim.x + threadIdx.x;
+        y = v / rw;
+        x = v - y * rw;
+        if (y >= h) return;                                       // whole warps: rw is a multiple of 32
+    } else {
+        const int v = blockIdx.x * blockDim.x + threadIdx.x;
+        if (v >= w * h) return;
+        x = v % w;
+        y = v / w;
     }
-    if (M) {
-        float mm[5];
-        flow_matrix(pr.R0 + p * pr.r_stride, pr.R1 + p * pr.r_stride, w, h, x, y, fx, fy, mm);
-        float* d = M + (p * pr.px_stride + idx) * 5;
+    bool on = false;
+    if (x < w) {
+        const int idx = y * w + x;
+        const double* s = S + (p * pr.px_stride + idx) * 5;
+        const double g11 = __dmul_rn(s[0], scale), g12 = __dmul_rn(s[1], scale), g22 = __dmul_rn(s[2], scale);
+        const double h1 = __dmul_rn(s[3], scale), h2 = __dmul_rn(s[4], scale);
+        const double idet = 1.0 / __dadd_rn(__dsub_rn(__dmul_rn(g11, g22), __dmul_rn(g12, g12)), 1e-3);
+        const float fx = (float)__dmul_rn(__dsub_rn(__dmul_rn(g11, h2), __dmul_rn(g12, h1)), idet);
+        const float fy = (float)__dmul_rn(__dsub_rn(__dmul_rn(g22, h1), __dmul_rn(g12, h2)), idet);
+        if (flow) flow[p * flow_stride + idx] = make_float2(fx, fy);
+        if (mask || bits.ring) {                                  // cv2.cartToPolar magnitude, then mag > thr
+            const float mag = __fsqrt_rn(__fadd_rn(__fmul_rn(fx, fx), __fmul_rn(fy, fy)));
+            on = mag > thr;
+            if (mask) mask[p * mask_stride + idx] = on ? 255 : 0;
+        }
+        if (M) {
+            float mm[5];
+            const size_t ro = flow_pair_offset(pr, (int)p);
+            flow_matrix(pr.R0 + ro, pr.R1 + ro, w, h, x, y, fx, fy, mm);
+            float* d = M + (p * pr.px_stride + idx) * 5;
 #pragma unroll
-        for (int c = 0; c < 5; ++c) d[c] = mm[c];
+            for (int c = 0; c < 5; ++c) d[c] = mm[c];
+        }
+    }
+    if (bits.ring) {
+        const uint32_t word = __ballot_sync(0xffffffffu, on);
+        if ((threadIdx.x & 31) == 0) {
+            const int q = pr.first + (int)p;
+            const long long f = bits.f0 + q % pr.run;
+            bits.ring[(size_t)(q / pr.run) * bits.stream_words + (size_t)(f % bits.cap) * bits.plane_words + (size_t)y * bits.wpr +
+                      (x >> 5)] = word;
+        }
     }
 }
 

@@ -2,8 +2,9 @@
 here (windows.py:13,151).  Contracts follow motion_compression_opt.py:8-247.  GPU (C ABI): the K-frame window
 vote (:84-86), close/open (:89-90), contours -> bounding rectangles (:93-97) and all of compress_with_motion's
 arithmetic (:152-183).  Farneback flow + cartToPolar + threshold (:71-83) run on the host by default, as in the
-reference; ``flow_device="gpu"`` moves gray conversion, flow and masks to the GPU (host_loop.flow_masks_gpu), which agrees
-with cv2 about as closely as cv2's own dispatch paths agree with each other (DESIGN.md section 6).  Codecs stay on the host.
+reference; ``flow_device="gpu"`` runs the whole of motion detection (:65-97: gray, flow, masks, vote, close/open,
+rectangles) in one flow-mode FramePipeline per video, whose flow agrees with cv2 about as closely as cv2's own dispatch
+paths agree with each other (DESIGN.md section 6).  Codecs stay on the host.
 """
 import logging
 import os
@@ -18,6 +19,7 @@ if _ROOT not in sys.path:
     sys.path.insert(0, _ROOT)
 
 from dynamic_video_compression_surveillance_b200 import host_loop as _hl  # noqa: E402
+from dynamic_video_compression_surveillance_b200 import pipeline as _P  # noqa: E402
 
 _CHUNK = 16
 _FARNEBACK = (0.3, 2, 9, 2, 5, 1.1, 0)          # pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags (:72-81)
@@ -36,7 +38,7 @@ def _open_writer(path, fps, size, color=True):
 def temporal_smoothing_flow(video_path, output_dir, flow_threshold=0.5, alpha_fraction=0.2, window_size=30, morph_kernel=2,
                             save_name="overlay.mp4", mask_save_name="mask.mp4", flow_device="cpu"):
     """motion_compression_opt.py:29-109 -> (frames, total seconds, seconds per frame).  flow_device "cpu" (default):
-    cv2 Farneback per frame on the host; "gpu": gray, flow and raw masks of each chunk on the GPU."""
+    cv2 Farneback per frame on the host; "gpu": every step from gray to the rectangle mask on the GPU."""
     if flow_device not in ("cpu", "gpu"):
         raise ValueError(f"flow_device must be 'cpu' or 'gpu', not {flow_device!r}")
     t_start = time.time()
@@ -54,8 +56,53 @@ def temporal_smoothing_flow(video_path, output_dir, flow_threshold=0.5, alpha_fr
         cap.release()
         return 0, 0, 0
 
-    on_gpu = flow_device == "gpu"
-    prev_gray = _hl.first_gray_gpu(frame) if on_gpu else cv2.cvtColor(frame, cv2.COLOR_BGR2GRAY)
+    if flow_device == "gpu":
+        n_frames = _motion_masks_gpu(cap, frame, out_overlay, out_mask, flow_threshold, alpha_fraction, window_size, morph_kernel)
+    else:
+        n_frames = _motion_masks_host_flow(cap, frame, out_overlay, out_mask, flow_threshold, alpha_fraction, window_size,
+                                           morph_kernel)
+    cap.release()
+    out_overlay.release()
+    out_mask.release()
+    total = time.time() - t_start
+    avg = total / n_frames if n_frames > 0 else 0
+    logging.info(f"Temporal smoothing flow completed for '{os.path.basename(video_path)}' in {total:.2f} seconds. Frames processed: {n_frames}")
+    return n_frames, total, avg
+
+
+def _motion_masks_gpu(cap, first, out_overlay, out_mask, flow_threshold, alpha_fraction, window_size, morph_kernel):
+    """motion_compression_opt.py:65-99 through one flow-mode FramePipeline: chunks of decoded frames in, rectangle masks
+    out; prev_gray, the raw-mask window and the last frame's flow pyramid stay on the GPU between chunks."""
+    h, w = first.shape[:2]
+    inp, masks = _P.pinned_empty((_CHUNK, h, w, 3)), _P.pinned_empty((_CHUNK, h, w))
+    inp_v, masks_v = inp.numpy(), masks.numpy()
+    n_frames = 0
+    with _P.FramePipeline(w, h, "flow", window_size=window_size, alpha_fraction=alpha_fraction, morph_kernel=morph_kernel,
+                          max_batch=_CHUNK, flow_threshold=flow_threshold, farneback=_FARNEBACK) as pipe:
+        pipe.begin_stream_frames(first)                   # :60
+        while True:
+            n = 0
+            while n < _CHUNK:
+                ok, frame = cap.read()
+                if not ok:
+                    break
+                inp_v[n] = frame
+                n += 1
+            if n == 0:
+                break
+            pipe.process_host(inp[:n], mask=masks[:n])
+            for i in range(n):
+                n_frames += 1
+                out_overlay.write(inp_v[i])
+                out_mask.write(masks_v[i])
+            if n < _CHUNK:
+                break
+    return n_frames
+
+
+def _motion_masks_host_flow(cap, first, out_overlay, out_mask, flow_threshold, alpha_fraction, window_size, morph_kernel):
+    """motion_compression_opt.py:65-99 with cv2's Farneback on the host and the mask steps on the GPU, a chunk at a time."""
+    prev_gray = cv2.cvtColor(first, cv2.COLOR_BGR2GRAY)
     n_frames, history, exhausted = 0, [], False
     while not exhausted:
         frames, raws = [], []
@@ -64,18 +111,14 @@ def temporal_smoothing_flow(video_path, output_dir, flow_threshold=0.5, alpha_fr
             if not ok:
                 exhausted = True
                 break
-            if not on_gpu:
-                gray = cv2.cvtColor(frame, cv2.COLOR_BGR2GRAY)
-                flow = cv2.calcOpticalFlowFarneback(prev_gray, gray, None, *_FARNEBACK)
-                mag, _ = cv2.cartToPolar(flow[..., 0], flow[..., 1])
-                raws.append((mag > flow_threshold).astype(np.uint8) * 255)
-                prev_gray = gray
+            gray = cv2.cvtColor(frame, cv2.COLOR_BGR2GRAY)
+            flow = cv2.calcOpticalFlowFarneback(prev_gray, gray, None, *_FARNEBACK)
+            mag, _ = cv2.cartToPolar(flow[..., 0], flow[..., 1])
+            raws.append((mag > flow_threshold).astype(np.uint8) * 255)
+            prev_gray = gray
             frames.append(frame)
         if not frames:
             break
-        if on_gpu:
-            masks, prev_gray = _hl.flow_masks_gpu(frames, prev_gray, flow_threshold, _FARNEBACK)
-            raws = list(masks)
         rects = _hl.smooth_rect_masks_gpu(raws, history, window_size, alpha_fraction, morph_kernel)
         seen = history + raws
         # while the stream is shorter than the window keep all of it (the vote's L = len(deque) must match);
@@ -85,13 +128,7 @@ def temporal_smoothing_flow(video_path, output_dir, flow_threshold=0.5, alpha_fr
             n_frames += 1
             out_overlay.write(frame)
             out_mask.write(mask)
-    cap.release()
-    out_overlay.release()
-    out_mask.release()
-    total = time.time() - t_start
-    avg = total / n_frames if n_frames > 0 else 0
-    logging.info(f"Temporal smoothing flow completed for '{os.path.basename(video_path)}' in {total:.2f} seconds. Frames processed: {n_frames}")
-    return n_frames, total, avg
+    return n_frames
 
 
 def compress_with_motion(input_video, mask_video, output_dir):

@@ -14,10 +14,11 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (DVC_DEGRADE_FD, DVC_DEGRADE_MCO, DVC_MODE_FD, DVC_MODE_WINDOW, DVC_SHAPE_ELLIPSE, DVC_SHAPE_RECT,
-                   DvcConfig, DvcCounters, check)
+from ._lib import (DVC_DEGRADE_FD, DVC_DEGRADE_MCO, DVC_MODE_FD, DVC_MODE_FLOW, DVC_MODE_WINDOW, DVC_SHAPE_ELLIPSE,
+                   DVC_SHAPE_RECT, DvcConfig, DvcCounters, check)
 
-_MODES = {"fd": DVC_MODE_FD, "window": DVC_MODE_WINDOW}
+_MODES = {"fd": DVC_MODE_FD, "window": DVC_MODE_WINDOW, "flow": DVC_MODE_FLOW}
+CALL_SITE_FARNEBACK = (0.3, 2, 9, 2, 5, 1.1, 0)      # motion_compression_opt.py:72-81
 _SHAPES = {"rect": DVC_SHAPE_RECT, "ellipse": DVC_SHAPE_ELLIPSE}
 _MORPH_OPS = {"erode": 0, "dilate": 1, "open": 2, "close": 3}
 
@@ -51,14 +52,26 @@ class FramePipeline:
     ``n_streams=S > 1`` makes the object a lock-step group of S independent camera streams (the reference processes its
     files one after another, windows.py:142-160; BASELINE config 4) whose kernels share every launch: all frame / output
     arrays gain a leading stream axis ([S, T, H, W, 3]), ``begin_stream`` takes [S, H, W] planes, and every call
-    advances each stream by T frames.  Results per stream equal those of S separate pipelines."""
+    advances each stream by T frames.  Results per stream equal those of S separate pipelines.
 
-    def __init__(self, width: int, height: int, mode: str = "fd", *, block_size: int = 4, motion_threshold: float = 0.5,
-                 min_area: float = 500, kernel_size: int = 7, release_factor: float = 0.5,
-                 quantization_level: float = 100, window_size: int = 30, alpha_fraction: float = 0.2,
-                 morph_kernel: int = 2, morph_shape: str = "ellipse", max_batch: int = 16, device: int | None = None,
-                 src_size: tuple | None = None, n_streams: int = 1):
+    ``mode="flow"`` runs temporal_smoothing_flow with compress_with_motion's arithmetic (motion_compression_opt.py:65-101,
+    152-183; BASELINE config 5): ``mask`` receives the rectangle mask (the mask.mp4 frame), ``compressed`` the degraded frame,
+    and there is no overlay (the reference's overlay.mp4 is the unmodified frame).  ``flow_threshold`` and ``farneback``
+    (pyr_scale, levels, winsize, iterations, poly_n, poly_sigma, flags) are the call's Farneback arguments; block_size
+    defaults to 8 and kernel_size to 0 in this mode (other values raise the library's error)."""
+
+    def __init__(self, width: int, height: int, mode: str = "fd", *, block_size: int | None = None,
+                 motion_threshold: float = 0.5, min_area: float = 500, kernel_size: int | None = None,
+                 release_factor: float = 0.5, quantization_level: float = 100, window_size: int = 30,
+                 alpha_fraction: float = 0.2, morph_kernel: int = 2, morph_shape: str = "ellipse", max_batch: int = 16,
+                 device: int | None = None, src_size: tuple | None = None, n_streams: int = 1, flow_threshold: float = 0.5,
+                 farneback: tuple = CALL_SITE_FARNEBACK):
         _require_cuda()
+        flow = mode == "flow"
+        if block_size is None:
+            block_size = 8 if flow else 4
+        if kernel_size is None:
+            kernel_size = 0 if flow else 7
         self._lib = _lib.load()
         self.width, self.height, self.mode = int(width), int(height), mode
         self.device = torch.cuda.current_device() if device is None else int(device)
@@ -81,6 +94,23 @@ class FramePipeline:
         self.max_batch = int(max_batch)
         self._h = C.c_void_p()
         check(self._lib.dvc_create(C.byref(cfg), C.byref(self._h)))
+        if flow:
+            self.flow_threshold, self.farneback = float(flow_threshold), tuple(farneback)
+            if (self.flow_threshold, self.farneback) != (0.5, CALL_SITE_FARNEBACK):
+                self.set_flow_params(self.flow_threshold, self.farneback)
+
+    def set_flow_params(self, flow_threshold: float = 0.5, farneback: tuple = CALL_SITE_FARNEBACK):
+        """Flow mode: the threshold and the Farneback arguments (pyr_scale, levels, winsize, iterations, poly_n, poly_sigma,
+        flags) of motion_compression_opt.py:72-83."""
+        self._check(self._lib.dvc_set_flow_params(self._h, float(flow_threshold), *_flow_args(*farneback)))
+        self.flow_threshold, self.farneback = float(flow_threshold), tuple(farneback)
+
+    @property
+    def flow_group(self) -> int:
+        """Flow mode: Farneback pairs per launch group, the library's rule (DESIGN.md section 6c): every pair of a batch,
+        n_streams * max_batch, as long as the group's scratch of 116 bytes per pixel and pair stays within 4 GiB."""
+        per_pair = self.width * self.height * 116
+        return max(1, min(self.n_streams * self.max_batch, (4 << 30) // per_pair, 4096))
 
     # -- lifecycle ----------------------------------------------------------------------------------
     def close(self):

@@ -50,7 +50,19 @@ enum {
      * (frame_differencing.py:92,96-97) -> K-frame window vote -> close/open
      * (motion_compression_opt.py:61-62,84-90) -> dilate -> overlay + block-DCT degrade
      * (frame_differencing.py:106,110-130). */
-    DVC_MODE_WINDOW = 1
+    DVC_MODE_WINDOW = 1,
+    /* temporal_smoothing_flow + compress_with_motion, motion_compression_opt.py:65-101 with the masks passed as arrays
+     * (BASELINE config 5): gray (:71) -> Farneback flow, |flow| > float32(threshold) (:72-83, as dvc_flow_masks_u8) ->
+     * window vote over the last min(t, K) raw masks (:84-86) -> MORPH_CLOSE, MORPH_OPEN (:89-90) -> contours -> filled
+     * bounding rectangles (:93-97, the mask.mp4 frame, mask_dev) -> compress_with_motion's degrade (:152-183, DVC_DEGRADE_MCO,
+     * 8x8) of the frame with that mask (compressed_dev).  Used fields: window_size, alpha_fraction, morph_kernel, morph_shape,
+     * quantization_level, max_batch, n_streams, device.  block_size must be 8 (else DVC_ERR_UNSUPPORTED), kernel_size 0 (else
+     * DVC_ERR_INVALID: no dilate), src_width / src_height 0 (else DVC_ERR_UNSUPPORTED); overlay_dev / overlay_host must be
+     * NULL (DVC_ERR_INVALID: the reference's overlay.mp4 is the unmodified frame, :99).  Farneback parameters and threshold:
+     * dvc_set_flow_params.  State: prev_gray and the raw-mask window as in DVC_MODE_WINDOW; the handle also keeps each
+     * stream's last polynomial pyramid, rebuilt from prev_gray by dvc_begin_stream*, dvc_set_state and dvc_set_flow_params.
+     * All scratch is allocated by dvc_create (DESIGN.md section 6c gives the sizes). */
+    DVC_MODE_FLOW = 2
 };
 
 enum { DVC_MORPH_ERODE = 0, DVC_MORPH_DILATE = 1, DVC_MORPH_OPEN = 2, DVC_MORPH_CLOSE = 3 };
@@ -125,11 +137,20 @@ int dvc_set_state(dvc_handle* h, const void* host_buf, size_t bytes);
 int dvc_get_counters(dvc_handle* h, dvc_counters* out);   /* synchronises the handle's streams */
 int dvc_reset_counters(dvc_handle* h);
 
+/* Farneback parameters and threshold of a DVC_MODE_FLOW handle (motion_compression_opt.py:65,72-81): the arguments of
+ * cv2.calcOpticalFlowFarneback, with the argument rules and error codes of dvc_farneback_flow_f32.  At create the handle holds
+ * the call site's values, threshold 0.5 and (0.3, 2, 9, 2, 5, 1.1, 0).  DVC_ERR_INVALID on a handle of another mode.
+ * Synchronous: rebuilds every stream's kept pyramid from its prev_gray, the stream state is otherwise unchanged. */
+int dvc_set_flow_params(dvc_handle* h, float flow_threshold, double pyr_scale, int32_t levels, int32_t winsize, int32_t iterations,
+                        int32_t poly_n, double poly_sigma, int32_t flags);
+
 /* ---- the loop body: frame_differencing.py:85-133 for n_frames consecutive frames ----------------
  * frames_dev   [n][H][W][3]  input frames (after cap.read(), frame_differencing.py:87)
  * overlay_dev  [n][H][W][3]  what mask_out.write() receives (:110-112), may be NULL
  * compressed_dev [n][H][W][3] what final_out.write() receives (:115-131), may be NULL
- * mask_dev     [n][H][W]     accumulated_mask after each frame (FD) / final mask (WINDOW), may be NULL
+ * mask_dev     [n][H][W]     accumulated_mask after each frame (FD) / final mask (WINDOW) / rectangle mask (FLOW), may be NULL
+ * The degrade kernel runs only when overlay_dev or compressed_dev is given: with both NULL the counters advance frames, pixels
+ * and blocks but not motion_pixels and static_blocks.
  * n_frames <= cfg.max_batch.  When W % 16 == 0, frames_dev must be 16-byte aligned: the front kernels load it
  * 16 bytes at a time. */
 int dvc_process_batch(dvc_handle* h, const uint8_t* frames_dev, int32_t n_frames, uint8_t* overlay_dev,
@@ -151,12 +172,12 @@ int dvc_process_host(dvc_handle* h, const uint8_t* frames_host, int64_t n_frames
 /* ---- measurement hooks (bench.py): per kernel group, time between CUDA events recorded on the launching
  *      stream around the group's launches inside dvc_process_batch / dvc_process_host ------------- */
 enum {
-    DVC_PROF_FRONT = 0,   /* K1: gray (+blur5) (+absdiff+threshold in window mode) */
+    DVC_PROF_FRONT = 0,   /* K1: gray (+blur5) (+absdiff+threshold in window mode); flow mode: gray, pyramids and flow */
     DVC_PROF_DIFF = 1,    /* K1 fd mode: absdiff + threshold on blurred planes */
     DVC_PROF_VOTE = 2,    /* K2: window vote */
     DVC_PROF_EMA = 3,     /* K2: addWeighted EMA */
     DVC_PROF_MORPH = 4,   /* K3: morphology chain */
-    DVC_PROF_CCL = 5,     /* contour filter */
+    DVC_PROF_CCL = 5,     /* contour filter; flow mode: bounding rectangles */
     DVC_PROF_DEGRADE = 6, /* K4: overlay + degrade + statistics */
     DVC_PROF_MISC = 7,    /* mask unpacking for callers that ask for uint8 masks */
     DVC_PROF_KERNELS = 8
