@@ -61,10 +61,26 @@ static int flow_rebuild_prev(dvc_handle* h);
 static constexpr int RECT_FRAMES = 8;      // flow loop: planes per launch of the rectangle kernels
 
 // ------------------------------------------------------------------------------------------------
-// structuring elements -> MorphChain
+// structuring elements -> MorphPlan (k_morph_chain runs and large primitives)
 // ------------------------------------------------------------------------------------------------
-// Row runs of np.ones((k,k)) or cv2.getStructuringElement(MORPH_ELLIPSE,(k,k)) relative to the default
-// anchor (k/2, k/2).  The ellipse restates OpenCV's morph code: row i spans |dx| <= rint(c*sqrt(r^2-dy^2)/r).
+// Columns [j1, j2) of row i of np.ones((k,k)) or cv2.getStructuringElement(MORPH_ELLIPSE,(k,k)) (empty when j2 <= j1).
+// The ellipse restates OpenCV's morph code: row i spans |dx| <= rint(c*sqrt(r^2-dy^2)/r).
+static void element_row(int shape, int k, int i, int& j1, int& j2) {
+    j1 = 0; j2 = k;
+    if (shape == DVC_SHAPE_ELLIPSE) {
+        const int r = k / 2, c = k / 2;
+        const double inv_r2 = r ? 1.0 / ((double)r * r) : 0.0;
+        const int dy = i - r;
+        j1 = j2 = 0;
+        if (std::abs(dy) <= r) {
+            const int dx = (int)std::nearbyint(c * std::sqrt((r * r - dy * dy) * inv_r2));
+            j1 = std::max(c - dx, 0);
+            j2 = std::min(c + dx + 1, k);
+        }
+    }
+}
+
+// Row runs of the element relative to the default anchor (k/2, k/2).
 static bool make_prim(int shape, int k, bool erode, MorphPrim& p) {
     if (k < 1 || k > MORPH_MAX_K) return false;
     memset(&p, 0, sizeof(p));
@@ -72,18 +88,8 @@ static bool make_prim(int shape, int k, bool erode, MorphPrim& p) {
     const int a = k / 2;
     int n = 0;
     for (int i = 0; i < k; ++i) {
-        int j1 = 0, j2 = k;
-        if (shape == DVC_SHAPE_ELLIPSE) {
-            const int r = k / 2, c = k / 2;
-            const double inv_r2 = r ? 1.0 / ((double)r * r) : 0.0;
-            const int dy = i - r;
-            j1 = j2 = 0;
-            if (std::abs(dy) <= r) {
-                const int dx = (int)std::nearbyint(c * std::sqrt((r * r - dy * dy) * inv_r2));
-                j1 = std::max(c - dx, 0);
-                j2 = std::min(c + dx + 1, k);
-            }
-        }
+        int j1, j2;
+        element_row(shape, k, i, j1, j2);
         if (j2 <= j1) continue;
         p.dy[n] = (int8_t)(i - a);
         p.lo[n] = (int8_t)(j1 - a);
@@ -112,40 +118,68 @@ static bool make_prim(int shape, int k, bool erode, MorphPrim& p) {
     return true;
 }
 
-static bool chain_push(MorphChain& ch, int op, int shape, int k) {
+// One primitive with an element of at most MORPH_MAX_K appended to a k_morph_chain run
+static bool chain_push_small(MorphChain& ch, bool erode, int shape, int k) {
+    // Two consecutive odd rectangles of the same polarity are one rectangle: the Minkowski sum (k1 + k2 - 1), which is
+    // exact with cv2's "ignore what is outside the image" borders because the intermediate pixel of any two-step path
+    // lies between its end points, inside the image.  CLOSE, OPEN, DILATE with one k x k element (BASELINE config 3)
+    // is D E E D D = D(k) E(2k-1) D(2k-1): three passes instead of five, and a pass costs the same for any k.
+    if (ch.n > 0 && shape == DVC_SHAPE_RECT && (k & 1) && k >= 3) {
+        MorphPrim& q = ch.p[ch.n - 1];
+        const int kq = q.kind - 100;
+        if (q.kind >= 103 && (bool)q.erode == erode && kq + k - 1 <= MORPH_MAX_K) {
+            if (!make_prim(DVC_SHAPE_RECT, kq + k - 1, erode, q)) return false;
+            ch.halo_top += k / 2;
+            ch.halo_bot += k / 2;
+            ch.pad = std::max<int>(ch.pad, (kq + k - 1) / 2);
+            return true;
+        }
+    }
+    // Likewise MORPH_ELLIPSE (2, 2) twice (the E E in the middle of CLOSE, OPEN): one pass with the summed element (kind 3)
+    if (ch.n > 0 && shape == DVC_SHAPE_ELLIPSE && k == 2) {
+        MorphPrim& q = ch.p[ch.n - 1];
+        if (q.kind == 1 && (bool)q.erode == erode) {
+            q.kind = 3;
+            ch.halo_top += 1;           // the element reaches one more row up; nothing below the anchor
+            return true;
+        }
+    }
+    if (ch.n >= MORPH_MAX_PRIMS) return false;
+    MorphPrim& p = ch.p[ch.n];
+    if (!make_prim(shape, k, erode, p)) return false;
+    ch.halo_top += -std::min<int>(p.dy[0], 0);
+    ch.halo_bot += std::max<int>(p.dy[p.nrows - 1], 0);
+    if (p.kind >= 100) ch.pad = std::max<int>(ch.pad, (p.kind - 100) / 2);       // rect_pass<K> reads K / 2 rows beyond its run
+    ++ch.n;
+    return true;
+}
+
+// A primitive whose element is larger than MORPH_MAX_K (k_mask.cuh: k_mlarge_*).  Its row table depends on the frame size
+// (rows and runs are clipped to the frame) and is built by large_prepare.
+constexpr int MORPH_LARGE_MAX_K = 32767;
+struct LargePrim {
+    int shape, k, erode;
+    int levels;                        // table rows sorted by doubling level: level p is rows [lv_beg[p], lv_beg[p + 1])
+    int lv_beg[17];
+    int dy0, B;                        // rect: the vertical reach [dy0, dy0 + B - 1], clipped to the frame
+    LargeRow* rows_dev;                // the table on the device: allocated by the handle at create, or per call
+};
+// A chain as launched: runs of small primitives (one k_morph_chain launch each) and large primitives between them
+struct MorphSeg { int large; MorphChain ch; LargePrim lp; };
+struct MorphPlan { int n; MorphSeg seg[MORPH_MAX_PRIMS]; };
+
+static bool chain_push(MorphPlan& pl, int op, int shape, int k) {
     auto push = [&](bool erode) {
-        // Two consecutive odd rectangles of the same polarity are one rectangle: the Minkowski sum (k1 + k2 - 1), which is
-        // exact with cv2's "ignore what is outside the image" borders because the intermediate pixel of any two-step path
-        // lies between its end points, inside the image.  CLOSE, OPEN, DILATE with one k x k element (BASELINE config 3)
-        // is D E E D D = D(k) E(2k-1) D(2k-1): three passes instead of five, and a pass costs the same for any k.
-        if (ch.n > 0 && shape == DVC_SHAPE_RECT && (k & 1) && k >= 3) {
-            MorphPrim& q = ch.p[ch.n - 1];
-            const int kq = q.kind - 100;
-            if (q.kind >= 103 && (bool)q.erode == erode && kq + k - 1 <= MORPH_MAX_K) {
-                if (!make_prim(DVC_SHAPE_RECT, kq + k - 1, erode, q)) return false;
-                ch.halo_top += k / 2;
-                ch.halo_bot += k / 2;
-                ch.pad = std::max<int>(ch.pad, (kq + k - 1) / 2);
-                return true;
-            }
+        if (k < 1 || k > MORPH_LARGE_MAX_K) return false;
+        const bool large = k > MORPH_MAX_K;
+        if (large || pl.n == 0 || pl.seg[pl.n - 1].large) {
+            if (pl.n >= MORPH_MAX_PRIMS) return false;
+            MorphSeg& s = pl.seg[pl.n++];
+            memset(&s, 0, sizeof(s));
+            s.large = large;
+            if (large) { s.lp.shape = shape; s.lp.k = k; s.lp.erode = erode; return true; }
         }
-        // Likewise MORPH_ELLIPSE (2, 2) twice (the E E in the middle of CLOSE, OPEN): one pass with the summed element (kind 3)
-        if (ch.n > 0 && shape == DVC_SHAPE_ELLIPSE && k == 2) {
-            MorphPrim& q = ch.p[ch.n - 1];
-            if (q.kind == 1 && (bool)q.erode == erode) {
-                q.kind = 3;
-                ch.halo_top += 1;           // the element reaches one more row up; nothing below the anchor
-                return true;
-            }
-        }
-        if (ch.n >= MORPH_MAX_PRIMS) return false;
-        MorphPrim& p = ch.p[ch.n];
-        if (!make_prim(shape, k, erode, p)) return false;
-        ch.halo_top += -std::min<int>(p.dy[0], 0);
-        ch.halo_bot += std::max<int>(p.dy[p.nrows - 1], 0);
-        if (p.kind >= 100) ch.pad = std::max<int>(ch.pad, (p.kind - 100) / 2);       // rect_pass<K> reads K / 2 rows beyond its run
-        ++ch.n;
-        return true;
+        return chain_push_small(pl.seg[pl.n - 1].ch, erode, shape, k);
     };
     switch (op) {
         case DVC_MORPH_ERODE: return push(true);
@@ -154,6 +188,35 @@ static bool chain_push(MorphChain& ch, int op, int shape, int k) {
         case DVC_MORPH_CLOSE: return push(false) && push(true);
     }
     return false;
+}
+
+// The row table of a large primitive for an H x W frame.  Offsets beyond the frame reach nothing, so rows with |dy| > H - 1
+// are dropped and runs are clipped to [-(W - 1), W - 1]: the work and the table stay bounded by the frame.  A rect is one
+// run (horizontal pass) and a vertical reach (van Herk pass).
+static void large_prepare(LargePrim& lp, int H, int W, std::vector<LargeRow>& rows) {
+    const int k = lp.k, a = k / 2;
+    std::vector<LargeRow> by_level[17];
+    int levels = 0;
+    for (int i = 0; i < k; ++i) {
+        const int dy = i - a;
+        if (lp.shape == DVC_SHAPE_RECT ? dy != 0 : (dy < -(H - 1) || dy > H - 1)) continue;
+        int j1, j2;
+        element_row(lp.shape, k, i, j1, j2);
+        if (j2 <= j1) continue;
+        LargeRow e = {lp.shape == DVC_SHAPE_RECT ? 0 : dy, std::max(j1 - a, -(W - 1)), std::min(j2 - 1 - a, W - 1), 0};
+        int p = 0;
+        while ((2 << p) <= e.hi - e.lo + 1) ++p;
+        by_level[p].push_back(e);
+        levels = std::max(levels, p + 1);
+    }
+    rows.clear();
+    for (int p = 0; p <= levels; ++p) {
+        lp.lv_beg[p] = (int)rows.size();
+        if (p < levels) rows.insert(rows.end(), by_level[p].begin(), by_level[p].end());
+    }
+    lp.levels = levels;
+    lp.dy0 = std::max(-a, -(H - 1));
+    lp.B = std::min(k - 1 - a, H - 1) - lp.dy0 + 1;
 }
 
 // python: smallest c with c*255 >= alpha*L*255, evaluated in doubles exactly as motion_compression_opt.py:86
@@ -249,6 +312,104 @@ static int launch_morph_chain(char* ERRBUF, const uint32_t* src, uint32_t* dst, 
     if (threads == 256) k_morph_chain<256><<<grid, 256, smem, st>>>(src, dst, H, W, wpr, band, ch);
     else k_morph_chain<1024><<<grid, threads, smem, st>>>(src, dst, H, W, wpr, band, ch);
     CHECK_LAUNCH();
+    return DVC_OK;
+}
+
+// Planes per launch group of a large primitive: its two level sets take 2 x H x mlarge_rs(wpr) words a plane, at most 256 MiB.
+static int large_chunk(int n, int H, int wpr) {
+    const size_t per_plane = 2 * (size_t)H * mlarge_rs(wpr) * 4;
+    return (int)std::max<size_t>(1, std::min<size_t>({(size_t)n, 65535, ((size_t)256 << 20) / per_plane}));
+}
+// Scratch words for running a plan with a large primitive on n planes: two level sets of large_chunk planes, then n planes
+// that the plan's outputs alternate with dst.
+static size_t plan_scratch_words(int n, int H, int W) {
+    const int wpr = words_per_row(W);
+    return 2 * (size_t)large_chunk(n, H, wpr) * H * mlarge_rs(wpr) + (size_t)n * H * wpr;
+}
+static bool plan_has_large(const MorphPlan& pl) {
+    for (int i = 0; i < pl.n; ++i) if (pl.seg[i].large) return true;
+    return false;
+}
+static int large_launches(const LargePrim& lp, int n, int H, int W) {
+    int last = -1, nonempty = 0;
+    for (int p = 0; p < lp.levels; ++p) if (lp.lv_beg[p + 1] > lp.lv_beg[p]) { last = p; ++nonempty; }
+    const int per_chunk = 1 + last + nonempty + (lp.shape == DVC_SHAPE_RECT ? 2 : 0);
+    const int chunk = large_chunk(n, H, words_per_row(W));
+    return per_chunk * ((n + chunk - 1) / chunk);
+}
+static int plan_launches(const MorphPlan& pl, int n, int H, int W) {
+    int c = 0;
+    for (int i = 0; i < pl.n; ++i) c += pl.seg[i].large ? large_launches(pl.seg[i].lp, n, H, W) : 1;
+    return c;
+}
+
+// One large primitive, src -> dst (may be the same planes: src is read only by the first launch of each group of planes).
+// F: the two level sets (plan_scratch_words).
+static int launch_large(char* ERRBUF, const uint32_t* src, uint32_t* dst, int n, int H, int W, const LargePrim& lp,
+                        uint32_t* F, cudaStream_t st) {
+    const int wpr = words_per_row(W);
+    if (wpr > 256) return set_err(ERRBUF, DVC_ERR_UNSUPPORTED, "frames wider than 8192 pixels are not supported by the morphology kernel");
+    const size_t pw = (size_t)H * wpr, lw = (size_t)H * mlarge_rs(wpr);
+    const uint32_t flip = lp.erode ? 0xffffffffu : 0u;
+    const bool rect = lp.shape == DVC_SHAPE_RECT;
+    int last = -1;
+    for (int p = 0; p < lp.levels; ++p) if (lp.lv_beg[p + 1] > lp.lv_beg[p]) last = p;
+    const int chunk = large_chunk(n, H, wpr);
+    for (int c0 = 0; c0 < n; c0 += chunk) {
+        const int cn = std::min(chunk, n - c0);
+        const uint32_t* s = src + (size_t)c0 * pw;
+        uint32_t* d = dst + (size_t)c0 * pw;
+        uint32_t* L0 = F;
+        uint32_t* L1 = F + (size_t)chunk * lw;
+        const dim3 gl(cdiv(lw, 256), cn), gw(cdiv(pw, 256), cn);
+        k_mlarge_level0<<<gl, 256, 0, st>>>(s, L0, H, W, wpr, flip);
+        CHECK_LAUNCH();
+        bool first = true;
+        for (int p = 0; p <= last; ++p) {
+            if (p > 0) {
+                k_mlarge_double<<<gl, 256, 0, st>>>(L0, L1, H, wpr, 1 << (p - 1));
+                CHECK_LAUNCH();
+                std::swap(L0, L1);
+            }
+            if (lp.lv_beg[p + 1] == lp.lv_beg[p]) continue;
+            k_mlarge_rows<<<gw, 256, 0, st>>>(L0, d, H, W, wpr, lp.rows_dev, lp.lv_beg[p], lp.lv_beg[p + 1], p, first,
+                                              !rect && p == last ? flip : 0u);
+            CHECK_LAUNCH();
+            first = false;
+        }
+        if (rect) {         // the level sets are free again: g and h of the column pass
+            uint32_t* g = F;
+            uint32_t* h = F + (size_t)chunk * lw;
+            k_mlarge_vscan<<<dim3(cdiv((size_t)((H + lp.B - 1) / lp.B) * wpr, 256), cn), 256, 0, st>>>(d, g, h, H, wpr, lp.B);
+            CHECK_LAUNCH();
+            k_mlarge_vcombine<<<gw, 256, 0, st>>>(g, h, d, H, W, wpr, lp.B, lp.dy0, flip);
+            CHECK_LAUNCH();
+        }
+    }
+    return DVC_OK;
+}
+
+// A whole chain: each run of small primitives is one k_morph_chain launch, each large primitive its own launch group.  The
+// segments' outputs alternate between dst and the scratch's plane set so that no k_morph_chain launch reads the planes it
+// writes; the last segment writes dst.  A chain of small primitives only is exactly one launch_morph_chain.
+static int launch_morph_plan(char* ERRBUF, const uint32_t* src, uint32_t* dst, int n, int H, int W, const MorphPlan& pl,
+                             uint32_t* scratch, cudaStream_t st) {
+    if (pl.n == 0) {
+        if (src != dst) CU(cudaMemcpyAsync(dst, src, (size_t)n * H * words_per_row(W) * 4, cudaMemcpyDeviceToDevice, st));
+        return DVC_OK;
+    }
+    const int wpr = words_per_row(W);
+    uint32_t* const tmp = scratch ? scratch + 2 * (size_t)large_chunk(n, H, wpr) * H * mlarge_rs(wpr) : nullptr;
+    uint32_t* out[MORPH_MAX_PRIMS];
+    out[pl.n - 1] = dst;
+    for (int i = pl.n - 2; i >= 0; --i) out[i] = pl.seg[i + 1].large ? out[i + 1] : (out[i + 1] == dst ? tmp : dst);
+    const uint32_t* in = src;
+    for (int i = 0; i < pl.n; ++i) {
+        const int rc = pl.seg[i].large ? launch_large(ERRBUF, in, out[i], n, H, W, pl.seg[i].lp, scratch, st)
+                                       : launch_morph_chain(ERRBUF, in, out[i], n, H, W, pl.seg[i].ch, st);
+        if (rc) return rc;
+        in = out[i];
+    }
     return DVC_OK;
 }
 
@@ -655,7 +816,8 @@ struct dvc_handle {
     uint8_t* blurred;             // FD: [max_batch] gray planes
     CclScratch ccl;
     FlowLoop* flow;               // FLOW only
-    MorphChain chain;
+    MorphPlan plan;               // the mask clean-up chain; large primitives' row tables are allocated at create
+    uint32_t* morph_scratch;      // plan_scratch_words(max_batch * S planes) when the plan has a large primitive
     Counters* counters_dev;
     dvc_counters counters_host;   // frames / pixels / blocks are counted on the host
     // two-stream software pipeline: mask kernels of batch c+1 overlap the degrade kernel of batch c
@@ -807,14 +969,14 @@ static int create_impl(const dvc_config* cfg, dvc_handle* h) {
     }
     CU(cudaMalloc(&h->counters_dev, sizeof(Counters)));
     CU(cudaMemset(h->counters_dev, 0, sizeof(Counters)));
-    h->chain.n = 0; h->chain.pad = 0; h->chain.halo_top = h->chain.halo_bot = 0;
+    h->plan.n = 0;
     if (cfg->mode == DVC_MODE_FD) {
         CU(cudaMalloc(&h->acc, h->plane_bytes * S));
         CU(cudaMemset(h->acc, 0, h->plane_bytes * S));
         int rc = ccl_scratch_alloc(h->err, h->ccl, std::min(T, std::max(1, measure_env("DVC_CCL_CHUNK", 256))), h->H, h->W);
         if (rc) return rc;
-        if (cfg->kernel_size > 0 && !chain_push(h->chain, DVC_MORPH_DILATE, DVC_SHAPE_RECT, cfg->kernel_size))
-            return set_err(h->err, DVC_ERR_UNSUPPORTED, "kernel_size %d: supported range is 1..%d", cfg->kernel_size, MORPH_MAX_K);
+        if (cfg->kernel_size > 0 && !chain_push(h->plan, DVC_MORPH_DILATE, DVC_SHAPE_RECT, cfg->kernel_size))
+            return set_err(h->err, DVC_ERR_UNSUPPORTED, "kernel_size %d: supported range is 1..%d", cfg->kernel_size, MORPH_LARGE_MAX_K);
     } else {
         if (cfg->window_size < 1 || cfg->window_size > WINDOW_MAX)
             return set_err(h->err, DVC_ERR_UNSUPPORTED, "window_size %d: supported range is 1..%d", cfg->window_size, WINDOW_MAX);
@@ -823,14 +985,25 @@ static int create_impl(const dvc_config* cfg, dvc_handle* h) {
         CU(cudaMemset(h->ring, 0, h->plane_words * 4 * h->ring_cap * S));
         window_min_counts(cfg->alpha_fraction, cfg->window_size, h->min_counts);
         if (cfg->morph_kernel > 0) {
-            if (!chain_push(h->chain, DVC_MORPH_CLOSE, cfg->morph_shape, cfg->morph_kernel) ||
-                !chain_push(h->chain, DVC_MORPH_OPEN, cfg->morph_shape, cfg->morph_kernel))
-                return set_err(h->err, DVC_ERR_UNSUPPORTED, "morph_kernel %d: supported range is 1..%d", cfg->morph_kernel, MORPH_MAX_K);
+            if (!chain_push(h->plan, DVC_MORPH_CLOSE, cfg->morph_shape, cfg->morph_kernel) ||
+                !chain_push(h->plan, DVC_MORPH_OPEN, cfg->morph_shape, cfg->morph_kernel))
+                return set_err(h->err, DVC_ERR_UNSUPPORTED, "morph_kernel %d: supported range is 1..%d", cfg->morph_kernel, MORPH_LARGE_MAX_K);
         }
-        if (cfg->kernel_size > 0 && !chain_push(h->chain, DVC_MORPH_DILATE, DVC_SHAPE_RECT, cfg->kernel_size))
-            return set_err(h->err, DVC_ERR_UNSUPPORTED, "kernel_size %d: supported range is 1..%d", cfg->kernel_size, MORPH_MAX_K);
-        if (cfg->mode == DVC_MODE_FLOW) return flow_create(h);
+        if (cfg->kernel_size > 0 && !chain_push(h->plan, DVC_MORPH_DILATE, DVC_SHAPE_RECT, cfg->kernel_size))
+            return set_err(h->err, DVC_ERR_UNSUPPORTED, "kernel_size %d: supported range is 1..%d", cfg->kernel_size, MORPH_LARGE_MAX_K);
     }
+    if (plan_has_large(h->plan)) {
+        std::vector<LargeRow> rows;
+        for (int i = 0; i < h->plan.n; ++i) {
+            LargePrim& lp = h->plan.seg[i].lp;
+            if (!h->plan.seg[i].large) continue;
+            large_prepare(lp, h->H, h->W, rows);
+            CU(cudaMalloc(&lp.rows_dev, rows.size() * sizeof(LargeRow)));
+            CU(cudaMemcpy(lp.rows_dev, rows.data(), rows.size() * sizeof(LargeRow), cudaMemcpyHostToDevice));
+        }
+        CU(cudaMalloc(&h->morph_scratch, plan_scratch_words(T, h->H, h->W) * 4));
+    }
+    if (cfg->mode == DVC_MODE_FLOW) return flow_create(h);
     return DVC_OK;
 }
 
@@ -848,6 +1021,8 @@ extern "C" int dvc_destroy(dvc_handle* h) {
     if (h->ev_user) cudaEventDestroy(h->ev_user);
     for (int s = 0; s < 2; ++s) { if (h->ev_front[s]) cudaEventDestroy(h->ev_front[s]); if (h->ev_mask[s]) cudaEventDestroy(h->ev_mask[s]); if (h->ev_k4[s]) cudaEventDestroy(h->ev_k4[s]); }
     ccl_scratch_free(h->ccl);
+    for (int i = 0; i < h->plan.n; ++i) if (h->plan.seg[i].large) cudaFree(h->plan.seg[i].lp.rows_dev);
+    cudaFree(h->morph_scratch);
     flow_destroy(h);
     if (h->staging) {
         for (int b = 0; b < 2; ++b) {
@@ -1114,9 +1289,9 @@ static int process_batch_impl(dvc_handle* h, const uint8_t* frames, int T, uint8
         CHECK_LAUNCH();
         }
         const uint32_t* fin = bits_a;
-        if (h->chain.n) {
-            ProfScope ps(h, DVC_PROF_MORPH, 1, st);
-            int rc = launch_morph_chain(h->err, bits_a, bits_b, ST, H, W, h->chain, st);
+        if (h->plan.n) {
+            ProfScope ps(h, DVC_PROF_MORPH, plan_launches(h->plan, ST, H, W), st);
+            int rc = launch_morph_plan(h->err, bits_a, bits_b, ST, H, W, h->plan, h->morph_scratch, st);
             if (rc) return rc;
             fin = bits_b;
         }
@@ -1154,8 +1329,8 @@ static int process_batch_impl(dvc_handle* h, const uint8_t* frames, int T, uint8
         rc = launch_contour_filter(h->err, bits_a, bits_b, ST, H, W, h->cfg.min_area, h->ccl, st);
         }
         if (rc) return rc;
-        { ProfScope ps(h, DVC_PROF_MORPH, 1, st);
-        rc = launch_morph_chain(h->err, bits_b, bits_a, ST, H, W, h->chain, st);      // dilate -> bits_a
+        { ProfScope ps(h, DVC_PROF_MORPH, std::max(1, plan_launches(h->plan, ST, H, W)), st);
+        rc = launch_morph_plan(h->err, bits_b, bits_a, ST, H, W, h->plan, h->morph_scratch, st);      // dilate -> bits_a
         }
         if (rc) return rc;
         const float alpha = (float)h->cfg.release_factor, beta = (float)(1.0 - h->cfg.release_factor);
@@ -1478,17 +1653,30 @@ extern "C" int dvc_morph_u8(const uint8_t* src, uint8_t* dst, int32_t n, int32_t
     if (!src || !dst) return set_err(nullptr, DVC_ERR_INVALID, "dvc_morph_u8: null pointer");
     if (op < DVC_MORPH_ERODE || op > DVC_MORPH_CLOSE || (shape != DVC_SHAPE_RECT && shape != DVC_SHAPE_ELLIPSE))
         return set_err(nullptr, DVC_ERR_INVALID, "dvc_morph_u8: bad op/shape");
-    MorphChain ch;
-    ch.n = 0; ch.pad = 0; ch.halo_top = ch.halo_bot = 0;
-    if (!chain_push(ch, op, shape, k)) return set_err(nullptr, DVC_ERR_UNSUPPORTED, "dvc_morph_u8: kernel size %d outside 1..%d", k, MORPH_MAX_K);
+    MorphPlan pl;
+    pl.n = 0;
+    if (!chain_push(pl, op, shape, k)) return set_err(nullptr, DVC_ERR_UNSUPPORTED, "dvc_morph_u8: kernel size %d outside 1..%d", k, MORPH_LARGE_MAX_K);
     cudaStream_t st = (cudaStream_t)stream;
     const size_t pw = (size_t)H * words_per_row(W);
-    ScopedAsyncBuf a(st), b(st);
+    ScopedAsyncBuf a(st), b(st), scratch(st), rows0(st), rows1(st);
+    ScopedAsyncBuf* rows_buf[2] = {&rows0, &rows1};          // an op is at most two primitives
+    std::vector<LargeRow> rows;
+    for (int i = 0; i < pl.n; ++i) {
+        if (!pl.seg[i].large) continue;
+        large_prepare(pl.seg[i].lp, H, W, rows);
+        CU(rows_buf[i]->alloc(rows.size() * sizeof(LargeRow)));
+        CU(cudaMemcpyAsync(rows_buf[i]->p, rows.data(), rows.size() * sizeof(LargeRow), cudaMemcpyHostToDevice, st));
+        pl.seg[i].lp.rows_dev = (LargeRow*)rows_buf[i]->p;
+    }
+    if (plan_has_large(pl)) {
+        if (words_per_row(W) > 256) return set_err(nullptr, DVC_ERR_UNSUPPORTED, "frames wider than 8192 pixels are not supported by the morphology kernel");
+        CU(scratch.alloc(plan_scratch_words(n, H, W) * 4));
+    }
     CU(a.alloc(pw * 4 * n));
     CU(b.alloc(pw * 4 * n));
     rc = pack_to_bits(src, (uint32_t*)a.p, n, H, W, st);
     if (rc) return rc;
-    rc = launch_morph_chain(nullptr, (const uint32_t*)a.p, (uint32_t*)b.p, n, H, W, ch, st);
+    rc = launch_morph_plan(nullptr, (const uint32_t*)a.p, (uint32_t*)b.p, n, H, W, pl, (uint32_t*)scratch.p, st);
     if (rc) return rc;
     return unpack_from_bits((const uint32_t*)b.p, dst, n, H, W, st);
 }

@@ -12,6 +12,8 @@
 //                   with one cp.async.bulk (TMA) copy, every primitive of the chain runs out of shared
 //                   memory (separable OR-doubling: the binary form of van Herk/Gil-Werman), one
 //                   write of the final band
+//   k_mlarge_*      primitives whose element is larger than MORPH_MAX_K: doubling tables for the horizontal runs, van Herk
+//                   down the columns for rectangles, one launch group per primitive between global bit-planes
 #pragma once
 #include "common.cuh"
 #include "k_front.cuh"
@@ -676,6 +678,104 @@ k_morph_chain(const uint32_t* __restrict__ src, uint32_t* __restrict__ dst, int 
     // write the band
     const int out_rows = min(band_rows, H - y0);
     for (int i = tid; i < out_rows * wpr; i += nt) dp[(size_t)y0 * wpr + i] = A[ch.halo_top * wpr + i];
+}
+
+// ------------------------------------------------------------------------------------------------
+// structuring elements larger than MORPH_MAX_K: one primitive at a time, between global bit-planes
+// ------------------------------------------------------------------------------------------------
+// Horizontal runs of any length come from a doubling table: level p holds F_p(x) = OR of the dilation-domain bits
+// [x, x + 2^p), and a run [x + lo, x + hi] of length L, 2^p <= L < 2^(p+1), is F_p(x + lo) | F_p(x + hi + 1 - 2^p): two
+// funnel-shifted reads per output word whatever L is.  Runs are clipped to the frame on the host (|lo|, |hi| <= W - 1), so a
+// level row needs wpr words of zeros on the left and wpr + 1 on the right: MLARGE_RS(wpr) words, image word 0 at offset wpr.
+// Bits outside the image are 0 in the dilation domain, so erosion is NOT dilate NOT with cv2's ignored borders, as in
+// k_morph_chain.
+//   rect      rows of one run: the horizontal run at level p, then van Herk / Gil-Werman down the columns (k_mlarge_vscan
+//             + k_mlarge_vcombine), whose cost does not depend on k
+//   ellipse   not separable: out(y) = OR over the element rows dy of the run of row y + dy, one k_mlarge_rows launch per level
+//             with the rows of that level
+__host__ __device__ inline int mlarge_rs(int wpr) { return 3 * wpr + 1; }
+struct LargeRow { int dy, lo, hi, pad; };   // one element row clipped to the frame: run [lo, hi] of row y + dy
+
+// level 0: the input in the dilation domain, zeros in the padding.  grid: (words of H padded rows, planes)
+__global__ void __launch_bounds__(256)
+k_mlarge_level0(const uint32_t* __restrict__ src, uint32_t* __restrict__ F, int H, int W, int wpr, uint32_t flip) {
+    const int rs = mlarge_rs(wpr);
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)H * rs) return;
+    const int y = (int)(i / rs), w = (int)(i % rs) - wpr;
+    uint32_t v = 0u;
+    if (w >= 0 && w < wpr) v = (src[((size_t)blockIdx.y * H + y) * wpr + w] ^ flip) & valid_mask(w, W);
+    F[(size_t)blockIdx.y * H * rs + i] = v;
+}
+
+// level q from level q - 1: F_q(x) = F_{q-1}(x) | F_{q-1}(x + s), s = 2^(q-1); words beyond the padding read as zero
+__global__ void __launch_bounds__(256)
+k_mlarge_double(const uint32_t* __restrict__ Fi, uint32_t* __restrict__ Fo, int H, int wpr, int s) {
+    const int rs = mlarge_rs(wpr);
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)H * rs) return;
+    const int c = (int)(i % rs), c0 = c + (s >> 5);
+    const size_t base = (size_t)blockIdx.y * H * rs + i - c;
+    const uint32_t a = c0 < rs ? Fi[base + c0] : 0u, b = c0 + 1 < rs ? Fi[base + c0 + 1] : 0u;
+    Fo[base + c] = Fi[base + c] | __funnelshift_r(a, b, s & 31);
+}
+
+// out(y) |= OR over table rows [beg, end) (all at level p) of the run [x + lo, x + hi] of level row y + dy.  `first` starts
+// from zero instead of the dilation-domain value already in dst; the result is stored as (acc ^ xor_out) & valid, so the
+// last launch of a primitive passes its flip and the others 0.  grid: (words of H rows, planes)
+__global__ void __launch_bounds__(256)
+k_mlarge_rows(const uint32_t* __restrict__ F, uint32_t* __restrict__ dst, int H, int W, int wpr,
+              const LargeRow* __restrict__ rows, int beg, int end, int p, int first, uint32_t xor_out) {
+    const int rs = mlarge_rs(wpr);
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)H * wpr) return;
+    const int y = (int)(i / wpr), j = (int)(i % wpr), x0 = j * 32, tail = 1 - (1 << p);
+    const size_t o = (size_t)blockIdx.y * H * wpr + i;
+    const uint32_t* Fp = F + (size_t)blockIdx.y * H * rs + wpr;
+    uint32_t acc = first ? 0u : dst[o];
+    for (int r = beg; r < end; ++r) {
+        const LargeRow e = rows[r];
+        const int yy = y + e.dy;
+        if (yy < 0 || yy >= H) continue;
+        const uint32_t* row = Fp + (size_t)yy * rs;
+        const int pa = x0 + e.lo, pb = x0 + e.hi + tail;           // >= -(W - 1) and < 2 W: inside the padded row
+        const int wa = pa >> 5, wb = pb >> 5;
+        acc |= __funnelshift_r(row[wa], row[wa + 1], pa & 31) | __funnelshift_r(row[wb], row[wb + 1], pb & 31);
+    }
+    dst[o] = (acc ^ xor_out) & valid_mask(j, W);
+}
+
+// van Herk / Gil-Werman down the columns, blocks of B rows from row 0: g(y) = OR of rows [block start, y], h(y) = OR of rows
+// [y, block end] (clipped to H).  One thread per (word column, block).  grid: (word columns x blocks, planes)
+__global__ void __launch_bounds__(256)
+k_mlarge_vscan(const uint32_t* __restrict__ in, uint32_t* __restrict__ g, uint32_t* __restrict__ h, int H, int wpr, int B) {
+    const int nb = (H + B - 1) / B;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nb * wpr) return;
+    const int j = i % wpr, y0 = (i / wpr) * B, y1 = min(H, y0 + B);
+    const size_t off = (size_t)blockIdx.y * H * wpr + j;
+    in += off; g += off; h += off;
+    uint32_t a = 0u;
+    for (int y = y0; y < y1; ++y) { a |= in[(size_t)y * wpr]; g[(size_t)y * wpr] = a; }
+    a = 0u;
+    for (int y = y1 - 1; y >= y0; --y) { a |= in[(size_t)y * wpr]; h[(size_t)y * wpr] = a; }
+}
+
+// out(y) = OR of rows [y + dy0, y + dy0 + B - 1] = h(s) | g(e), s = y + dy0 <= y, e = s + B - 1 >= y.  Rows outside the image
+// are zero: h(s < 0) is the suffix of an all-outside block; g(e >= H) is g(H - 1) when row H - 1 is in e's block, else zero.
+__global__ void __launch_bounds__(256)
+k_mlarge_vcombine(const uint32_t* __restrict__ g, const uint32_t* __restrict__ h, uint32_t* __restrict__ dst, int H, int W,
+                  int wpr, int B, int dy0, uint32_t flip) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)H * wpr) return;
+    const int y = (int)(i / wpr), j = (int)(i % wpr);
+    const size_t pl = (size_t)blockIdx.y * H * wpr;
+    const int s = y + dy0, e = s + B - 1;
+    uint32_t v = 0u;
+    if (s >= 0) v |= h[pl + (size_t)s * wpr + j];
+    if (e < H) v |= g[pl + (size_t)e * wpr + j];
+    else if ((e / B) * B <= H - 1) v |= g[pl + (size_t)(H - 1) * wpr + j];
+    dst[pl + i] = (v ^ flip) & valid_mask(j, W);
 }
 
 }  // namespace dvc

@@ -208,7 +208,7 @@ int dvc_temporal_ema_u8(uint8_t* acc_inout_dev, const uint8_t* dilated_dev, uint
                         int32_t H, int32_t W, double release_factor, void* stream);
 /* cv2.erode / cv2.dilate / cv2.morphologyEx(OPEN|CLOSE) on binary (0 / non-zero) masks,
  * frame_differencing.py:106, motion_compression_opt.py:89-90.  k x k rect (np.ones) or
- * getStructuringElement(MORPH_ELLIPSE); k <= 33.  n images. */
+ * getStructuringElement(MORPH_ELLIPSE); 1 <= k <= 32767 (elements larger than the image included).  n images. */
 int dvc_morph_u8(const uint8_t* src_dev, uint8_t* dst_dev, int32_t n, int32_t H, int32_t W, int32_t op,
                  int32_t shape, int32_t k, void* stream);
 /* findContours(RETR_EXTERNAL) + contourArea > min_area + drawContours(FILLED),
